@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """HiPAC hot-path benchmark: patches/sec through tile + tissue/lesion mask + ResNet18 features.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): a synthetic level-0 image, 16384 x 16384 RGB per GPU, tiled
 into 1792^2 patches on the reference CLI's 224-px grid (src/main.py:611 -> stride 224 at every
@@ -40,6 +40,26 @@ ALGO_OUT_BYTES = 224 * 224 * 3 * 2 + 9
 # what the kernels really write per survivor: the S2D16 operand layout of conv1 (16 of 12 channels, 115 of 112 columns)
 S2D_BYTES = 112 * 115 * 16 * 2
 REF_STRIDE_MULT = 20              # --impl reference: the reference's own stride argument = 224 * this (every 20th grid column/row)
+DUMP_LIMIT_BYTES = 64_000_000     # --dump-outputs: larger patch sets are reduced to a fixed, seeded sample of rows
+
+
+def dump_outputs(out_dir: str, res: dict):
+    """Write the patch set a caller of the timed path receives (coords, labels, features, logits) as
+    ``out_dir/<name>.npy`` in float32 (coordinates and labels are small integers, exact in float32).  If the set exceeds
+    DUMP_LIMIT_BYTES, the same seeded sample of rows (kept in canonical order) is taken from every array, and its row
+    indices are written as ``rows.npy``; otherwise every row is written."""
+    n = int(res["coords"].shape[0])
+    row_bytes = sum(4 * int(np.prod(v.shape[1:])) for v in res.values())
+    if n * row_bytes + 1024 * len(res) <= DUMP_LIMIT_BYTES:
+        rows = None
+    else:                                                  # + 8 bytes per row for rows.npy, 1 KB per .npy header
+        keep = (DUMP_LIMIT_BYTES - 1024 * (len(res) + 1)) // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in res.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), np.ascontiguousarray((v if rows is None else v[rows]).astype(np.float32)))
+    if rows is not None:
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 def ncu_traffic():
@@ -317,6 +337,8 @@ def run_ours(args):
     launches = int(_lib.lib().hipac_launch_count(1)) // (args.steps + args.warmup)
     # the gathered, canonically sorted patch set of the last resident step (every rank holds the same one)
     res = {k: v.cpu().numpy() for k, v in last_gathered["out"].items()}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
     order = np.lexsort((res["coords"][:, 1], res["coords"][:, 0]))
     canonical = bool(np.array_equal(order, np.arange(len(order))))     # the exchange already delivers (x, y) order
     import zlib
@@ -341,7 +363,7 @@ def run_ours(args):
         v["ms"] *= 2.0 / prof_steps
         v["work"] *= 2.0 / prof_steps
         v["launches"] = int(round(v["launches"] * 2.0 / prof_steps))
-    ms_e2e, total_surv_e, n_e2e_rows = timed(step_e2e, max(2, args.steps // 2), 1)
+    ms_e2e, total_surv_e, n_e2e_rows = timed(step_e2e, args.steps, 1)
     # round 1's methodology, for comparison only: a 2-step profiled pass after the (PCIe-bound, cooler) e2e leg, i.e. at boost clocks
     _lib.profile(True)
     for _ in range(2):
@@ -756,8 +778,14 @@ def main():
     ap.add_argument("--groups", type=int, default=12, help="row groups of the pipelined host->device upload (e2e leg)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--config", type=int, default=1, choices=[0, 1],
-                    help="1 (default): BASELINE configs[1], the bench workload; 0: configs[0] on both arms, whole config (not a driver line)")
+                    help="1 (default): BASELINE configs[1], the bench workload; 0: configs[0] on both arms, whole config")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the patch set of the last timed step (coords, labels, features, logits) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 1 or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the default workload of --impl ours")
     if args.config == 0:
         run_config0(args)
     elif args.impl == "reference":

@@ -7,7 +7,7 @@
 there (SURVEY.md section 8c "GPU box caveat", VERDICT r01 item 6).  ``baseline/_ref/`` is listed in ``.gitignore`` (the
 reference's sources never enter this repository's history) but not in ``.gpurunignore``, so the copy travels with the
 snapshot exactly like the built ``.so``.  Only the files ``src/main.py`` imports on the hot path are copied, unmodified.
-``__graft_entry__.build()`` calls this when the checkout is present.
+Run it by hand where the checkout is present; the build does not depend on it.
 """
 from __future__ import annotations
 

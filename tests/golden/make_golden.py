@@ -1,6 +1,7 @@
-"""Generate tests/golden/*.npz by running the REAL reference (dev container only).
+"""Generate tests/golden/*.npz.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py            # stage-1 and stage-2 fixtures: needs the reference checkout
+    python tests/golden/make_golden.py config0    # the configs[0] fixture: needs only this repository
 
 Each stage-1 fixture freezes what the reference's own ``extract_patches``
 (src/main.py:609-732) emitted for one synthetic slide / level / stride:
@@ -9,6 +10,9 @@ reference's ``transforms.Resize((224,224))`` (src/main.py:814) and a few full
 224x224x3 images.  The stage-2 fixture freezes features of the reference's
 ``ResNet18FeatureExtractor`` (src/models/resnet.py:22-40) fed through its own
 transform chain, for seeded weights.
+
+The configs[0] fixture freezes the whole BASELINE configs[0] (see ``config0_case``) as computed by the CPU oracle, whose
+stage 1 the fixtures above pin to the reference and whose fp32 ResNet18 is the reference's feature extractor.
 """
 from __future__ import annotations
 
@@ -90,9 +94,32 @@ def stage2_case():
                 weight_abs_sum=wsum, seed=0)
 
 
+CONFIG0 = dict(size0=32768, slide_seed=1234, level=3, weight_seed=0)   # bench.py --config 0's slide: 361 candidates
+
+
+def config0_case():
+    """Every survivor of BASELINE configs[0]: the 4096 x 4096 level-3 image of a 32768^2 synthetic slide, P = S = 224,
+    tissue filter + lesion labels + fp32 ResNet18 features and logits of the seeded weights.  The unmodified reference
+    kept 116 of the 361 candidates of this slide (profiles/r02_bench_config0.json)."""
+    c = CONFIG0
+    slide = SyntheticSlide(c["size0"], c["size0"], seed=c["slide_seed"])
+    want = orc.extract_patches_oracle(slide.level_array(c["level"]), slide.lesion_mask(c["level"]), c["level"])
+    assert want["candidates"] == 361 and len(want["coords"]) == 116, (want["candidates"], len(want["coords"]))
+    net = orc.make_resnet18(seed=c["weight_seed"], classifier=True)
+    feats, logits = orc.resnet18_features_fp32(net, want["images"])
+    wsum = float(sum(v.double().abs().sum() for v in net.state_dict().values()))
+    return dict(**c, candidates=want["candidates"], coords=want["coords"], labels=want["labels"],
+                features=feats.astype(np.float32), logits=logits.astype(np.float32), weight_abs_sum=wsum)
+
+
 def main():
-    assert rh.reference_available(), "needs /root/reference"
     only = sys.argv[1:]
+    if only == ["config0"]:
+        d = config0_case()
+        np.savez_compressed(os.path.join(HERE, "config0.npz"), **d)
+        print(f"config0: {len(d['coords'])} survivors of {d['candidates']} candidates, {int(d['labels'].sum())} tumor")
+        return
+    assert rh.reference_available(), "needs the reference checkout (HIPAC_REFERENCE_ROOT)"
     for name in CASES:
         if only and name not in only:
             continue
