@@ -159,8 +159,10 @@ int hipac_resnet18_forward_dcount(const void* d_packed, int num_classes,
                                   float* d_feats, float* d_logits,
                                   void* d_workspace, size_t workspace_bytes, int chunk, void* stream);
 
-/* Test hook: one conv layer of the network on its own (layer index 0..19, network order), bf16 NHWC in/out
- * (layer 0 takes the S2D16 batch), optional residual.  Used by the per-layer parity tests. */
+/* Test hook: one conv layer of the network on its own (layer index 1..19 in network order, except 7), bf16 NHWC in/out,
+ * optional residual.  Used by the per-layer parity tests.  Layer 0 (conv1) exists only fused with the max pool and layer 7
+ * (layer2.0's projection shortcut) only fused into layer2.0.conv2: both are refused with -1, see hipac_resnet18_stem and
+ * hipac_resnet18_conv_ds_fused. */
 int hipac_resnet18_conv_layer(const void* d_packed, int num_classes, int layer,
                               const void* d_in, const void* d_residual, void* d_out,
                               int n_patches, int relu, void* stream);

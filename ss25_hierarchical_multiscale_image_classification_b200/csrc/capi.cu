@@ -1,5 +1,4 @@
 // Error reporting, launch counting and the optional per-kernel CUDA-event profiler of the C ABI.
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <utility>
@@ -24,14 +23,6 @@ int ensure_dyn_smem_impl(const void* func, int bytes) {
   HIPAC_CHECK_CUDA(cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   done[{func, dev}] = bytes;
   return 0;
-}
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("HIPAC_PDL");
-    return !(e && atoi(e) == 0);
-  }();
-  return on;
 }
 
 int device_sm_count(int* sms) {

@@ -52,12 +52,11 @@ int ensure_dyn_smem_impl(const void* func, int bytes);
 template <typename F>
 static inline int ensure_dyn_smem(F* func, int bytes) { return ensure_dyn_smem_impl(reinterpret_cast<const void*>(func), bytes); }
 int device_sm_count(int* sms);
-bool pdl_enabled();   // HIPAC_PDL=0 switches programmatic dependent launch off (A/B and debugging)
 
 // Launch with optional thread-block cluster and programmatic stream serialization (see ptx::pdl_wait in umma.cuh).
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, int cluster_x,
-                                    bool pdl, Args&&... args) {
+                                    Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = stream;
   cudaLaunchAttribute attr[2];
@@ -67,11 +66,9 @@ static inline cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 bl
     attr[na].val.clusterDim.x = (unsigned)cluster_x, attr[na].val.clusterDim.y = 1, attr[na].val.clusterDim.z = 1;
     na++;
   }
-  if (pdl && pdl_enabled()) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    na++;
-  }
+  attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[na].val.programmaticStreamSerializationAllowed = 1;
+  na++;
   cfg.attrs = attr, cfg.numAttrs = (unsigned)na;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }

@@ -1,6 +1,14 @@
 // Row-tile 3x3 / stride-1 / pad-1 convolution on CTA PAIRS (tcgen05 cta_group::2), included by resnet18.cu inside
-// namespace hipac after conv_rows.cuh (same tile geometry: one M-tile = R whole image rows in padded-width coordinates,
-// all nine taps read ONE staged region through shifted UMMA descriptors).
+// namespace hipac after conv_umma2.cuh.
+//
+// The im2col kernel re-reads every activation byte nine times through L2 (once per filter tap), which
+// makes the 64- and 128-channel layers L2-bandwidth bound.  Here one M-tile is R whole image rows in
+// PADDED-width coordinates (Wp = W + 2 positions per row, R * Wp <= 128): a single tiled TMA load brings
+// the (R + 2) x Wp input pixels of one 64-channel slice into shared memory -- TMA's out-of-bounds zero
+// fill materialises the conv padding -- and all nine taps read that ONE staged region through UMMA
+// descriptors that differ only in their start address (tap (r, s) starts r * Wp + s pixels = rows of
+// 128 B further; tests/test_umma_shift_gpu.py pins that hardware behaviour).  Positions x >= W of each
+// padded row produce junk accumulator rows that are simply not stored.
 //
 // Why pairs.  A cta_group::1 UMMA of M = 128 x N x K = 16 reads (128 + N) * 32 bytes of operands from shared memory in
 // N / 2 cycles: 192 B/clk at N = 64 and 128 B/clk at N = 128 against a 128 B/clk shared-memory pipe, so the 64- and
@@ -19,9 +27,49 @@
 //   warps 2.. epilogue: wait the LOCAL tfull, drain their CTA's 128 accumulator rows, arrive on the LEADER's tempty
 #pragma once
 
+struct RowConvParams {
+  int n_img;
+  int num_tiles;  // n_img * (H / R)
+  int relu;
+  const float* bias;
+  const __nv_bfloat16* residual;
+  __nv_bfloat16* out;
+  const int* n_dev;  // device-count mode, see effective_patches()
+  int n_base;
+  int reverse;       // tile order, see g_reverse
+};
+
+// bias + residual (16-byte chunk of 8 bf16, already loaded) + ReLU on 8 accumulator columns -> 8 bf16
+__device__ __forceinline__ uint4 epilogue_chunk8(const uint32_t* v, const float* __restrict__ bias, uint4 res, bool has_res, int relu) {
+  const float4 b0 = __ldg(reinterpret_cast<const float4*>(bias)), b1 = __ldg(reinterpret_cast<const float4*>(bias) + 1);
+  float x[8] = {__uint_as_float(v[0]) + b0.x, __uint_as_float(v[1]) + b0.y, __uint_as_float(v[2]) + b0.z, __uint_as_float(v[3]) + b0.w,
+                __uint_as_float(v[4]) + b1.x, __uint_as_float(v[5]) + b1.y, __uint_as_float(v[6]) + b1.z, __uint_as_float(v[7]) + b1.w};
+  if (has_res) {
+    const __nv_bfloat162* r2 = reinterpret_cast<const __nv_bfloat162*>(&res);
+#pragma unroll
+    for (int i = 0; i < 4; i++) x[2 * i] += __bfloat162float(r2[i].x), x[2 * i + 1] += __bfloat162float(r2[i].y);
+  }
+  if (relu) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) x[i] = fmaxf(x[i], 0.f);
+  }
+  uint4 o;
+  __nv_bfloat162 t;
+  t = __floats2bfloat162_rn(x[0], x[1]), o.x = *reinterpret_cast<uint32_t*>(&t);
+  t = __floats2bfloat162_rn(x[2], x[3]), o.y = *reinterpret_cast<uint32_t*>(&t);
+  t = __floats2bfloat162_rn(x[4], x[5]), o.z = *reinterpret_cast<uint32_t*>(&t);
+  t = __floats2bfloat162_rn(x[6], x[7]), o.w = *reinterpret_cast<uint32_t*>(&t);
+  return o;
+}
+
 // TEPI: the epilogue moves through shared-memory staging and TMA (always for BN = 64; for BN = 128 only the RESIDUAL variant,
 // whose per-thread 256-byte residual fetch is what the LSU cannot keep up with -- it trades one region stage for a
-// single staging tile of two 64-channel halves)
+// single staging tile of two 64-channel halves).  With per-thread stores every epilogue thread owns one output pixel and
+// writes its 64 channels (128 bytes) straight to global memory, and fetches the 128 residual bytes the same way: a warp
+// instruction touches 32 different 128-byte lines, i.e. 32 LSU wavefronts, 512 wavefronts per warp and tile with a
+// residual.  Staged, the residual tile arrives by ONE TMA load into a 128-byte-swizzled buffer, every thread reads /
+// rewrites only its own 128-byte row of that buffer (16-byte accesses, conflict free) and the finished tile leaves by ONE
+// TMA store.
 template <int BN, int KC, int W, int R, int KDS, bool TEPI = (BN == 64)>
 struct Row2Cfg {
   static constexpr int Wp = W + 2;
@@ -33,7 +81,7 @@ struct Row2Cfg {
   static constexpr int kBBlock = kBHalf * 128;              // one (tap, 64-channel slice) block of this CTA's half
   static constexpr int kNumB = 9 * KC + KDS;
   static constexpr int kBBytes = kNumB * kBBlock;
-  // 64-channel tiles leave through shared-memory staging + TMA (see conv_rows_tma.cuh): [warpgroup][buffer] tiles of R x W x 128 B
+  // 64-channel tiles leave through shared-memory staging + TMA (see TEPI above): [warpgroup][buffer] tiles of R x W x 128 B
   static constexpr bool kTmaEpi = TEPI;
   static constexpr int kTileBytes = R * W * 128;                                  // one 64-channel half of an output tile
   static constexpr int kStageBytes = (kTileBytes + 1023) / 1024 * 1024;
@@ -259,7 +307,8 @@ k_conv3x3_rows2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     if (gt == 0) ptx::bulk_wait_group<0>();
   } else if constexpr (Cfg::kTmaEpi) {
     // ===================== epilogue, 64 channels: TMEM -> staging tile (residual in place) -> TMA store =====================
-    // (same protocol as k_conv3x3_rows_tma; the accumulator-drained arrive goes to the LEADER's tempty barrier)
+    // Two staging buffers per epilogue warpgroup: the store of tile j and the residual load of tile j + 1 overlap the math
+    // of tile j.  The accumulator-drained arrive goes to the LEADER's tempty barrier.
     const int wq = warp & 3;
     const int grp = (warp - 2) >> 2;
     const int gt = threadIdx.x - 64 - 128 * grp;

@@ -12,8 +12,8 @@
 // stores one pooled row.  Post-ReLU values are >= 0, so the pool's -inf padding is equivalent to skipping
 // the out-of-range taps.
 //
-// PAIR = true: two CTAs of a cluster work on two blocks with ONE UMMA of M = 256 per tap (tcgen05 cta_group::2, the protocol
-// of conv_rows2.cuh): this kernel is bound by shared-memory bandwidth -- per conv row the UMMAs read 16 x (4 KB of A +
+// Two CTAs of a cluster work on two blocks with ONE UMMA of M = 256 per tap (tcgen05 cta_group::2, the protocol of
+// conv_rows2.cuh): this kernel is bound by shared-memory bandwidth -- per conv row the UMMAs read 16 x (4 KB of A +
 // 2 KB of weights), the pooling exchange and the TMA writes another ~22 KB, against 128 B/clk -- and in a pair each CTA
 // holds and reads only HALF of the weight rows (16 x 1 KB).  Both CTAs then run the same 17 conv rows per block: for the
 // top block of an image row "-1" is computed from the zero-filled halo and the epilogue drops it.
@@ -25,8 +25,8 @@ constexpr int kStemRegionLoad = kStemRows * kS2dW * 32;
 constexpr int kStemRegionBytes = (kStemRegionLoad + 128 * 32 + 1023) / 1024 * 1024;  // + slack for the 128-row UMMA window
 constexpr int kStemWBytes = 64 * 256 * 2;
 constexpr int kStemVBytes = 112 * 128;            // one conv row of bf16 [112][64]
-constexpr int kStemSmem = 2 * kStemRegionBytes + kStemWBytes + 2 * kStemVBytes + 1024 + 256;
-constexpr int kStemSmemPair = kStemSmem - kStemWBytes / 2;
+constexpr int kStemWHalf = kStemWBytes / 2;       // one CTA's 32 weight rows
+constexpr int kStemSmem = 2 * kStemRegionBytes + kStemWHalf + 2 * kStemVBytes + 1024 + 256;
 
 struct StemParams {
   int num_blocks;  // n_img * (56 / kStemPB)
@@ -53,27 +53,25 @@ __device__ __forceinline__ uint4 bf16x8_max(uint4 a, uint4 b) {
 constexpr int kStemDrainWarps = 16;
 constexpr int kStemThreads = 64 + 32 * kStemDrainWarps + 128;
 
-template <bool PAIR>
 __global__ void __launch_bounds__(kStemThreads, 1)
 k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const StemParams p) {
-  constexpr int kWBytes = PAIR ? kStemWBytes / 2 : kStemWBytes;   // this CTA's weight rows: 32 or 64 of [64 x 256]
-  constexpr int kWBlock = kWBytes / 4;                            // one 64-wide K block of them
+  constexpr int kWBlock = kStemWHalf / 4;               // one 64-wide K block of this CTA's weight rows
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sA = base;                                   // 2 block regions
-  uint8_t* sW = base + 2 * kStemRegionBytes;            // resident weights, 4 k-blocks of [64 | 32 x 64] (128B swizzle)
-  uint8_t* sV = sW + kWBytes;                           // 2 x completed vertical max [112][64] bf16 (16B chunks XOR-swizzled)
-  uint64_t* a_full = reinterpret_cast<uint64_t*>(sV + 2 * kStemVBytes);   // PAIR: the leader's
+  uint8_t* sW = base + 2 * kStemRegionBytes;            // resident weights, 4 k-blocks of [32 x 64] (128B swizzle)
+  uint8_t* sV = sW + kStemWHalf;                        // 2 x completed vertical max [112][64] bf16 (16B chunks XOR-swizzled)
+  uint64_t* a_full = reinterpret_cast<uint64_t*>(sV + 2 * kStemVBytes);   // the leader's
   uint64_t* a_empty = a_full + 2;
-  uint64_t* w_full = a_empty + 2;                                          // PAIR: the leader's
+  uint64_t* w_full = a_empty + 2;                                          // the leader's
   uint64_t* tfull = w_full + 1;
-  uint64_t* tempty = tfull + 2;                                            // PAIR: the leader's
+  uint64_t* tempty = tfull + 2;                                            // the leader's
   uint64_t* v_full = tempty + 2;                                           // vertical max of a pooled row is in sV[buf]
   uint64_t* v_empty = v_full + 2;                                          // ... and has been pooled and stored
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(v_empty + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;
+  const uint32_t rank = ptx::cluster_ctarank();
   const bool leader = rank == 0;
   ptx::pdl_launch_dependents();
   if (threadIdx.x == 0) {
@@ -81,43 +79,34 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     ptx::prefetch_tensormap(&tmB);
     for (int s = 0; s < 2; s++) ptx::mbar_init(&a_full[s], 1), ptx::mbar_init(&a_empty[s], 1);
     ptx::mbar_init(w_full, 1);
-    for (int a = 0; a < 2; a++) ptx::mbar_init(&tfull[a], 1), ptx::mbar_init(&tempty[a], (PAIR ? 2 : 1) * kStemDrainWarps);
+    for (int a = 0; a < 2; a++) ptx::mbar_init(&tfull[a], 1), ptx::mbar_init(&tempty[a], 2 * kStemDrainWarps);
     for (int b = 0; b < 2; b++) ptx::mbar_init(&v_full[b], kStemDrainWarps), ptx::mbar_init(&v_empty[b], 4);
     ptx::fence_barrier_init();
   }
   if (warp == 1) {
-    if constexpr (PAIR) {
-      ptx::tmem_alloc2(tmem_slot, 128);
-      ptx::tmem_relinquish2();
-    } else {
-      ptx::tmem_alloc(tmem_slot, 128);
-      ptx::tmem_relinquish();
-    }
+    ptx::tmem_alloc2(tmem_slot, 128);
+    ptx::tmem_relinquish2();
   }
   ptx::tc_fence_before();
-  if constexpr (PAIR) ptx::cluster_sync_all();
-  else __syncthreads();
+  ptx::cluster_sync_all();
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   constexpr int BLOCKS_PER_IMG = 56 / kStemPB;
   if (warp == 0) {   // resident weights: constant data, loaded before the dependency wait
     if (ptx::elect_one()) {
-      if (leader) ptx::mbar_arrive_expect_tx(w_full, kStemWBytes);
-      for (int kb = 0; kb < 4; kb++) {
-        if constexpr (PAIR) ptx::tma2_load_2d(sW + kb * kWBlock, &tmB, w_full, kb * 64, (int)rank * 32);
-        else ptx::tma_load_2d(sW + kb * kWBlock, &tmB, w_full, kb * 64, 0);
-      }
+      if (leader) ptx::mbar_arrive_expect_tx(w_full, kStemWBytes);   // both CTAs' halves
+      for (int kb = 0; kb < 4; kb++) ptx::tma2_load_2d(sW + kb * kWBlock, &tmB, w_full, kb * 64, (int)rank * 32);
     }
     __syncwarp();
   }
   ptx::pdl_wait();
   const int num_blocks = effective_patches(p.n_dev, p.n_base, p.num_blocks / BLOCKS_PER_IMG) * BLOCKS_PER_IMG;
-  // work items: blocks (single CTA) or pairs of consecutive blocks; a phantom second block of an odd count re-reads the last
-  // real one and stores nothing
-  const int num_items = PAIR ? (num_blocks + 1) >> 1 : num_blocks;
-  const int item0 = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, item_step = PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  // work items: pairs of consecutive blocks; a phantom second block of an odd count re-reads the last real one and stores
+  // nothing
+  const int num_items = (num_blocks + 1) >> 1;
+  const int item0 = (int)(blockIdx.x >> 1), item_step = (int)(gridDim.x >> 1);
   auto block_of = [&](int it, bool& active) {
-    int b = PAIR ? 2 * it + (int)rank : it;
+    int b = 2 * it + (int)rank;
     active = b < num_blocks;
     if (!active) b = num_blocks - 1;
     return p.reverse ? num_blocks - 1 - b : b;
@@ -133,21 +122,16 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       const int img = vb / BLOCKS_PER_IMG, py0 = (vb - img * BLOCKS_PER_IMG) * kStemPB;
       ptx::mbar_wait(&a_empty[s], ph ^ 1);
       if (ptx::elect_one()) {
-        if constexpr (PAIR) {
-          if (leader) ptx::mbar_arrive_expect_tx(&a_full[s], 2 * kStemRegionLoad);
-          ptx::tma2_load_4d(sA + s * kStemRegionBytes, &tmA, &a_full[s], 0, 0, 2 * py0 - 3, img);
-        } else {
-          ptx::mbar_arrive_expect_tx(&a_full[s], kStemRegionLoad);
-          ptx::tma_load_4d(sA + s * kStemRegionBytes, &tmA, &a_full[s], 0, 0, 2 * py0 - 3, img);
-        }
+        if (leader) ptx::mbar_arrive_expect_tx(&a_full[s], 2 * kStemRegionLoad);
+        ptx::tma2_load_4d(sA + s * kStemRegionBytes, &tmA, &a_full[s], 0, 0, 2 * py0 - 3, img);
       }
       __syncwarp();
       if (++s == 2) s = 0, ph ^= 1;
     }
   } else if (warp == 1) {
-    // ===================== MMA issuer (PAIR: the leader's only) =====================
+    // ===================== MMA issuer (the leader's only) =====================
     if (leader) {
-      constexpr uint32_t idesc = ptx::make_idesc_bf16(PAIR ? 256 : 128, 64);
+      constexpr uint32_t idesc = ptx::make_idesc_bf16(256, 64);
       ptx::mbar_wait(w_full, 0);
       const uint64_t wdesc = ptx::make_smem_desc(ptx::smem_u32(sW), 128);
       int s = 0;
@@ -158,8 +142,8 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         ptx::mbar_wait(&a_full[s], ph);
         ptx::tc_fence_after();
         const uint64_t rdesc = ptx::make_smem_desc(ptx::smem_u32(sA + s * kStemRegionBytes), 32);
-        // conv row 2*py0 - 1 + t; row -1 does not exist: skipped by a single CTA, computed and dropped by a pair
-        for (int t = (!PAIR && py0 == 0 ? 1 : 0); t <= 2 * kStemPB; t++) {
+        // conv row 2*py0 - 1 + t; row -1 does not exist: computed and dropped
+        for (int t = 0; t <= 2 * kStemPB; t++) {
           ptx::mbar_wait(&tempty[acc], acc_phase ^ 1);
           ptx::tc_fence_after();
           const uint32_t d_tmem = tmem_base + acc * 64;
@@ -169,20 +153,15 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 #pragma unroll
               for (int b = 0; b < 4; b++) {
                 const uint64_t ad = rdesc + (uint64_t)(((t + a) * kS2dW + b) * 2), bd = wdesc + (uint64_t)(a * (kWBlock / 16) + b * 2);
-                if constexpr (PAIR) ptx::umma2_bf16(d_tmem, ad, bd, idesc, (a | b) != 0 ? 1u : 0u);
-                else ptx::umma_bf16(d_tmem, ad, bd, idesc, (a | b) != 0 ? 1u : 0u);
+                ptx::umma2_bf16(d_tmem, ad, bd, idesc, (a | b) != 0 ? 1u : 0u);
               }
-            if constexpr (PAIR) ptx::umma2_commit_mc(&tfull[acc]);
-            else ptx::umma_commit(&tfull[acc]);
+            ptx::umma2_commit_mc(&tfull[acc]);
           }
           __syncwarp();
           acc ^= 1;
           if (acc == 0) acc_phase ^= 1;
         }
-        if (ptx::elect_one()) {
-          if constexpr (PAIR) ptx::umma2_commit_mc(&a_empty[s]);
-          else ptx::umma_commit(&a_empty[s]);
-        }
+        if (ptx::elect_one()) ptx::umma2_commit_mc(&a_empty[s]);
         __syncwarp();
         if (++s == 2) s = 0, ph ^= 1;
       }
@@ -208,7 +187,7 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       bool active;
       const int py0 = (block_of(it, active) % BLOCKS_PER_IMG) * kStemPB;
       const int t_first = py0 == 0 ? 1 : 0;           // first existing conv row of the block: starts the running max
-      for (int t = (PAIR ? 0 : t_first); t <= 2 * kStemPB; t++) {
+      for (int t = 0; t <= 2 * kStemPB; t++) {
         const bool init = t == t_first;
         const bool closes = t > 0 && (t & 1) == 0;    // conv row 2*py + 1: pooled row py = py0 + t/2 - 1 is complete
         ptx::mbar_wait(&tfull[acc], acc_phase);
@@ -224,7 +203,7 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         }
         acc ^= 1;
         if (acc == 0) acc_phase ^= 1;
-        if (PAIR && t < t_first) continue;            // the pair's row "-1" of a top block
+        if (t < t_first) continue;                    // row "-1" of a top block
         __nv_bfloat162 cur[8];  // this pixel's 16 channels: + folded-BN bias (packed fp32 adds), bf16
 #pragma unroll
         for (int i = 0; i < 8; i++) {
@@ -298,11 +277,6 @@ k_conv1_pool(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     }
   }
   ptx::tc_fence_before();
-  if constexpr (PAIR) {
-    ptx::cluster_sync_all();
-    if (warp == 1) ptx::tmem_dealloc2(tmem_base, 128);
-  } else {
-    __syncthreads();
-    if (warp == 1) ptx::tmem_dealloc(tmem_base, 128);
-  }
+  ptx::cluster_sync_all();
+  if (warp == 1) ptx::tmem_dealloc2(tmem_base, 128);
 }

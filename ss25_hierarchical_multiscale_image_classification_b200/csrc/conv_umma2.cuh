@@ -1,6 +1,6 @@
 // The im2col implicit-GEMM kernel on CTA PAIRS (tcgen05 cta_group::2), BN = 256: layer3 and layer4, including their
 // stride-2 entry convolutions and the blocks with a fused 1x1 / stride-2 projection (extra K-blocks from a second im2col
-// map).  Included by resnet18.cu inside namespace hipac after k_conv_umma (shares ConvParams and epilogue_row).
+// map).  Included by resnet18.cu inside namespace hipac after ConvParams and epilogue_row.
 //
 // Why pairs here.  With one CTA per tile every 128-pixel tile re-streams the whole weight matrix through its ring: 32 KB of
 // weights + 16 KB of activations per 64-wide K-block.  A pair computes TWO pixel tiles against ONE copy of the weights:
@@ -14,14 +14,13 @@ template <int BN_>
 struct Conv2Cfg {
   static constexpr int BN = BN_;
   static constexpr int kBHalfBytes = (BN / 2) * 128;          // this CTA's half of one [BN x 64] weight block
-  static constexpr int kStage = kABytes + kBHalfBytes;        // 32 KB (BN = 256) / 24 KB (BN = 128)
-  static constexpr int kStages = BN == 256 ? 6 : 8;           // 192 KB in flight per SM
-  static constexpr int kTmemCols = 2 * BN;                    // BN = 256: the whole TMEM of both SMs
+  static constexpr int kStage = kABytes + kBHalfBytes;        // 32 KB
+  static constexpr int kStages = 6;                           // 192 KB in flight per SM
+  static constexpr int kTmemCols = 2 * BN;                    // the whole TMEM of both SMs
   static constexpr int kSmemBytes = kStages * kStage + 1024 + 256;
+  static_assert(BN == 256, "layer3 / layer4 only");
 };
 
-// BN = 128 serves layer2.0.conv1 (3x3 / stride 2, 64 -> 128): its single-CTA form keeps the weights resident and has room for
-// only 80 KB of activations in flight per SM, less than HBM latency x bandwidth.
 template <int BN>
 __global__ void __launch_bounds__(conv_threads(BN), 1)
 k_conv_umma2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,

@@ -8,7 +8,6 @@
 #include <cuda.h>
 
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <vector>
@@ -20,9 +19,9 @@
 namespace hipac {
 
 // ==========================================================================================
-// implicit-GEMM convolution kernel
+// what the convolution kernels (conv_*.cuh) share
 // ==========================================================================================
-struct ConvParams {
+struct ConvParams {   // the im2col kernel's (conv_umma2.cuh)
   int M_total;       // images * hout * wout (GEMM M)
   int hw_out, wout;  // hout*wout, wout
   int stride, pad_w, pad_h;
@@ -59,7 +58,6 @@ static thread_local int g_reverse = 0;
 constexpr int kBM = 128;
 constexpr int kS2dW = HIPAC_S2D16_WIDTH;  // 112 + 3 explicit zero columns (2 left, 1 right)
 constexpr int kABytes = kBM * 128;  // 128 rows x 64 bf16
-constexpr int kConvThreads = 192;   // warp 0: TMA producer, warp 1: MMA issuer + TMEM owner, warps 2-5: epilogue
 // 64-wide tiles have so little MMA work per tile that one epilogue warpgroup cannot keep up: they get two, which
 // take alternate tiles (= alternate TMEM accumulator buffers).  Wider tiles keep one (register budget).
 __host__ __device__ constexpr int epi_groups(int bn) { return bn == 64 ? 2 : 1; }
@@ -128,163 +126,7 @@ __device__ __forceinline__ void epilogue_row(uint32_t tmem_row, const float* __r
   }
 }
 
-// RESB: the whole weight matrix (<= kResBlocks k-blocks of [BN x 64]) stays resident in shared memory for the lifetime of the
-// persistent CTA and the ring carries the im2col A tiles only.  Used where it fits (layer2.0.conv1: 9 x 16 KB): the
-// streamed form re-reads 16 KB of weights from L2 per 16 KB of activations, which makes that layer L2-bandwidth bound.
-template <int BN, bool RESB = false>
-struct ConvCfg {
-  static constexpr int kBBytes = BN * 128;
-  static constexpr int kResBlocks = RESB ? 9 : 0;
-  static constexpr int kStage = RESB ? kABytes : kABytes + kBBytes;
-  static constexpr int kStages = RESB ? 5 : (BN == 256 ? 4 : 6);
-  static constexpr int kTmemCols = 2 * BN;
-  static constexpr int kSmemBytes = kStages * kStage + kResBlocks * kBBytes + 1024 /*alignment slack*/ + 256 /*barriers*/;
-  static_assert(kSmemBytes <= 232448, "shared memory budget");
-};
-
-template <int BN, bool RESB = false>
-__global__ void __launch_bounds__(conv_threads(BN), 1)
-k_conv_umma(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-            const __grid_constant__ CUtensorMap tmA2, const ConvParams p) {
-  using Cfg = ConvCfg<BN, RESB>;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* resB = base + Cfg::kStages * Cfg::kStage;
-  uint64_t* full = reinterpret_cast<uint64_t*>(resB + Cfg::kResBlocks * Cfg::kBBytes);
-  uint64_t* empty = full + Cfg::kStages;
-  uint64_t* tfull = empty + Cfg::kStages;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* b_full = tempty + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(b_full + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  ptx::pdl_launch_dependents();
-  if (threadIdx.x == 0) {
-    ptx::prefetch_tensormap(&tmA);
-    ptx::prefetch_tensormap(&tmB);
-    if (p.num_kb2) ptx::prefetch_tensormap(&tmA2);
-    for (int s = 0; s < Cfg::kStages; s++) ptx::mbar_init(&full[s], 1), ptx::mbar_init(&empty[s], 1);
-    for (int a = 0; a < 2; a++) ptx::mbar_init(&tfull[a], 1), ptx::mbar_init(&tempty[a], 4);
-    ptx::mbar_init(b_full, 1);
-    ptx::fence_barrier_init();
-  }
-  if (warp == 1) {
-    ptx::tmem_alloc(tmem_slot, Cfg::kTmemCols);
-    ptx::tmem_relinquish();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  if (RESB && warp == 0) {   // resident weights: constant data, loaded before the dependency wait
-    if (ptx::elect_one()) {
-      ptx::mbar_arrive_expect_tx(b_full, (uint32_t)(p.num_kb * Cfg::kBBytes));
-      for (int kb = 0; kb < p.num_kb; kb++) ptx::tma_load_2d(resB + kb * Cfg::kBBytes, &tmB, b_full, kb * 64, 0);
-    }
-    __syncwarp();
-  }
-  ptx::pdl_wait();           // the producer kernel's activations (and the device-side patch count) are visible from here on
-  const int M_total = effective_patches(p.n_dev, p.n_base, p.M_total / p.hw_out) * p.hw_out;
-  const int num_tiles = ((M_total + kBM - 1) / kBM) * p.num_n_tiles;
-
-  if (warp == 0) {
-    // ===================== TMA producer =====================
-    // The whole warp runs the loop with warp-uniform values (descriptors and coordinates then live in uniform
-    // registers); one elected lane issues the TMA instructions.
-    {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int vt = p.reverse ? num_tiles - 1 - tile : tile;
-        const int m_tile = vt / p.num_n_tiles, n_tile = vt - m_tile * p.num_n_tiles;
-        const int m0 = m_tile * kBM;
-        const int img = m0 / p.hw_out, rem = m0 - img * p.hw_out;
-        const int p0 = rem / p.wout, q0 = rem - p0 * p.wout;
-        const int cw = q0 * p.stride - p.pad_w, ch = p0 * p.stride - p.pad_h;
-        for (int kb = 0; kb < p.num_kb + p.num_kb2; kb++) {
-          ptx::mbar_wait(&empty[stage], phase ^ 1);
-          uint8_t* a_dst = base + stage * Cfg::kStage;
-          uint8_t* b_dst = a_dst + kABytes;
-          const int tap = kb / p.kc_blocks, kc = kb - tap * p.kc_blocks;
-          const int r = tap / p.kw, s = tap - r * p.kw;
-          if (ptx::elect_one()) {
-            ptx::mbar_arrive_expect_tx(&full[stage], Cfg::kStage);
-            if (kb < p.num_kb)
-              ptx::tma_load_im2col_4d(a_dst, &tmA, &full[stage], kc * 64, cw, ch, img, (uint16_t)s, (uint16_t)r);
-            else  // fused projection shortcut: 1x1 / stride2 / pad 0 over the block input, channels (kb - num_kb) * 64
-              ptx::tma_load_im2col_4d(a_dst, &tmA2, &full[stage], (kb - p.num_kb) * 64, q0 * p.stride2, p0 * p.stride2, img, 0, 0);
-            if (!RESB) ptx::tma_load_2d(b_dst, &tmB, &full[stage], kb * 64, n_tile * BN);
-          }
-          __syncwarp();
-          if (++stage == Cfg::kStages) stage = 0, phase ^= 1;
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer =====================
-    // Warp-uniform loop; one elected lane (always the same one) issues the UMMAs and their commits.
-    {
-      constexpr uint32_t idesc = ptx::make_idesc_bf16(kBM, BN);
-      int stage = 0;
-      uint32_t phase = 0, acc = 0, acc_phase = 0;
-      if (RESB) ptx::mbar_wait(b_full, 0);
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        ptx::mbar_wait(&tempty[acc], acc_phase ^ 1);  // epilogue has drained this accumulator
-        ptx::tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
-        for (int kb = 0; kb < p.num_kb + p.num_kb2; kb++) {
-          ptx::mbar_wait(&full[stage], phase);
-          ptx::tc_fence_after();
-          const uint32_t a_addr = ptx::smem_u32(base + stage * Cfg::kStage);
-          const uint64_t adesc = ptx::make_smem_desc(a_addr, 128);
-          const uint64_t bdesc = ptx::make_smem_desc(RESB ? ptx::smem_u32(resB + kb * Cfg::kBBytes) : a_addr + kABytes, 128);
-          if (ptx::elect_one()) {
-#pragma unroll
-            for (int k = 0; k < 4; k++)  // 4 x (K = 16) per 64-wide k-block: +32 B = +2 in the descriptor's address field
-              ptx::umma_bf16(d_tmem, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
-            ptx::umma_commit(&empty[stage]);  // smem slot reusable once these MMAs retire
-          }
-          __syncwarp();
-          if (++stage == Cfg::kStages) stage = 0, phase ^= 1;
-        }
-        if (ptx::elect_one()) ptx::umma_commit(&tfull[acc]);  // accumulator complete -> epilogue
-        __syncwarp();
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1;
-      }
-    }
-  } else {
-    // ===================== epilogue: TMEM -> +bias (+residual) -> ReLU -> bf16 NHWC =====================
-    const int wq = warp & 3;  // TMEM lane quarter this warp may access
-    const int row = wq * 32 + lane;
-    const int grp = (warp - 2) >> 2;
-    int it = 0;
-    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
-      if (epi_groups(BN) == 2 && (it & 1) != grp) continue;
-      const uint32_t acc = it & 1, acc_phase = (it >> 1) & 1;
-      const int vt = p.reverse ? num_tiles - 1 - tile : tile;
-      const int m_tile = vt / p.num_n_tiles, n_tile = vt - m_tile * p.num_n_tiles;
-      const int m = m_tile * kBM + row;
-      const bool valid = m < M_total;
-      {
-        const size_t off = (size_t)m * p.cout + (size_t)n_tile * BN;
-        epilogue_row<BN>(tmem_base + ((uint32_t)(wq * 32) << 16) + acc * BN, p.bias + n_tile * BN,
-                         p.residual ? p.residual + off : nullptr, p.out + off, p.relu, valid, &tfull[acc], acc_phase);
-      }
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&tempty[acc]);
-    }
-  }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 1) ptx::tmem_dealloc(tmem_base, Cfg::kTmemCols);
-}
-
 #include "conv_umma2.cuh"
-#include "conv_rows.cuh"
-#include "conv_rows_tma.cuh"
 #include "conv_rows2.cuh"
 #include "conv_rows2_s2.cuh"
 #include "conv_stem.cuh"
@@ -292,41 +134,6 @@ k_conv_umma(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 // ==========================================================================================
 // small memory-bound kernels
 // ==========================================================================================
-// MaxPool 3x3 / stride 2 / pad 1 on bf16 NHWC [n,112,112,64] -> [n,56,56,64]; 8 channels per thread.
-__global__ void __launch_bounds__(256) k_maxpool(const __nv_bfloat16* __restrict__ in, __nv_bfloat16* __restrict__ out,
-                                                 int n_img) {
-  const int64_t total = (int64_t)n_img * 56 * 56 * 8;
-  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
-    const int cg = (int)(t & 7);
-    int64_t pix = t >> 3;
-    const int ox = (int)(pix % 56);
-    pix /= 56;
-    const int oy = (int)(pix % 56);
-    const int img = (int)(pix / 56);
-    __nv_bfloat162 m[4];
-    bool first = true;
-#pragma unroll
-    for (int dy = -1; dy <= 1; dy++) {
-      const int iy = 2 * oy + dy;
-      if (iy < 0 || iy >= 112) continue;
-#pragma unroll
-      for (int dx = -1; dx <= 1; dx++) {
-        const int ix = 2 * ox + dx;
-        if (ix < 0 || ix >= 112) continue;
-        const uint4 v = __ldg(reinterpret_cast<const uint4*>(in + (((int64_t)img * 112 + iy) * 112 + ix) * 64 + cg * 8));
-        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v);
-        if (first) {
-          m[0] = h[0], m[1] = h[1], m[2] = h[2], m[3] = h[3];
-          first = false;
-        } else {
-          m[0] = __hmax2(m[0], h[0]), m[1] = __hmax2(m[1], h[1]), m[2] = __hmax2(m[2], h[2]), m[3] = __hmax2(m[3], h[3]);
-        }
-      }
-    }
-    *reinterpret_cast<uint4*>(out + (((int64_t)img * 56 + oy) * 56 + ox) * 64 + cg * 8) = *reinterpret_cast<uint4*>(m);
-  }
-}
-
 // Global average pool over 7x7 (fp32 accumulate) + optional Linear(512,k) in fp32. One CTA per patch.
 __global__ void __launch_bounds__(256) k_avgpool_fc(const __nv_bfloat16* __restrict__ in, float* __restrict__ feats,
                                                     float* __restrict__ logits, const float* __restrict__ fc_w,
@@ -394,40 +201,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 static EncodeIm2colFn g_encode_im2col = nullptr;
 static EncodeTiledFn g_encode_tiled = nullptr;
 static thread_local int g_num_sms = 0;   // SM count of the CURRENT device, refreshed by init_driver_api() on every entry
-static bool g_use_fused_stem = true;   // HIPAC_FUSED_STEM=0 runs conv1 and the max pool as two kernels
-static bool g_fuse_downsample = true; // HIPAC_FUSE_DS=0 runs the 1x1 projection shortcuts as separate kernels
-static bool g_use_row_kernels = true;  // HIPAC_CONV_ROWS=0 forces the im2col kernel everywhere (A/B comparison)
-static bool g_use_cta_pairs = true;    // HIPAC_CTA_PAIRS=0: single-CTA row kernels instead of the cta_group::2 ones
-static bool g_use_cta_pairs_stem = true;   // HIPAC_CTA_PAIRS_STEM=0: the fused stem on single CTAs
-static bool g_use_cta_pairs_c128_im2col = false;  // HIPAC_CTA_PAIRS_C128_IM2COL=1: layer2.0.conv1 on CTA pairs instead of a single CTA with resident weights (measured 2 % slower)
-static bool g_use_s2_rows = true;          // HIPAC_S2_ROWS=0: layer2.0.conv1 through im2col (k_conv_umma<128, RESB>)
-static bool g_use_cta_pairs_c256 = true;   // HIPAC_CTA_PAIRS_C256=0: layer3 / layer4 on single CTAs (k_conv_umma<256>)
-static bool g_resident_weights = true; // HIPAC_RESIDENT_B=0: the im2col kernel streams the weights of layer2.0.conv1 like everywhere else
-static bool g_tma_epilogue_c128 = true;   // HIPAC_TMA_EPILOGUE_C128=0: the 128-channel residual layer keeps per-thread stores / residual loads
-static bool g_tma_epilogue = true;     // HIPAC_TMA_EPILOGUE=0: 64-channel layers store / fetch the residual per thread (k_conv3x3_rows)
-static bool g_use_cta_pairs_c64 = true;   // HIPAC_CTA_PAIRS_C64=0: layer1 on single CTAs (k_conv3x3_rows_tma)
-
-// A/B switches for measurements; read once (the workspace size depends on them).
-static bool g_boustrophedon = true;   // alternate the tile order from layer to layer (A/B switch: HIPAC_BOUSTROPHEDON=0)
-static void read_env_flags() {
-  static std::once_flag once;
-  std::call_once(once, [] {
-    if (const char* e = getenv("HIPAC_CONV_ROWS")) g_use_row_kernels = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_CTA_PAIRS")) g_use_cta_pairs = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_CTA_PAIRS_C64")) g_use_cta_pairs_c64 = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_TMA_EPILOGUE")) g_tma_epilogue = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_RESIDENT_B")) g_resident_weights = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_CTA_PAIRS_C256")) g_use_cta_pairs_c256 = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_CTA_PAIRS_STEM")) g_use_cta_pairs_stem = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_S2_ROWS")) g_use_s2_rows = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_CTA_PAIRS_C128_IM2COL")) g_use_cta_pairs_c128_im2col = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_TMA_EPILOGUE_C128")) g_tma_epilogue_c128 = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_FUSED_STEM")) g_use_fused_stem = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_FUSE_DS")) g_fuse_downsample = atoi(e) != 0;
-    if (const char* e = getenv("HIPAC_BOUSTROPHEDON")) g_boustrophedon = atoi(e) != 0;
-  });
-}
-
 // Called at the top of every entry point: driver entry points once per process, the SM count for the CURRENT device.
 static int init_driver_api() {
   static std::mutex mu;
@@ -444,9 +217,7 @@ static int init_driver_api() {
       g_encode_tiled = (EncodeTiledFn)fn;
     }
   }
-  if (int e = device_sm_count(&g_num_sms)) return e;
-  read_env_flags();
-  return 0;
+  return device_sm_count(&g_num_sms);
 }
 
 // NHWC activation tensor [n][h][w][c] (bf16) as an im2col map: box = 128 output pixels x `chan_box` channels.
@@ -510,30 +281,6 @@ static int make_region_map(CUtensorMap* map, const void* ptr, int n, int h, int 
   return 0;
 }
 
-template <int BN, int KC, int W, int R, bool RESIDENT>
-static int launch_rows_t(const uint8_t* d_packed, const PackedLayout& L, int layer, const void* in, const void* residual, void* out,
-                         int n, bool relu, cudaStream_t stream, const char* name) {
-  using Cfg = RowCfg<BN, KC, W, R, RESIDENT>;
-  if (int e = ensure_dyn_smem(k_conv3x3_rows<BN, KC, W, R, RESIDENT>, Cfg::kSmemBytes)) return e;
-  CUtensorMap tmA, tmB;
-  if (int e = make_region_map(&tmA, in, n, W, W, KC * 64, R)) return e;
-  if (int e = make_weight_map(&tmB, d_packed + L.w_off[layer], BN, 9 * KC * 64, BN)) return e;
-  RowConvParams p;
-  p.n_img = n, p.num_tiles = n * (W / R), p.relu = relu ? 1 : 0;
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
-  p.bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
-  p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
-  p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  const int grid = p.num_tiles < g_num_sms ? p.num_tiles : g_num_sms;
-  {
-    ProfileScope ps(name, stream, 2.0 * n * W * W * BN * 9 * KC * 64);
-    k_conv3x3_rows<BN, KC, W, R, RESIDENT><<<grid, conv_threads(BN), Cfg::kSmemBytes, stream>>>(tmA, tmB, p);
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
-  return 0;
-}
-
 // NHWC activation tensor as a strided tiled map for the fused 1x1 / stride-2 projection: the box spans 2*wp x 2*r input
 // pixels with element strides 2, i.e. delivers wp x r pixels x 64 channels (out-of-range pixels zero filled).
 static int make_strided_map(CUtensorMap* map, const void* ptr, int n, int h, int w, int c, int wp, int r) {
@@ -565,38 +312,6 @@ static int make_tile_map(CUtensorMap* map, const void* ptr, int n, int h, int w,
     set_error("cuTensorMapEncodeTiled (tile map) failed with CUresult " + std::to_string((int)res));
     return -5;
   }
-  return 0;
-}
-
-// 64-channel row kernel with the TMA epilogue (conv_rows_tma.cuh).
-template <int KC, int W, int R>
-static int launch_rows_tma_t(const uint8_t* d_packed, const PackedLayout& L, int layer, const void* in, const void* residual, void* out,
-                             int n, bool relu, cudaStream_t stream, const char* name) {
-  using Cfg = RowTmaCfg<KC, W, R>;
-  if (int e = ensure_dyn_smem(k_conv3x3_rows_tma<KC, W, R>, Cfg::kSmemBytes)) return e;
-  CUtensorMap tmA, tmB, tmO, tmR;
-  if (int e = make_region_map(&tmA, in, n, W, W, KC * 64, R)) return e;
-  if (int e = make_weight_map(&tmB, d_packed + L.w_off[layer], 64, 9 * KC * 64, 64)) return e;
-  if (int e = make_tile_map(&tmO, out, n, W, W, 64, R)) return e;
-  if (residual) {
-    if (int e = make_tile_map(&tmR, residual, n, W, W, 64, R)) return e;
-  } else {
-    tmR = tmO;
-  }
-  RowConvParams p;
-  p.n_img = n, p.num_tiles = n * (W / R), p.relu = relu ? 1 : 0;
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
-  p.bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
-  p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
-  p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  const int grid = p.num_tiles < g_num_sms ? p.num_tiles : g_num_sms;
-  {
-    ProfileScope ps(name, stream, 2.0 * n * W * W * 64 * 9 * KC * 64);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv3x3_rows_tma<KC, W, R>, dim3(grid), dim3(conv_threads(64)), Cfg::kSmemBytes, stream, 1, true, tmA, tmB, tmO,
-                               tmR, p));
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -634,7 +349,7 @@ static int launch_rows2_t(const void* w_ptr, const float* bias, const void* in, 
   {
     ProfileScope ps(name, stream, flops);
     HIPAC_CHECK_CUDA(launch_ex(k_conv3x3_rows2<BN, KC, W, R, KDS, TEPI>, dim3((unsigned)grid), dim3((unsigned)conv_threads(BN)), Cfg::kSmemBytes,
-                               stream, 2, true, tmA, tmB, tmA2, tmO, tmR, p));
+                               stream, 2, tmA, tmB, tmA2, tmO, tmR, p));
   }
   count_launch(1);
   HIPAC_CHECK_CUDA(cudaGetLastError());
@@ -658,7 +373,7 @@ static int launch_rows2_s2(const void* w_ptr, const float* bias, const void* in,
   const int grid = 2 * (pairs < max_pairs ? pairs : max_pairs);
   {
     ProfileScope ps(name, stream, flops);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv3x3s2_rows2, dim3((unsigned)grid), dim3((unsigned)conv_threads(128)), Cfg::kSmemBytes, stream, 2, true, tmE,
+    HIPAC_CHECK_CUDA(launch_ex(k_conv3x3s2_rows2, dim3((unsigned)grid), dim3((unsigned)conv_threads(128)), Cfg::kSmemBytes, stream, 2, tmE,
                                tmO, tmB, p));
   }
   count_launch(1);
@@ -666,10 +381,9 @@ static int launch_rows2_s2(const void* w_ptr, const float* bias, const void* in,
   return 0;
 }
 
-// Fused conv1 + BN + ReLU + maxpool on the S2D16 batch -> [n][56][56][64].
+// Fused conv1 + BN + ReLU + maxpool on the S2D16 batch -> [n][56][56][64], on CTA pairs (conv_stem.cuh).
 static int run_stem(const uint8_t* d_packed, const PackedLayout& L, const void* in, void* out, int n, cudaStream_t stream) {
-  const bool pair = g_use_cta_pairs && g_use_cta_pairs_stem;
-  if (int e = pair ? ensure_dyn_smem(k_conv1_pool<true>, kStemSmemPair) : ensure_dyn_smem(k_conv1_pool<false>, kStemSmem)) return e;
+  if (int e = ensure_dyn_smem(k_conv1_pool, kStemSmem)) return e;
   CUtensorMap tmA, tmB;
   {
     cuuint64_t dims[4] = {16, (cuuint64_t)kS2dW, 112, (cuuint64_t)n};
@@ -684,55 +398,34 @@ static int run_stem(const uint8_t* d_packed, const PackedLayout& L, const void* 
       return -5;
     }
   }
-  if (int e = make_weight_map(&tmB, d_packed + L.w_off[0], 64, 256, pair ? 32 : 64)) return e;
+  if (int e = make_weight_map(&tmB, d_packed + L.w_off[0], 64, 256, 32)) return e;
   StemParams p;
   p.num_blocks = n * (56 / kStemPB);
   p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
   p.bias = reinterpret_cast<const float*>(d_packed + L.b_off[0]);
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  const int items = pair ? (p.num_blocks + 1) / 2 : p.num_blocks, slots = pair ? g_num_sms / 2 : g_num_sms;
-  const int grid = (pair ? 2 : 1) * (items < slots ? items : slots);
+  const int pairs = (p.num_blocks + 1) / 2, max_pairs = g_num_sms / 2;
+  const int grid = 2 * (pairs < max_pairs ? pairs : max_pairs);
   {
     ProfileScope ps("conv1_pool_fused", stream, 2.0 * n * 112 * 112 * 64 * 147);
-    if (pair)
-      HIPAC_CHECK_CUDA(launch_ex(k_conv1_pool<true>, dim3(grid), dim3(kStemThreads), kStemSmemPair, stream, 2, true, tmA, tmB, p));
-    else
-      HIPAC_CHECK_CUDA(launch_ex(k_conv1_pool<false>, dim3(grid), dim3(kStemThreads), kStemSmem, stream, 1, true, tmA, tmB, p));
+    HIPAC_CHECK_CUDA(launch_ex(k_conv1_pool, dim3(grid), dim3(kStemThreads), kStemSmem, stream, 2, tmA, tmB, p));
   }
   count_launch(1);
   HIPAC_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
-template <int BN, bool RESB = false>
-static int launch_conv_t(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvParams& p, cudaStream_t stream,
-                         const char* name, double flops, const CUtensorMap* tmA2 = nullptr) {
-  using Cfg = ConvCfg<BN, RESB>;
-  if (int e = ensure_dyn_smem(k_conv_umma<BN, RESB>, Cfg::kSmemBytes)) return e;
-  const int tiles = p.num_m_tiles * p.num_n_tiles;
-  const int grid = tiles < g_num_sms ? tiles : g_num_sms;
-  {
-    ProfileScope ps(name, stream, flops);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv_umma<BN, RESB>, dim3(grid), dim3(conv_threads(BN)), Cfg::kSmemBytes, stream, 1, true, tmA, tmB,
-                               tmA2 ? *tmA2 : tmA, p));
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
-  return 0;
-}
-
-// im2col layers on CTA pairs (conv_umma2.cuh); tmB must have been built with a box of BN/2 weight rows.
-template <int BN>
+// im2col layers on CTA pairs (conv_umma2.cuh); tmB must have been built with a box of 128 weight rows.
 static int launch_conv2(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvParams& p, cudaStream_t stream, const char* name,
                         double flops, const CUtensorMap* tmA2 = nullptr) {
-  using Cfg = Conv2Cfg<BN>;
-  if (int e = ensure_dyn_smem(k_conv_umma2<BN>, Cfg::kSmemBytes)) return e;
+  using Cfg = Conv2Cfg<256>;
+  if (int e = ensure_dyn_smem(k_conv_umma2<256>, Cfg::kSmemBytes)) return e;
   const int ptiles = ((p.num_m_tiles + 1) / 2) * p.num_n_tiles;
   const int max_pairs = g_num_sms / 2;
   const int grid = 2 * (ptiles < max_pairs ? ptiles : max_pairs);
   {
     ProfileScope ps(name, stream, flops);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv_umma2<BN>, dim3((unsigned)grid), dim3((unsigned)conv_threads(BN)), Cfg::kSmemBytes, stream, 2, true, tmA,
+    HIPAC_CHECK_CUDA(launch_ex(k_conv_umma2<256>, dim3((unsigned)grid), dim3((unsigned)conv_threads(256)), Cfg::kSmemBytes, stream, 2, tmA,
                                tmB, tmA2 ? *tmA2 : tmA, p));
   }
   count_launch(1);
@@ -740,74 +433,47 @@ static int launch_conv2(const CUtensorMap& tmA, const CUtensorMap& tmB, const Co
   return 0;
 }
 
-// One conv layer of the network on `n` patches. in/out are bf16 NHWC (layer 0: S2D16 input).
+// One conv layer of the network on `n` patches, bf16 NHWC in / out.  Not for layer 0 (conv1, which exists only fused with
+// the max pool: run_stem) or layer 7 (layer2.0's projection shortcut, which exists only fused: run_conv_ds_fused).
 static int run_conv(const uint8_t* d_packed, const PackedLayout& L, int layer, const void* in, const void* residual, void* out,
                     int n, bool relu, cudaStream_t stream) {
   const ConvSpec& cs = kConvs[layer];
-  const int K = conv_gemm_k(layer);
-  if (g_use_row_kernels && g_use_cta_pairs && g_use_s2_rows && cs.k == 3 && cs.stride == 2 && cs.cin == 64 && cs.cout == 128 && cs.hin == 56 &&
-      residual == nullptr)
-    return launch_rows2_s2(d_packed + L.w_off[layer], reinterpret_cast<const float*>(d_packed + L.b_off[layer]), in, out, n, relu, stream,
-                           "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 576);
-  if (g_use_row_kernels && cs.k == 3 && cs.stride == 1) {
-    const float* bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
-    if (cs.cin == 64 && cs.hin == 56) {
-      if (g_use_cta_pairs && g_use_cta_pairs_c64)
-        return launch_rows2_t<64, 1, 56, 2, 0>(d_packed + L.w_off[layer], bias, in, nullptr, residual, out, n, relu, stream, "conv3x3_c64",
-                                               2.0 * n * 56 * 56 * 64 * 576);
-      if (g_tma_epilogue) return launch_rows_tma_t<1, 56, 2>(d_packed, L, layer, in, residual, out, n, relu, stream, "conv3x3_c64");
-      return launch_rows_t<64, 1, 56, 2, true>(d_packed, L, layer, in, residual, out, n, relu, stream, "conv3x3_c64");
-    }
-    if (cs.cin == 128 && cs.hin == 28) {
-      if (g_use_cta_pairs && residual && g_tma_epilogue_c128)   // the residual variant: staged epilogue (see conv_rows2.cuh)
-        return launch_rows2_t<128, 2, 28, 4, 0, true>(d_packed + L.w_off[layer], bias, in, nullptr, residual, out, n, relu, stream,
-                                                      "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 1152);
-      if (g_use_cta_pairs)
-        return launch_rows2_t<128, 2, 28, 4, 0>(d_packed + L.w_off[layer], bias, in, nullptr, residual, out, n, relu, stream, "conv3x3_c128",
-                                                2.0 * n * 28 * 28 * 128 * 1152);
-      return launch_rows_t<128, 2, 28, 4, false>(d_packed, L, layer, in, residual, out, n, relu, stream, "conv3x3_c128");
-    }
+  const uint8_t* w = d_packed + L.w_off[layer];
+  const float* bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
+  if (cs.cout == 64)   // layer1: 3x3 / s1 at 56x56
+    return launch_rows2_t<64, 1, 56, 2, 0>(w, bias, in, nullptr, residual, out, n, relu, stream, "conv3x3_c64", 2.0 * n * 56 * 56 * 64 * 576);
+  if (cs.cout == 128 && cs.stride == 2) {   // layer2.0.conv1: 3x3 / s2, 64 -> 128
+    HIPAC_REQUIRE(residual == nullptr, "layer2.0.conv1 takes no residual");
+    return launch_rows2_s2(w, bias, in, out, n, relu, stream, "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 576);
   }
+  if (cs.cout == 128) {   // layer2: 3x3 / s1 at 28x28; the residual variant has the staged epilogue (see conv_rows2.cuh)
+    if (residual)
+      return launch_rows2_t<128, 2, 28, 4, 0, true>(w, bias, in, nullptr, residual, out, n, relu, stream, "conv3x3_c128",
+                                                    2.0 * n * 28 * 28 * 128 * 1152);
+    return launch_rows2_t<128, 2, 28, 4, 0>(w, bias, in, nullptr, nullptr, out, n, relu, stream, "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 1152);
+  }
+  // layer3 / layer4: im2col on CTA pairs
+  const int K = conv_gemm_k(layer);
   ConvParams p;
   p.M_total = n * cs.hout * cs.hout;
   p.hw_out = cs.hout * cs.hout, p.wout = cs.hout;
   p.cout = cs.cout;
   p.relu = relu ? 1 : 0;
-  p.bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
+  p.bias = bias;
   p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
   p.num_m_tiles = (p.M_total + kBM - 1) / kBM;
   p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
   p.num_kb2 = 0, p.stride2 = 1;
-  const int bn = cs.cout >= 256 ? 256 : (cs.cout >= 128 ? 128 : 64);
-  p.num_n_tiles = cs.cout / bn;
-  const bool pairs256 = bn >= 128 && layer != 0 && g_use_cta_pairs && (bn == 256 ? g_use_cta_pairs_c256 : g_use_cta_pairs_c128_im2col);
-  CUtensorMap tmA, tmB;
-  if (int e = make_weight_map(&tmB, d_packed + L.w_off[layer], cs.cout, K, pairs256 ? bn / 2 : bn)) return e;
-  if (layer == 0) {
-    // 7x7/s2/p3 over 3 channels == 4x4/s1 over the 2x2 space-to-depth image (16 ch), pad 2 before / 1 after.
-    // The S2D16 batch stores the W padding explicitly ([n][112][115][16], zero columns 0,1,114), so the four
-    // W-taps of one filter row are 64 CONTIGUOUS bf16: the conv is a 4x1 filter over a 64-"channel" view whose
-    // pixel stride (32 B) is smaller than its channel extent (128 B).  H padding stays TMA zero fill.
-    p.stride = 1, p.pad_w = 0, p.pad_h = 2, p.kw = 1, p.kc_blocks = 1, p.num_kb = 4;
-    Im2colDesc d{n, 112, 112, 64, 32, (int64_t)kS2dW * 32, (int64_t)112 * kS2dW * 32, 4, 1, 1, 0, 0, 2, 1};
-    if (int e = make_im2col_map(&tmA, in, d)) return e;
-    return launch_conv_t<64>(tmA, tmB, p, stream, "conv1_7x7s2_c64", 2.0 * p.M_total * 64 * 147);
-  }
+  p.num_n_tiles = cs.cout / 256;
   p.stride = cs.stride, p.pad_w = p.pad_h = cs.pad, p.kw = cs.k, p.kc_blocks = cs.cin / 64, p.num_kb = cs.k * cs.k * p.kc_blocks;
+  CUtensorMap tmA, tmB;
+  if (int e = make_weight_map(&tmB, w, cs.cout, K, 128)) return e;
   Im2colDesc d{n, cs.hin, cs.hin, cs.cin, (int64_t)cs.cin * 2, (int64_t)cs.hin * cs.cin * 2, (int64_t)cs.hin * cs.hin * cs.cin * 2,
                cs.k, cs.k, cs.stride, cs.pad, cs.pad, cs.pad, cs.pad};
   if (int e = make_im2col_map(&tmA, in, d)) return e;
-  static const char* kNames[4][2] = {{"conv3x3_c64", "conv1x1_c64"}, {"conv3x3_c128", "conv1x1_c128"},
-                                     {"conv3x3_c256", "conv1x1_c256"}, {"conv3x3_c512", "conv1x1_c512"}};
-  const int gi = cs.cout == 64 ? 0 : cs.cout == 128 ? 1 : cs.cout == 256 ? 2 : 3;
-  const char* name = kNames[gi][cs.k == 1 ? 1 : 0];
-  const double flops = 2.0 * p.M_total * cs.cout * K;
-  if (pairs256) return bn == 256 ? launch_conv2<256>(tmA, tmB, p, stream, name, flops) : launch_conv2<128>(tmA, tmB, p, stream, name, flops);
-  if (bn == 256) return launch_conv_t<256>(tmA, tmB, p, stream, name, flops);
-  if (bn == 128 && g_resident_weights && p.num_n_tiles == 1 && p.num_kb <= ConvCfg<128, true>::kResBlocks)
-    return launch_conv_t<128, true>(tmA, tmB, p, stream, name, flops);      // layer2.0.conv1: the 144 KB of weights stay in shared memory
-  return bn == 128 ? launch_conv_t<128>(tmA, tmB, p, stream, name, flops) : launch_conv_t<64>(tmA, tmB, p, stream, name, flops);
+  static const char* kNames[2][2] = {{"conv3x3_c256", "conv1x1_c256"}, {"conv3x3_c512", "conv1x1_c512"}};
+  return launch_conv2(tmA, tmB, p, stream, kNames[cs.cout == 512][cs.k == 1], 2.0 * p.M_total * cs.cout * K);
 }
 
 // conv2 of a stage's first block with its projection shortcut fused: out = relu(conv3x3(in) + conv1x1_s2(block_in) + bias).
@@ -816,11 +482,12 @@ static int run_conv_ds_fused(const uint8_t* d_packed, const PackedLayout& L, int
                              int n, cudaStream_t stream) {
   const int lc = fused_conv_layer(s), ld = fused_ds_layer(s);
   const ConvSpec &cs = kConvs[lc], &ds = kConvs[ld];
-  if (s == 0 && g_use_row_kernels && g_use_cta_pairs) {
+  if (s == 0) {
     // layer2.0: 3x3 128 -> 128 at 28x28 + 1x1/s2 64 -> 128 from the 56x56 block input, on CTA pairs with resident weights
     return launch_rows2_t<128, 2, 28, 4, 1>(d_packed + L.wf_off[0], reinterpret_cast<const float*>(d_packed + L.bf_off[0]), in, block_in,
                                             nullptr, out, n, true, stream, "conv3x3+ds_c128", 2.0 * n * 28 * 28 * 128 * fused_gemm_k(0));
   }
+  // layer3.0 / layer4.0: im2col on CTA pairs, the shortcut from a second im2col map
   ConvParams p;
   p.M_total = n * cs.hout * cs.hout;
   p.hw_out = cs.hout * cs.hout, p.wout = cs.hout;
@@ -830,13 +497,11 @@ static int run_conv_ds_fused(const uint8_t* d_packed, const PackedLayout& L, int
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
   p.num_m_tiles = (p.M_total + kBM - 1) / kBM;
   p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
-  const int bn = cs.cout >= 256 ? 256 : 128;
-  p.num_n_tiles = cs.cout / bn;
+  p.num_n_tiles = cs.cout / 256;
   p.stride = 1, p.pad_w = p.pad_h = 1, p.kw = 3, p.kc_blocks = cs.cin / 64, p.num_kb = 9 * p.kc_blocks;
   p.num_kb2 = ds.cin / 64, p.stride2 = 2;
-  const bool pairs256 = bn == 256 && g_use_cta_pairs && g_use_cta_pairs_c256;
   CUtensorMap tmA, tmA2, tmB;
-  if (int e = make_weight_map(&tmB, d_packed + L.wf_off[s], cs.cout, fused_gemm_k(s), pairs256 ? bn / 2 : bn)) return e;
+  if (int e = make_weight_map(&tmB, d_packed + L.wf_off[s], cs.cout, fused_gemm_k(s), 128)) return e;
   Im2colDesc d{n, cs.hin, cs.hin, cs.cin, (int64_t)cs.cin * 2, (int64_t)cs.hin * cs.cin * 2, (int64_t)cs.hin * cs.hin * cs.cin * 2,
                3, 3, 1, 1, 1, 1, 1};
   if (int e = make_im2col_map(&tmA, in, d)) return e;
@@ -844,10 +509,7 @@ static int run_conv_ds_fused(const uint8_t* d_packed, const PackedLayout& L, int
                 1, 1, 2, 0, 0, 0, 0};
   if (int e = make_im2col_map(&tmA2, block_in, d2)) return e;
   static const char* kNames[3] = {"conv3x3+ds_c128", "conv3x3+ds_c256", "conv3x3+ds_c512"};
-  const double flops = 2.0 * p.M_total * cs.cout * fused_gemm_k(s);
-  if (pairs256) return launch_conv2<256>(tmA, tmB, p, stream, kNames[s], flops, &tmA2);
-  return bn == 256 ? launch_conv_t<256>(tmA, tmB, p, stream, kNames[s], flops, &tmA2)
-                   : launch_conv_t<128>(tmA, tmB, p, stream, kNames[s], flops, &tmA2);
+  return launch_conv2(tmA, tmB, p, stream, kNames[s], 2.0 * p.M_total * cs.cout * fused_gemm_k(s), &tmA2);
 }
 
 static uint16_t host_bf16(float f) {
@@ -859,7 +521,6 @@ static uint16_t host_bf16(float f) {
 }
 
 // per-chunk activation buffers (bf16 NHWC), sizes per patch
-constexpr size_t kC1Bytes = (size_t)112 * 112 * 64 * 2;  // conv1 output
 constexpr size_t kActBytes = (size_t)56 * 56 * 64 * 2;   // largest post-pool activation
 constexpr size_t kS2dBytes = (size_t)112 * kS2dW * 16 * 2;
 
@@ -938,16 +599,17 @@ extern "C" int hipac_resnet18_pack(const float* const* t, int num_tensors, int n
 extern "C" size_t hipac_resnet18_workspace_bytes(int n_patches, int chunk) {
   if (n_patches <= 0) return 256;
   const size_t c = (size_t)clamp_chunk(chunk, n_patches);
-  read_env_flags();
-  // conv1's 112x112x64 output and the projection-shortcut tensor only exist in the unfused A/B modes; the S2D16
-  // repack buffer only when the caller hands the plain NHWC3 layout (sized for it unconditionally: 0.4 MB / patch)
-  return c * ((g_use_fused_stem ? 0 : kC1Bytes) + (g_fuse_downsample ? 3 : 4) * kActBytes + kS2dBytes) + 6 * 1024;
+  // three activation buffers; the S2D16 repack buffer is needed only when the caller hands the plain NHWC3 layout (sized
+  // for it unconditionally: 0.4 MB / patch)
+  return c * (3 * kActBytes + kS2dBytes) + 6 * 1024;
 }
 
 extern "C" int hipac_resnet18_conv_layer(const void* d_packed, int num_classes, int layer, const void* d_in,
                                          const void* d_residual, void* d_out, int n_patches, int relu, void* stream_) {
   HIPAC_REQUIRE(d_packed && d_in && d_out, "null pointer");
   HIPAC_REQUIRE(layer >= 0 && layer < HIPAC_RESNET18_NUM_CONVS, "layer index out of range");
+  HIPAC_REQUIRE(layer != 0, "layer 0 (conv1) runs only fused with the max pool: use hipac_resnet18_stem");
+  HIPAC_REQUIRE(layer != 7, "layer 7 (layer2.0.downsample) runs only fused into layer2.0.conv2: use hipac_resnet18_conv_ds_fused");
   HIPAC_REQUIRE(n_patches > 0, "n_patches must be positive");
   if (int e = init_driver_api()) return e;
   const PackedLayout L = packed_layout(num_classes);
@@ -998,11 +660,9 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
     ws += align_up(bytes, 1024);
     return r;
   };
-  uint8_t* c1 = g_use_fused_stem ? nullptr : carve(cmax * kC1Bytes);
   uint8_t* A = carve(cmax * kActBytes);
   uint8_t* B = carve(cmax * kActBytes);
   uint8_t* C = carve(cmax * kActBytes);
-  uint8_t* D = g_fuse_downsample ? nullptr : carve(cmax * kActBytes);
   uint8_t* s2d = carve(cmax * kS2dBytes);
 
   for (int i0 = 0; i0 < n_patches; i0 += cmax) {
@@ -1021,27 +681,13 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
       x0 = s2d;
     }
     // the batch was written in ascending patch order, so the first layer walks it descending, the next ascending, ...
-    int order = 1;
-    auto next_order = [&]() {
-      g_reverse = g_boustrophedon ? order : 0;
-      order ^= 1;
-    };
+    g_reverse = 1;
     auto conv = [&](int layer, const void* in, const void* res, void* out, bool relu) {
-      next_order();
+      g_reverse ^= 1;
       return run_conv(pk, L, layer, in, res, out, n, relu, stream);
     };
     int e = 0;
-    if (g_use_fused_stem) {
-      next_order();
-      if ((e = run_stem(pk, L, x0, A, n, stream))) return e;
-    } else {
-      if ((e = conv(0, x0, nullptr, c1, true))) return e;
-      {
-        ProfileScope ps("maxpool3x3s2", stream, (double)n * (kC1Bytes + kActBytes));
-        k_maxpool<<<g_num_sms * 8, 256, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(c1), reinterpret_cast<__nv_bfloat16*>(A), n);
-      }
-      count_launch(1);
-    }
+    if ((e = run_stem(pk, L, x0, A, n, stream))) return e;
     // layer1 (two basic blocks, identity shortcuts)
     if ((e = conv(1, A, nullptr, B, true)) || (e = conv(2, B, A, C, true))) return e;
     if ((e = conv(3, C, nullptr, B, true)) || (e = conv(4, B, C, A, true))) return e;
@@ -1049,17 +695,12 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
     for (int s = 0; s < 3; s++) {
       const int l0 = 5 + 5 * s;
       if ((e = conv(l0, A, nullptr, B, true))) return e;           // 3x3 / stride 2
-      if (g_fuse_downsample) {
-        next_order();
-        if ((e = run_conv_ds_fused(pk, L, s, B, A, C, n, stream))) return e;   // 3x3 + 1x1/s2 projection + ReLU, one accumulator
-      } else {
-        if ((e = conv(l0 + 2, A, nullptr, D, false))) return e;    // downsample 1x1 / stride 2 (+BN), no ReLU
-        if ((e = conv(l0 + 1, B, D, C, true))) return e;           // 3x3 + shortcut + ReLU
-      }
+      g_reverse ^= 1;
+      if ((e = run_conv_ds_fused(pk, L, s, B, A, C, n, stream))) return e;   // 3x3 + 1x1/s2 projection + ReLU, one accumulator
       if ((e = conv(l0 + 3, C, nullptr, B, true)) || (e = conv(l0 + 4, B, C, A, true))) return e;
     }
     ProfileScope ps_pool("avgpool_fc", stream, (double)n * (49 * 512 * 2 + 512 * 4));
-    HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc, dim3(n), dim3(256), 0, stream, 1, true, reinterpret_cast<const __nv_bfloat16*>(A),
+    HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc, dim3(n), dim3(256), 0, stream, 1, reinterpret_cast<const __nv_bfloat16*>(A),
                                d_feats + (size_t)i0 * 512, d_logits ? d_logits + (size_t)i0 * num_classes : nullptr,
                                reinterpret_cast<const float*>(pk + L.fc_w_off), reinterpret_cast<const float*>(pk + L.fc_b_off),
                                num_classes, g_n_dev, g_n_base));

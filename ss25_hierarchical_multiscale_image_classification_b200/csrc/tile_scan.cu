@@ -233,10 +233,10 @@ static int launch_compact(const ScanParams& p, const uint8_t* flags, int n_cand,
   const int nb = (n_cand + kCompactBlock - 1) / kCompactBlock;
   ProfileScope ps("compact", stream, (double)n_cand);
   if (nb > 1) {
-    HIPAC_CHECK_CUDA(launch_ex(k_compact_count, dim3(nb), dim3(kCompactBlock), 0, stream, 1, true, flags, n_cand, keep_all, block_tot));
+    HIPAC_CHECK_CUDA(launch_ex(k_compact_count, dim3(nb), dim3(kCompactBlock), 0, stream, 1, flags, n_cand, keep_all, block_tot));
     count_launch(1);
   }
-  HIPAC_CHECK_CUDA(launch_ex(k_compact, dim3(nb), dim3(kCompactBlock), 0, stream, 1, true, p, flags, n_cand, d_coords, d_labels, src_idx, d_count,
+  HIPAC_CHECK_CUDA(launch_ex(k_compact, dim3(nb), dim3(kCompactBlock), 0, stream, 1, p, flags, n_cand, d_coords, d_labels, src_idx, d_count,
                              capacity, keep_all, (const int32_t*)block_tot));
   count_launch(1);
   return 0;

@@ -686,7 +686,7 @@ static int launch_scan_planes_f(const ScanParams& p, const FusedGeom& G, cudaStr
   Z.srow_hi = min(p.H, (G.cy0 + G.ncy) * G.g);
   const int items = Z.n_strips * Z.n_chunks;
   ProfileScope ps("scan_planes", stream, (double)p.H * p.W * 3);
-  HIPAC_CHECK_CUDA(launch_ex(k_scan_planes<F>, dim3((items + kStreamWarps - 1) / kStreamWarps), dim3(kStreamWarps * 32), smem, stream, 1, true, p, G, Z));
+  HIPAC_CHECK_CUDA(launch_ex(k_scan_planes<F>, dim3((items + kStreamWarps - 1) / kStreamWarps), dim3(kStreamWarps * 32), smem, stream, 1, p, G, Z));
   count_launch(1);
   return 0;
 }
@@ -728,7 +728,7 @@ static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* fla
     const int64_t want = (chunks + 1023) / 1024;
     const int grid = (int)(want < 148 * 16 ? want : 148 * 16);
     ProfileScope ps("cell_votes", stream, (double)cell_rows * p.W);
-    HIPAC_CHECK_CUDA(launch_ex(k_cell_votes, dim3(grid), dim3(256), 0, stream, 1, true, p, G, G.cy0 * G.g, cell_rows));
+    HIPAC_CHECK_CUDA(launch_ex(k_cell_votes, dim3(grid), dim3(256), 0, stream, 1, p, G, G.cy0 * G.g, cell_rows));
     count_launch(1);
   } else if (!stream_ok || p.mask) {
     dim3 grid(G.ncx, (cell_rows + 31) / 32);
@@ -738,7 +738,7 @@ static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* fla
   }
   {
     ProfileScope ps("patch_flags", stream, 0.0);
-    HIPAC_CHECK_CUDA(launch_ex(k_patch_flags, dim3((n_cand + 255) / 256), dim3(256), 0, stream, 1, true, p, G, flags, n_cand));
+    HIPAC_CHECK_CUDA(launch_ex(k_patch_flags, dim3((n_cand + 255) / 256), dim3(256), 0, stream, 1, p, G, flags, n_cand));
   }
   count_launch(1);
   if (int e = launch_compact(p, flags, n_cand, d_coords, d_labels, src_idx, d_count, capacity, keep_all, block_tot, stream)) return e;
@@ -755,8 +755,8 @@ static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* fla
     }
     dim3 grid((unsigned)min(n_cand, capacity), OUT / 2 / kGatherPairs);
     ProfileScope ps("gather", stream, 0.0);
-    if (G.f == 1) HIPAC_CHECK_CUDA(launch_ex(k_gather<true>, grid, dim3(128), 0, stream, 1, true, p, G, o, (const int32_t*)d_coords, (const int32_t*)d_count, capacity));
-    else HIPAC_CHECK_CUDA(launch_ex(k_gather<false>, grid, dim3(128), 0, stream, 1, true, p, G, o, (const int32_t*)d_coords, (const int32_t*)d_count, capacity));
+    if (G.f == 1) HIPAC_CHECK_CUDA(launch_ex(k_gather<true>, grid, dim3(128), 0, stream, 1, p, G, o, (const int32_t*)d_coords, (const int32_t*)d_count, capacity));
+    else HIPAC_CHECK_CUDA(launch_ex(k_gather<false>, grid, dim3(128), 0, stream, 1, p, G, o, (const int32_t*)d_coords, (const int32_t*)d_count, capacity));
     count_launch(1);
   }
   HIPAC_CHECK_CUDA(cudaGetLastError());

@@ -40,7 +40,7 @@ def _folded(net, layer):
 
 
 @pytest.mark.parametrize("n", [1, 3])
-@pytest.mark.parametrize("layer", list(range(20)))
+@pytest.mark.parametrize("layer", [l for l in range(20) if l not in (0, 7)])   # 0 and 7 exist only fused: tests below
 def test_conv_layer_vs_torch_fp32(net_and_packed, layer, n):
     from ss25_hierarchical_multiscale_image_classification_b200 import features
     net, packed = net_and_packed
@@ -54,20 +54,27 @@ def test_conv_layer_vs_torch_fp32(net_and_packed, layer, n):
     res = torch.randn((n, hout, hout, cout), generator=g, device="cuda").bfloat16() if use_res else None
     if res is not None:
         ref = ref + res.float().permute(0, 3, 1, 2)
-    relu = layer not in (7, 12, 17)
+    relu = layer not in (12, 17)
     if relu:
         ref = torch.relu(ref)
-    if layer == 0:
-        xin = torch.zeros((n, 112, 115, 16), dtype=torch.bfloat16, device="cuda")
-        xin[:, :, 2:114, :12] = x.reshape(n, 112, 2, 112, 2, 3).permute(0, 1, 3, 2, 4, 5).reshape(n, 112, 112, 12)
-    else:
-        xin = x
-    out = features.conv_layer(packed, layer, xin, res, relu)
+    out = features.conv_layer(packed, layer, x, res, relu)
     torch.cuda.synchronize()
     got = out.float().permute(0, 3, 1, 2)
     scale = float(ref.abs().max())
     err = float((got - ref).abs().max())
     assert err <= 1.5 * 2.0 ** -8 * scale + 1e-3, f"layer {layer}: max err {err} at scale {scale}"
+
+
+@pytest.mark.parametrize("layer,fused_hook", [(0, "hipac_resnet18_stem"), (7, "hipac_resnet18_conv_ds_fused")])
+def test_conv_layer_refuses_fused_only_layers(net_and_packed, layer, fused_hook):
+    """conv1 exists only fused with the max pool, layer2.0's projection shortcut only fused into layer2.0.conv2: the per-layer
+    hook refuses both and names the fused hook that computes them."""
+    from ss25_hierarchical_multiscale_image_classification_b200 import features
+    _, packed = net_and_packed
+    cin, _, _, _, _, hin = SPECS[layer]
+    x = torch.zeros((1, hin, hin, cin), dtype=torch.bfloat16, device="cuda")
+    with pytest.raises(RuntimeError, match=fused_hook):
+        features.conv_layer(packed, layer, x, None, layer == 0)
 
 
 def _metrics(got, ref):
