@@ -36,7 +36,7 @@ struct RowConvParams {
   __nv_bfloat16* out;
   const int* n_dev;  // device-count mode, see effective_patches()
   int n_base;
-  int reverse;       // tile order, see g_reverse
+  int reverse;       // tile order, see Launch::reverse
 };
 
 // bias + residual (16-byte chunk of 8 bf16, already loaded) + ReLU on 8 accumulator columns -> 8 bf16

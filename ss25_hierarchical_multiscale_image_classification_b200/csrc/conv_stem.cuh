@@ -34,7 +34,7 @@ struct StemParams {
   __nv_bfloat16* out;  // [n][56][56][64]
   const int* n_dev;    // device-count mode, see effective_patches()
   int n_base;
-  int reverse;         // block order, see g_reverse
+  int reverse;         // block order, see Launch::reverse
 };
 
 using ptx::named_bar_sync;

@@ -38,7 +38,7 @@ struct ConvParams {   // the im2col kernel's (conv_umma2.cuh)
   __nv_bfloat16* out;
   const int* n_dev;  // device-side patch count (null: the host-side sizes above are exact)
   int n_base;        // first patch of this chunk: the kernel works on clamp(*n_dev - n_base, 0, host n) patches
-  int reverse;       // walk the tiles from the last to the first (see g_reverse)
+  int reverse;       // walk the tiles from the last to the first (see Launch::reverse)
 };
 
 // Device-count mode: the host sizes grids, tensor maps and buffers for a CAPACITY; the number of patches that actually
@@ -48,12 +48,6 @@ __device__ __forceinline__ int effective_patches(const int* n_dev, int n_base, i
   const int n = __ldg(n_dev) - n_base;
   return n < 0 ? 0 : (n < n_cap ? n : n_cap);
 }
-static thread_local const int* g_n_dev = nullptr;   // set by hipac_resnet18_forward_dcount around its launches
-static thread_local int g_n_base = 0;
-// Boustrophedon tile order across the layers of one forward pass: a layer whose producer wrote images 0..n-1 walks
-// them n-1..0, so its first ~100 MB of reads are the producer's LAST writes and still sit in the 126 MB L2 (with the
-// same order on both sides they would be the oldest, long evicted).  Flipped after every launch of a forward pass.
-static thread_local int g_reverse = 0;
 
 constexpr int kBM = 128;
 constexpr int kS2dW = HIPAC_S2D16_WIDTH;  // 112 + 3 explicit zero columns (2 left, 1 right)
@@ -200,40 +194,44 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeIm2colFn g_encode_im2col = nullptr;
 static EncodeTiledFn g_encode_tiled = nullptr;
-static thread_local int g_num_sms = 0;   // SM count of the CURRENT device, refreshed by init_driver_api() on every entry
-// Called at the top of every entry point: driver entry points once per process, the SM count for the CURRENT device.
+// Called at the top of every entry point: resolves the driver entry points once per process.
 static int init_driver_api() {
   static std::mutex mu;
-  {
-    std::lock_guard<std::mutex> lk(mu);
-    if (!(g_encode_im2col && g_encode_tiled)) {
-      cudaDriverEntryPointQueryResult q;
-      void* fn = nullptr;
-      HIPAC_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &fn, cudaEnableDefault, &q));
-      HIPAC_REQUIRE(fn && q == cudaDriverEntryPointSuccess, "driver lacks cuTensorMapEncodeIm2col");
-      g_encode_im2col = (EncodeIm2colFn)fn;
-      HIPAC_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q));
-      HIPAC_REQUIRE(fn && q == cudaDriverEntryPointSuccess, "driver lacks cuTensorMapEncodeTiled");
-      g_encode_tiled = (EncodeTiledFn)fn;
-    }
+  std::lock_guard<std::mutex> lk(mu);
+  if (!(g_encode_im2col && g_encode_tiled)) {
+    cudaDriverEntryPointQueryResult q;
+    void* fn = nullptr;
+    HIPAC_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &fn, cudaEnableDefault, &q));
+    HIPAC_REQUIRE(fn && q == cudaDriverEntryPointSuccess, "driver lacks cuTensorMapEncodeIm2col");
+    g_encode_im2col = (EncodeIm2colFn)fn;
+    HIPAC_CHECK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q));
+    HIPAC_REQUIRE(fn && q == cudaDriverEntryPointSuccess, "driver lacks cuTensorMapEncodeTiled");
+    g_encode_tiled = (EncodeTiledFn)fn;
   }
-  return device_sm_count(&g_num_sms);
+  return 0;
 }
 
-// NHWC activation tensor [n][h][w][c] (bf16) as an im2col map: box = 128 output pixels x `chan_box` channels.
-struct Im2colDesc {
-  int n, h, w, c;                 // logical NHWC extents seen by TMA
-  int64_t pix_stride, row_stride, img_stride;  // bytes
-  int kh, kw, stride;             // filter extent and traversal stride
-  int pad_w_lo, pad_w_hi, pad_h_lo, pad_h_hi;
+// What a stage-2 launch needs besides its operands.  Each C entry point builds one and passes it down; forward_impl
+// sets n_base per chunk and reverse per launch.
+struct Launch {
+  cudaStream_t stream;
+  int sms;            // SM count of the current device
+  const int* n_dev;   // device-side patch count (device-count mode, see effective_patches) or null
+  int n_base;         // first patch of this chunk
+  // Boustrophedon tile order across the layers of one forward pass: a layer whose producer wrote images 0..n-1 walks
+  // them n-1..0, so its first ~100 MB of reads are the producer's LAST writes and still sit in the 126 MB L2 (with the
+  // same order on both sides they would be the oldest, long evicted).
+  int reverse;
 };
-static int make_im2col_map(CUtensorMap* map, const void* ptr, const Im2colDesc& d) {
-  cuuint64_t dims[4] = {(cuuint64_t)d.c, (cuuint64_t)d.w, (cuuint64_t)d.h, (cuuint64_t)d.n};
-  cuuint64_t strides[3] = {(cuuint64_t)d.pix_stride, (cuuint64_t)d.row_stride, (cuuint64_t)d.img_stride};
-  int lower[2] = {-d.pad_w_lo, -d.pad_h_lo};
-  int upper[2] = {d.pad_w_hi - (d.kw - 1), d.pad_h_hi - (d.kh - 1)};
-  cuuint32_t estr[4] = {1, (cuuint32_t)d.stride, (cuuint32_t)d.stride, 1};
-  const int n = d.n, h = d.h, w = d.w, c = d.c;
+
+// Input of conv `cs` on n patches, bf16 NHWC [n][hin][hin][cin], as an im2col map: box = 128 output pixels x 64 channels.
+static int make_im2col_map(CUtensorMap* map, const void* ptr, int n, const ConvSpec& cs) {
+  const int h = cs.hin, w = cs.hin, c = cs.cin;
+  cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
+  cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
+  int lower[2] = {-cs.pad, -cs.pad};
+  int upper[2] = {cs.pad - (cs.k - 1), cs.pad - (cs.k - 1)};
+  cuuint32_t estr[4] = {1, (cuuint32_t)cs.stride, (cuuint32_t)cs.stride, 1};
   CUresult r = g_encode_im2col(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, lower, upper,
                                64u, (cuuint32_t)kBM, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -265,195 +263,115 @@ static int make_weight_map(CUtensorMap* map, const void* ptr, int cout, int K, i
   return 0;
 }
 
-// NHWC activation tensor as a tiled 4-D map whose box is one row-tile region: 64 channels x (w+2) x (r+2) x 1.
-static int make_region_map(CUtensorMap* map, const void* ptr, int n, int h, int w, int c, int r) {
+// Activation tensor [n][h][w][c] (bf16) as a tiled 4-D map: box = box_c channels x box_w x box_h pixels x 1 image, element
+// stride `es` along w and h.  `what` names the map in the error message.
+static int make_act_map(CUtensorMap* map, const void* ptr, int n, int h, int w, int c, int box_c, int box_w, int box_h, int es,
+                        CUtensorMapSwizzle swizzle, const char* what) {
   cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
   cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)(w + 2), (cuuint32_t)(r + 2), 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
+  cuuint32_t box[4] = {(cuuint32_t)box_c, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
+  cuuint32_t estr[4] = {1, (cuuint32_t)es, (cuuint32_t)es, 1};
   CUresult res = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                                CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (res != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (region map) failed with CUresult " + std::to_string((int)res));
+    set_error(std::string("cuTensorMapEncodeTiled (") + what + ") failed with CUresult " + std::to_string((int)res));
     return -5;
   }
   return 0;
 }
 
-// NHWC activation tensor as a strided tiled map for the fused 1x1 / stride-2 projection: the box spans 2*wp x 2*r input
-// pixels with element strides 2, i.e. delivers wp x r pixels x 64 channels (out-of-range pixels zero filled).
-static int make_strided_map(CUtensorMap* map, const void* ptr, int n, int h, int w, int c, int wp, int r) {
-  cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
-  cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)(2 * wp), (cuuint32_t)(2 * r), 1};
-  cuuint32_t estr[4] = {1, 2, 2, 1};
-  CUresult res = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (res != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (strided projection map) failed with CUresult " + std::to_string((int)res));
-    return -5;
+// One launch of a CTA-pair kernel (clusters of 2) over `pairs` work items: at most one pair per two SMs, the persistent
+// pairs loop over the items.
+template <typename... KArgs, typename... Args>
+static int launch_pairs(const Launch& ctx, void (*kernel)(KArgs...), int pairs, int threads, int smem, const char* name, double flops,
+                        const Args&... args) {
+  if (int e = ensure_dyn_smem(kernel, smem)) return e;
+  const int max_pairs = ctx.sms / 2;
+  const int grid = 2 * (pairs < max_pairs ? pairs : max_pairs);
+  {
+    ProfileScope ps(name, ctx.stream, flops);
+    HIPAC_CHECK_CUDA(launch_ex(kernel, dim3((unsigned)grid), dim3((unsigned)threads), smem, ctx.stream, 2, args...));
   }
-  return 0;
-}
-
-// NHWC activation tensor as a tiled map whose box is one OUTPUT row tile: 64 channels x w x r x 1 (TMA store of the
-// epilogue's staging tile / TMA load of the residual tile).
-static int make_tile_map(CUtensorMap* map, const void* ptr, int n, int h, int w, int c, int r) {
-  cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
-  cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)w, (cuuint32_t)r, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult res = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (res != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (tile map) failed with CUresult " + std::to_string((int)res));
-    return -5;
-  }
+  count_launch(1);
+  HIPAC_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 
 // CTA-pair row kernel (conv_rows2.cuh).  weights = [BN][9*KC*64 (+ KDS*64)] K-major at w_ptr; ds_in = block input of the
 // fused projection shortcut (KDS = 1) or null.
 template <int BN, int KC, int W, int R, int KDS, bool TEPI = (BN == 64)>
-static int launch_rows2_t(const void* w_ptr, const float* bias, const void* in, const void* ds_in, const void* residual, void* out,
-                          int n, bool relu, cudaStream_t stream, const char* name, double flops) {
+static int launch_rows2_t(const Launch& ctx, const void* w_ptr, const float* bias, const void* in, const void* ds_in,
+                          const void* residual, void* out, int n, bool relu, const char* name, double flops) {
   using Cfg = Row2Cfg<BN, KC, W, R, KDS, TEPI>;
-  if (int e = ensure_dyn_smem(k_conv3x3_rows2<BN, KC, W, R, KDS, TEPI>, Cfg::kSmemBytes)) return e;
-  CUtensorMap tmA, tmB, tmA2;
-  if (int e = make_region_map(&tmA, in, n, W, W, KC * 64, R)) return e;
+  const CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B;
+  CUtensorMap tmA, tmB;
+  // the box is one row-tile region: 64 channels x (W + 2) x (R + 2)
+  if (int e = make_act_map(&tmA, in, n, W, W, KC * 64, 64, W + 2, R + 2, 1, sw, "region map")) return e;
   if (int e = make_weight_map(&tmB, w_ptr, BN, (9 * KC + KDS) * 64, BN / 2)) return e;
-  if (KDS) {
-    if (int e = make_strided_map(&tmA2, ds_in, n, 2 * W, 2 * W, 64, W + 2, R)) return e;
-  } else {
-    tmA2 = tmA;
-  }
-  CUtensorMap tmO = tmA, tmR = tmA;
+  CUtensorMap tmA2 = tmA, tmO = tmA, tmR = tmA;
+  // the 1x1 / stride-2 projection: the box spans 2 (W + 2) x 2 R input pixels with element strides 2, i.e. delivers
+  // (W + 2) x R pixels x 64 channels (out-of-range pixels zero filled)
+  if (KDS)
+    if (int e = make_act_map(&tmA2, ds_in, n, 2 * W, 2 * W, 64, 64, 2 * (W + 2), 2 * R, 2, sw, "strided projection map")) return e;
   if (Cfg::kTmaEpi) {
-    if (int e = make_tile_map(&tmO, out, n, W, W, BN, R)) return e;
+    // the box is one OUTPUT row tile, 64 channels x W x R (TMA store of the epilogue's staging tile / TMA load of the
+    // residual tile)
+    if (int e = make_act_map(&tmO, out, n, W, W, BN, 64, W, R, 1, sw, "tile map")) return e;
     tmR = tmO;
     if (residual)
-      if (int e = make_tile_map(&tmR, residual, n, W, W, BN, R)) return e;
+      if (int e = make_act_map(&tmR, residual, n, W, W, BN, 64, W, R, 1, sw, "tile map")) return e;
   }
   RowConvParams p;
   p.n_img = n, p.num_tiles = n * (W / R), p.relu = relu ? 1 : 0;
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
+  p.n_dev = ctx.n_dev, p.n_base = ctx.n_base, p.reverse = ctx.reverse;
   p.bias = bias;
   p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  const int pairs = (p.num_tiles + 1) / 2;
-  const int max_pairs = g_num_sms / 2;
-  const int grid = 2 * (pairs < max_pairs ? pairs : max_pairs);
-  {
-    ProfileScope ps(name, stream, flops);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv3x3_rows2<BN, KC, W, R, KDS, TEPI>, dim3((unsigned)grid), dim3((unsigned)conv_threads(BN)), Cfg::kSmemBytes,
-                               stream, 2, tmA, tmB, tmA2, tmO, tmR, p));
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
-  return 0;
+  return launch_pairs(ctx, k_conv3x3_rows2<BN, KC, W, R, KDS, TEPI>, (p.num_tiles + 1) / 2, conv_threads(BN), Cfg::kSmemBytes, name,
+                      flops, tmA, tmB, tmA2, tmO, tmR, p);
 }
 
 // layer2.0.conv1 (3x3 / stride 2, 64 -> 128, 56x56 -> 28x28) as a parity-split row kernel on CTA pairs (conv_rows2_s2.cuh).
-static int launch_rows2_s2(const void* w_ptr, const float* bias, const void* in, void* out, int n, bool relu, cudaStream_t stream,
+static int launch_rows2_s2(const Launch& ctx, const void* w_ptr, const float* bias, const void* in, void* out, int n, bool relu,
                            const char* name, double flops) {
   using Cfg = S2Cfg;
-  if (int e = ensure_dyn_smem(k_conv3x3s2_rows2, Cfg::kSmemBytes)) return e;
+  const CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B;
   CUtensorMap tmE, tmO, tmB;
-  if (int e = make_strided_map(&tmE, in, n, 56, 56, 64, Cfg::Wp, Cfg::R)) return e;
-  if (int e = make_strided_map(&tmO, in, n, 56, 56, 64, Cfg::Wp, Cfg::R + 1)) return e;
+  // element strides 2: the boxes deliver Wp x R (even input rows) and Wp x (R + 1) (odd input rows) pixels x 64 channels
+  if (int e = make_act_map(&tmE, in, n, 56, 56, 64, 64, 2 * Cfg::Wp, 2 * Cfg::R, 2, sw, "strided projection map")) return e;
+  if (int e = make_act_map(&tmO, in, n, 56, 56, 64, 64, 2 * Cfg::Wp, 2 * (Cfg::R + 1), 2, sw, "strided projection map")) return e;
   if (int e = make_weight_map(&tmB, w_ptr, Cfg::BN, 9 * 64, Cfg::BN / 2)) return e;
   RowConvParams p;
   p.n_img = n, p.num_tiles = n * (Cfg::W / Cfg::R), p.relu = relu ? 1 : 0;
   p.bias = bias, p.residual = nullptr, p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
-  const int pairs = (p.num_tiles + 1) / 2, max_pairs = g_num_sms / 2;
-  const int grid = 2 * (pairs < max_pairs ? pairs : max_pairs);
-  {
-    ProfileScope ps(name, stream, flops);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv3x3s2_rows2, dim3((unsigned)grid), dim3((unsigned)conv_threads(128)), Cfg::kSmemBytes, stream, 2, tmE,
-                               tmO, tmB, p));
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
-  return 0;
+  p.n_dev = ctx.n_dev, p.n_base = ctx.n_base, p.reverse = ctx.reverse;
+  return launch_pairs(ctx, k_conv3x3s2_rows2, (p.num_tiles + 1) / 2, conv_threads(128), Cfg::kSmemBytes, name, flops, tmE, tmO, tmB, p);
 }
 
 // Fused conv1 + BN + ReLU + maxpool on the S2D16 batch -> [n][56][56][64], on CTA pairs (conv_stem.cuh).
-static int run_stem(const uint8_t* d_packed, const PackedLayout& L, const void* in, void* out, int n, cudaStream_t stream) {
-  if (int e = ensure_dyn_smem(k_conv1_pool, kStemSmem)) return e;
+static int run_stem(const Launch& ctx, const uint8_t* d_packed, const PackedLayout& L, const void* in, void* out, int n) {
   CUtensorMap tmA, tmB;
-  {
-    cuuint64_t dims[4] = {16, (cuuint64_t)kS2dW, 112, (cuuint64_t)n};
-    cuuint64_t strides[3] = {32, (cuuint64_t)kS2dW * 32, (cuuint64_t)112 * kS2dW * 32};
-    cuuint32_t box[4] = {16, (cuuint32_t)kS2dW, (cuuint32_t)kStemRows, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult res = g_encode_tiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(in), dims, strides, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (res != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled (stem region map) failed with CUresult " + std::to_string((int)res));
-      return -5;
-    }
-  }
+  // S2D16 [n][112][kS2dW][16]: the box is one block region, all kS2dW pixels of kStemRows rows
+  if (int e = make_act_map(&tmA, in, n, 112, kS2dW, 16, 16, kS2dW, kStemRows, 1, CU_TENSOR_MAP_SWIZZLE_32B, "stem region map"))
+    return e;
   if (int e = make_weight_map(&tmB, d_packed + L.w_off[0], 64, 256, 32)) return e;
   StemParams p;
   p.num_blocks = n * (56 / kStemPB);
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
+  p.n_dev = ctx.n_dev, p.n_base = ctx.n_base, p.reverse = ctx.reverse;
   p.bias = reinterpret_cast<const float*>(d_packed + L.b_off[0]);
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  const int pairs = (p.num_blocks + 1) / 2, max_pairs = g_num_sms / 2;
-  const int grid = 2 * (pairs < max_pairs ? pairs : max_pairs);
-  {
-    ProfileScope ps("conv1_pool_fused", stream, 2.0 * n * 112 * 112 * 64 * 147);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv1_pool, dim3(grid), dim3(kStemThreads), kStemSmem, stream, 2, tmA, tmB, p));
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
-  return 0;
+  return launch_pairs(ctx, k_conv1_pool, (p.num_blocks + 1) / 2, kStemThreads, kStemSmem, "conv1_pool_fused",
+                      2.0 * n * 112 * 112 * 64 * 147, tmA, tmB, p);
 }
 
-// im2col layers on CTA pairs (conv_umma2.cuh); tmB must have been built with a box of 128 weight rows.
-static int launch_conv2(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvParams& p, cudaStream_t stream, const char* name,
-                        double flops, const CUtensorMap* tmA2 = nullptr) {
-  using Cfg = Conv2Cfg<256>;
-  if (int e = ensure_dyn_smem(k_conv_umma2<256>, Cfg::kSmemBytes)) return e;
-  const int ptiles = ((p.num_m_tiles + 1) / 2) * p.num_n_tiles;
-  const int max_pairs = g_num_sms / 2;
-  const int grid = 2 * (ptiles < max_pairs ? ptiles : max_pairs);
-  {
-    ProfileScope ps(name, stream, flops);
-    HIPAC_CHECK_CUDA(launch_ex(k_conv_umma2<256>, dim3((unsigned)grid), dim3((unsigned)conv_threads(256)), Cfg::kSmemBytes, stream, 2, tmA,
-                               tmB, tmA2 ? *tmA2 : tmA, p));
-  }
-  count_launch(1);
-  HIPAC_CHECK_CUDA(cudaGetLastError());
-  return 0;
-}
-
-// One conv layer of the network on `n` patches, bf16 NHWC in / out.  Not for layer 0 (conv1, which exists only fused with
-// the max pool: run_stem) or layer 7 (layer2.0's projection shortcut, which exists only fused: run_conv_ds_fused).
-static int run_conv(const uint8_t* d_packed, const PackedLayout& L, int layer, const void* in, const void* residual, void* out,
-                    int n, bool relu, cudaStream_t stream) {
+// layer3 / layer4 conv `layer` as the im2col GEMM on CTA pairs (conv_umma2.cuh).  With ds_in, the 1x1 / stride-2
+// projection shortcut `ds_layer` of the block input ds_in adds its K-blocks (read through a second im2col map) to the same
+// accumulator.  Weights [cout][K] at w_ptr, K = the conv's K followed by the shortcut's.
+static int launch_conv2(const Launch& ctx, int layer, int ds_layer, const void* w_ptr, const float* bias, const void* in,
+                        const void* ds_in, const void* residual, void* out, int n, bool relu, const char* name) {
   const ConvSpec& cs = kConvs[layer];
-  const uint8_t* w = d_packed + L.w_off[layer];
-  const float* bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
-  if (cs.cout == 64)   // layer1: 3x3 / s1 at 56x56
-    return launch_rows2_t<64, 1, 56, 2, 0>(w, bias, in, nullptr, residual, out, n, relu, stream, "conv3x3_c64", 2.0 * n * 56 * 56 * 64 * 576);
-  if (cs.cout == 128 && cs.stride == 2) {   // layer2.0.conv1: 3x3 / s2, 64 -> 128
-    HIPAC_REQUIRE(residual == nullptr, "layer2.0.conv1 takes no residual");
-    return launch_rows2_s2(w, bias, in, out, n, relu, stream, "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 576);
-  }
-  if (cs.cout == 128) {   // layer2: 3x3 / s1 at 28x28; the residual variant has the staged epilogue (see conv_rows2.cuh)
-    if (residual)
-      return launch_rows2_t<128, 2, 28, 4, 0, true>(w, bias, in, nullptr, residual, out, n, relu, stream, "conv3x3_c128",
-                                                    2.0 * n * 28 * 28 * 128 * 1152);
-    return launch_rows2_t<128, 2, 28, 4, 0>(w, bias, in, nullptr, nullptr, out, n, relu, stream, "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 1152);
-  }
-  // layer3 / layer4: im2col on CTA pairs
-  const int K = conv_gemm_k(layer);
+  const int K = conv_gemm_k(layer) + (ds_in ? conv_gemm_k(ds_layer) : 0);
   ConvParams p;
   p.M_total = n * cs.hout * cs.hout;
   p.hw_out = cs.hout * cs.hout, p.wout = cs.hout;
@@ -463,53 +381,61 @@ static int run_conv(const uint8_t* d_packed, const PackedLayout& L, int layer, c
   p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
   p.num_m_tiles = (p.M_total + kBM - 1) / kBM;
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
+  p.n_dev = ctx.n_dev, p.n_base = ctx.n_base, p.reverse = ctx.reverse;
   p.num_kb2 = 0, p.stride2 = 1;
   p.num_n_tiles = cs.cout / 256;
   p.stride = cs.stride, p.pad_w = p.pad_h = cs.pad, p.kw = cs.k, p.kc_blocks = cs.cin / 64, p.num_kb = cs.k * cs.k * p.kc_blocks;
   CUtensorMap tmA, tmB;
-  if (int e = make_weight_map(&tmB, w, cs.cout, K, 128)) return e;
-  Im2colDesc d{n, cs.hin, cs.hin, cs.cin, (int64_t)cs.cin * 2, (int64_t)cs.hin * cs.cin * 2, (int64_t)cs.hin * cs.hin * cs.cin * 2,
-               cs.k, cs.k, cs.stride, cs.pad, cs.pad, cs.pad, cs.pad};
-  if (int e = make_im2col_map(&tmA, in, d)) return e;
+  if (int e = make_weight_map(&tmB, w_ptr, cs.cout, K, 128)) return e;   // box of 128 weight rows: each CTA's half
+  if (int e = make_im2col_map(&tmA, in, n, cs)) return e;
+  CUtensorMap tmA2 = tmA;
+  if (ds_in) {
+    const ConvSpec& ds = kConvs[ds_layer];
+    p.num_kb2 = ds.cin / 64, p.stride2 = ds.stride;
+    if (int e = make_im2col_map(&tmA2, ds_in, n, ds)) return e;
+  }
+  return launch_pairs(ctx, k_conv_umma2<256>, ((p.num_m_tiles + 1) / 2) * p.num_n_tiles, conv_threads(256), Conv2Cfg<256>::kSmemBytes,
+                      name, 2.0 * p.M_total * cs.cout * K, tmA, tmB, tmA2, p);
+}
+
+// One conv layer of the network on `n` patches, bf16 NHWC in / out.  Not for layer 0 (conv1, which exists only fused with
+// the max pool: run_stem) or layer 7 (layer2.0's projection shortcut, which exists only fused: run_conv_ds_fused).
+static int run_conv(const Launch& ctx, const uint8_t* d_packed, const PackedLayout& L, int layer, const void* in, const void* residual,
+                    void* out, int n, bool relu) {
+  const ConvSpec& cs = kConvs[layer];
+  const uint8_t* w = d_packed + L.w_off[layer];
+  const float* bias = reinterpret_cast<const float*>(d_packed + L.b_off[layer]);
+  if (cs.cout == 64)   // layer1: 3x3 / s1 at 56x56
+    return launch_rows2_t<64, 1, 56, 2, 0>(ctx, w, bias, in, nullptr, residual, out, n, relu, "conv3x3_c64", 2.0 * n * 56 * 56 * 64 * 576);
+  if (cs.cout == 128 && cs.stride == 2) {   // layer2.0.conv1: 3x3 / s2, 64 -> 128
+    HIPAC_REQUIRE(residual == nullptr, "layer2.0.conv1 takes no residual");
+    return launch_rows2_s2(ctx, w, bias, in, out, n, relu, "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 576);
+  }
+  if (cs.cout == 128) {   // layer2: 3x3 / s1 at 28x28; the residual variant has the staged epilogue (see conv_rows2.cuh)
+    if (residual)
+      return launch_rows2_t<128, 2, 28, 4, 0, true>(ctx, w, bias, in, nullptr, residual, out, n, relu, "conv3x3_c128",
+                                                    2.0 * n * 28 * 28 * 128 * 1152);
+    return launch_rows2_t<128, 2, 28, 4, 0>(ctx, w, bias, in, nullptr, nullptr, out, n, relu, "conv3x3_c128", 2.0 * n * 28 * 28 * 128 * 1152);
+  }
+  // layer3 / layer4: im2col on CTA pairs
   static const char* kNames[2][2] = {{"conv3x3_c256", "conv1x1_c256"}, {"conv3x3_c512", "conv1x1_c512"}};
-  return launch_conv2(tmA, tmB, p, stream, kNames[cs.cout == 512][cs.k == 1], 2.0 * p.M_total * cs.cout * K);
+  return launch_conv2(ctx, layer, -1, w, bias, in, nullptr, residual, out, n, relu, kNames[cs.cout == 512][cs.k == 1]);
 }
 
 // conv2 of a stage's first block with its projection shortcut fused: out = relu(conv3x3(in) + conv1x1_s2(block_in) + bias).
 // Both GEMMs accumulate into the same TMEM tile (the shortcut is extra K-blocks), so the shortcut tensor never exists.
-static int run_conv_ds_fused(const uint8_t* d_packed, const PackedLayout& L, int s, const void* in, const void* block_in, void* out,
-                             int n, cudaStream_t stream) {
-  const int lc = fused_conv_layer(s), ld = fused_ds_layer(s);
-  const ConvSpec &cs = kConvs[lc], &ds = kConvs[ld];
+static int run_conv_ds_fused(const Launch& ctx, const uint8_t* d_packed, const PackedLayout& L, int s, const void* in,
+                             const void* block_in, void* out, int n) {
+  const void* w = d_packed + L.wf_off[s];
+  const float* bias = reinterpret_cast<const float*>(d_packed + L.bf_off[s]);
   if (s == 0) {
     // layer2.0: 3x3 128 -> 128 at 28x28 + 1x1/s2 64 -> 128 from the 56x56 block input, on CTA pairs with resident weights
-    return launch_rows2_t<128, 2, 28, 4, 1>(d_packed + L.wf_off[0], reinterpret_cast<const float*>(d_packed + L.bf_off[0]), in, block_in,
-                                            nullptr, out, n, true, stream, "conv3x3+ds_c128", 2.0 * n * 28 * 28 * 128 * fused_gemm_k(0));
+    return launch_rows2_t<128, 2, 28, 4, 1>(ctx, w, bias, in, block_in, nullptr, out, n, true, "conv3x3+ds_c128",
+                                            2.0 * n * 28 * 28 * 128 * fused_gemm_k(0));
   }
   // layer3.0 / layer4.0: im2col on CTA pairs, the shortcut from a second im2col map
-  ConvParams p;
-  p.M_total = n * cs.hout * cs.hout;
-  p.hw_out = cs.hout * cs.hout, p.wout = cs.hout;
-  p.cout = cs.cout, p.relu = 1;
-  p.bias = reinterpret_cast<const float*>(d_packed + L.bf_off[s]);
-  p.residual = nullptr;
-  p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  p.num_m_tiles = (p.M_total + kBM - 1) / kBM;
-  p.n_dev = g_n_dev, p.n_base = g_n_base, p.reverse = g_reverse;
-  p.num_n_tiles = cs.cout / 256;
-  p.stride = 1, p.pad_w = p.pad_h = 1, p.kw = 3, p.kc_blocks = cs.cin / 64, p.num_kb = 9 * p.kc_blocks;
-  p.num_kb2 = ds.cin / 64, p.stride2 = 2;
-  CUtensorMap tmA, tmA2, tmB;
-  if (int e = make_weight_map(&tmB, d_packed + L.wf_off[s], cs.cout, fused_gemm_k(s), 128)) return e;
-  Im2colDesc d{n, cs.hin, cs.hin, cs.cin, (int64_t)cs.cin * 2, (int64_t)cs.hin * cs.cin * 2, (int64_t)cs.hin * cs.hin * cs.cin * 2,
-               3, 3, 1, 1, 1, 1, 1};
-  if (int e = make_im2col_map(&tmA, in, d)) return e;
-  Im2colDesc d2{n, ds.hin, ds.hin, ds.cin, (int64_t)ds.cin * 2, (int64_t)ds.hin * ds.cin * 2, (int64_t)ds.hin * ds.hin * ds.cin * 2,
-                1, 1, 2, 0, 0, 0, 0};
-  if (int e = make_im2col_map(&tmA2, block_in, d2)) return e;
   static const char* kNames[3] = {"conv3x3+ds_c128", "conv3x3+ds_c256", "conv3x3+ds_c512"};
-  return launch_conv2(tmA, tmB, p, stream, kNames[s], 2.0 * p.M_total * cs.cout * fused_gemm_k(s), &tmA2);
+  return launch_conv2(ctx, fused_conv_layer(s), fused_ds_layer(s), w, bias, in, block_in, nullptr, out, n, true, kNames[s]);
 }
 
 static uint16_t host_bf16(float f) {
@@ -611,38 +537,39 @@ extern "C" int hipac_resnet18_conv_layer(const void* d_packed, int num_classes, 
   HIPAC_REQUIRE(layer != 0, "layer 0 (conv1) runs only fused with the max pool: use hipac_resnet18_stem");
   HIPAC_REQUIRE(layer != 7, "layer 7 (layer2.0.downsample) runs only fused into layer2.0.conv2: use hipac_resnet18_conv_ds_fused");
   HIPAC_REQUIRE(n_patches > 0, "n_patches must be positive");
+  int sms = 0;
   if (int e = init_driver_api()) return e;
+  if (int e = device_sm_count(&sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
-  return run_conv(reinterpret_cast<const uint8_t*>(d_packed), L, layer, d_in, d_residual, d_out, n_patches, relu != 0,
-                  (cudaStream_t)stream_);
+  return run_conv({(cudaStream_t)stream_, sms, nullptr, 0, 0}, reinterpret_cast<const uint8_t*>(d_packed), L, layer, d_in, d_residual,
+                  d_out, n_patches, relu != 0);
 }
 
 extern "C" int hipac_resnet18_conv_ds_fused(const void* d_packed, int num_classes, int stage, const void* d_in, const void* d_block_in,
                                             void* d_out, int n_patches, void* stream_) {
   HIPAC_REQUIRE(d_packed && d_in && d_block_in && d_out && n_patches > 0, "bad arguments");
   HIPAC_REQUIRE(stage >= 0 && stage < 3, "stage must be 0 (layer2), 1 (layer3) or 2 (layer4)");
+  int sms = 0;
   if (int e = init_driver_api()) return e;
+  if (int e = device_sm_count(&sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
-  return run_conv_ds_fused(reinterpret_cast<const uint8_t*>(d_packed), L, stage, d_in, d_block_in, d_out, n_patches,
-                           (cudaStream_t)stream_);
+  return run_conv_ds_fused({(cudaStream_t)stream_, sms, nullptr, 0, 0}, reinterpret_cast<const uint8_t*>(d_packed), L, stage, d_in,
+                           d_block_in, d_out, n_patches);
 }
 
 extern "C" int hipac_resnet18_stem(const void* d_packed, int num_classes, const void* d_in, void* d_out, int n_patches,
                                    void* stream_) {
   HIPAC_REQUIRE(d_packed && d_in && d_out && n_patches > 0, "bad arguments");
+  int sms = 0;
   if (int e = init_driver_api()) return e;
+  if (int e = device_sm_count(&sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
-  return run_stem(reinterpret_cast<const uint8_t*>(d_packed), L, d_in, d_out, n_patches, (cudaStream_t)stream_);
+  return run_stem({(cudaStream_t)stream_, sms, nullptr, 0, 0}, reinterpret_cast<const uint8_t*>(d_packed), L, d_in, d_out, n_patches);
 }
 
 static int forward_impl(const void* d_packed, int num_classes, const void* d_batch, int layout, int n_patches,
                         float* d_feats, float* d_logits, void* d_workspace, size_t workspace_bytes, int chunk,
                         void* stream_, const int* d_count) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  struct CountScope {   // every launch below picks the device count up from these thread-locals
-    explicit CountScope(const int* c) { g_n_dev = c, g_n_base = 0, g_reverse = 0; }
-    ~CountScope() { g_n_dev = nullptr, g_n_base = 0, g_reverse = 0; }
-  } count_scope(d_count);
   HIPAC_REQUIRE(n_patches >= 0, "negative n_patches");
   if (n_patches == 0) return 0;
   HIPAC_REQUIRE(d_packed && d_batch && d_feats && d_workspace, "null pointer");
@@ -650,7 +577,9 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
   HIPAC_REQUIRE(!d_logits || num_classes > 0, "logits requested but the packed weights have no classifier head");
   HIPAC_REQUIRE(workspace_bytes >= hipac_resnet18_workspace_bytes(n_patches, chunk), "workspace too small");
   HIPAC_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "workspace must be 256-byte aligned");
+  Launch ctx{(cudaStream_t)stream_, 0, d_count, 0, 0};
   if (int e = init_driver_api()) return e;
+  if (int e = device_sm_count(&ctx.sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
   const uint8_t* pk = reinterpret_cast<const uint8_t*>(d_packed);
   const int cmax = clamp_chunk(chunk, n_patches);
@@ -667,27 +596,32 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
 
   for (int i0 = 0; i0 < n_patches; i0 += cmax) {
     const int n = n_patches - i0 < cmax ? n_patches - i0 : cmax;
-    g_n_base = i0;
+    ctx.n_base = i0;
     const void* x0;
     if (layout == HIPAC_LAYOUT_S2D16_BF16) {
       x0 = reinterpret_cast<const uint8_t*>(d_batch) + (size_t)i0 * kS2dBytes;
     } else {
       const uint16_t* src = reinterpret_cast<const uint16_t*>(d_batch) + (size_t)i0 * 224 * 224 * 3;
       {
-        ProfileScope ps("pack_s2d16", stream, (double)n * (224 * 224 * 3 * 2 + kS2dBytes));
-        k_pack_s2d16<<<g_num_sms * 8, 256, 0, stream>>>(src, reinterpret_cast<uint16_t*>(s2d), n);
+        ProfileScope ps("pack_s2d16", ctx.stream, (double)n * (224 * 224 * 3 * 2 + kS2dBytes));
+        k_pack_s2d16<<<ctx.sms * 8, 256, 0, ctx.stream>>>(src, reinterpret_cast<uint16_t*>(s2d), n);
       }
       count_launch(1);
       x0 = s2d;
     }
-    // the batch was written in ascending patch order, so the first layer walks it descending, the next ascending, ...
-    g_reverse = 1;
+    // the batch was written in ascending patch order, so the first launch of the chunk walks it descending, the next
+    // ascending, ...
+    int pos = 0;   // position of the next launch in the chunk
+    auto next = [&] {
+      Launch c = ctx;
+      c.reverse = pos++ % 2 == 0;
+      return c;
+    };
     auto conv = [&](int layer, const void* in, const void* res, void* out, bool relu) {
-      g_reverse ^= 1;
-      return run_conv(pk, L, layer, in, res, out, n, relu, stream);
+      return run_conv(next(), pk, L, layer, in, res, out, n, relu);
     };
     int e = 0;
-    if ((e = run_stem(pk, L, x0, A, n, stream))) return e;
+    if ((e = run_stem(next(), pk, L, x0, A, n))) return e;
     // layer1 (two basic blocks, identity shortcuts)
     if ((e = conv(1, A, nullptr, B, true)) || (e = conv(2, B, A, C, true))) return e;
     if ((e = conv(3, C, nullptr, B, true)) || (e = conv(4, B, C, A, true))) return e;
@@ -695,15 +629,14 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
     for (int s = 0; s < 3; s++) {
       const int l0 = 5 + 5 * s;
       if ((e = conv(l0, A, nullptr, B, true))) return e;           // 3x3 / stride 2
-      g_reverse ^= 1;
-      if ((e = run_conv_ds_fused(pk, L, s, B, A, C, n, stream))) return e;   // 3x3 + 1x1/s2 projection + ReLU, one accumulator
+      if ((e = run_conv_ds_fused(next(), pk, L, s, B, A, C, n))) return e;   // 3x3 + 1x1/s2 projection + ReLU, one accumulator
       if ((e = conv(l0 + 3, C, nullptr, B, true)) || (e = conv(l0 + 4, B, C, A, true))) return e;
     }
-    ProfileScope ps_pool("avgpool_fc", stream, (double)n * (49 * 512 * 2 + 512 * 4));
-    HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc, dim3(n), dim3(256), 0, stream, 1, reinterpret_cast<const __nv_bfloat16*>(A),
+    ProfileScope ps_pool("avgpool_fc", ctx.stream, (double)n * (49 * 512 * 2 + 512 * 4));
+    HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc, dim3(n), dim3(256), 0, ctx.stream, 1, reinterpret_cast<const __nv_bfloat16*>(A),
                                d_feats + (size_t)i0 * 512, d_logits ? d_logits + (size_t)i0 * num_classes : nullptr,
                                reinterpret_cast<const float*>(pk + L.fc_w_off), reinterpret_cast<const float*>(pk + L.fc_b_off),
-                               num_classes, g_n_dev, g_n_base));
+                               num_classes, ctx.n_dev, ctx.n_base));
     count_launch(1);
   }
   HIPAC_CHECK_CUDA(cudaGetLastError());

@@ -427,7 +427,7 @@ extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch
                                int capacity, void* d_workspace, size_t workspace_bytes, int mode, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   const int keep_all = (mode & HIPAC_SCAN_KEEP_ALL) ? 1 : 0;
-  g_stream_disable = (mode & HIPAC_SCAN_NO_STREAM) ? 1 : 0;
+  const bool allow_stream = !(mode & HIPAC_SCAN_NO_STREAM);   // HIPAC_SCAN_NO_STREAM: force the cp.async kernels (cross-check)
   mode &= ~(HIPAC_SCAN_KEEP_ALL | HIPAC_SCAN_NO_STREAM);
   int nx, ny;
   if (int e = scan_geometry(H, W, P, S, iy_begin, iy_end, &nx, &ny)) return e;
@@ -467,7 +467,7 @@ extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch
   HIPAC_REQUIRE(mode != HIPAC_SCAN_FUSED || fused_ok,
                 "fused scan needs stride % (P/224) == 0, gcd(stride, P) % 32 == 0 and a 16-byte aligned image");
   if (mode != HIPAC_SCAN_DIRECT && fused_ok) {
-    return fused_scan_impl(p, o, flags, src_idx, block_tot, d_coords, d_labels, d_count, capacity, ws, stream, keep_all);
+    return fused_scan_impl(p, o, flags, src_idx, block_tot, d_coords, d_labels, d_count, capacity, ws, stream, keep_all, allow_stream);
   }
   {
     ProfileScope ps("stats_direct", stream, 0.0);

@@ -650,10 +650,8 @@ static int launch_planes(const ScanParams& p, const FusedGeom& G, cudaStream_t s
 }
 
 // ---- streaming pass (tile_scan_stream.cuh) ----
-static thread_local int g_stream_disable = 0;   // HIPAC_SCAN_NO_STREAM: force the cp.async kernels (cross-check)
-
 static bool stream_applicable(const ScanParams& p, const FusedGeom& G) {
-  if (g_stream_disable || G.f == 1) return false;
+  if (G.f == 1) return false;
   if ((p.pitch & 15) || (reinterpret_cast<uintptr_t>(p.rgb) & 15)) return false;
   if (G.Sf < 2) return false;
   const int cols = kStripUnits * (8 / G.f);
@@ -698,7 +696,8 @@ static int launch_scan_planes(const ScanParams& p, const FusedGeom& G, cudaStrea
 }
 
 static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* flags, int32_t* src_idx, int32_t* block_tot, int32_t* d_coords,
-                           uint8_t* d_labels, int32_t* d_count, int capacity, uint8_t* ws, cudaStream_t stream, int keep_all) {
+                           uint8_t* d_labels, int32_t* d_count, int capacity, uint8_t* ws, cudaStream_t stream, int keep_all,
+                           bool allow_stream) {
   FusedGeom G;
   if (!fused_geometry(p, &G)) {
     set_error("fused scan not applicable to this stride / patch size");
@@ -717,7 +716,7 @@ static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* fla
   G.ws_hi = ws + 1024;   // the tail pad hipac_tile_scan_workspace_bytes adds (the gather reads whole aligned words)
   const int n_cand = p.nx * p.ny;
   HIPAC_CHECK_CUDA(cudaMemsetAsync(G.cell_sum, 0, 2 * cell_bytes, stream));
-  const bool stream_ok = stream_applicable(p, G);
+  const bool stream_ok = allow_stream && stream_applicable(p, G);
   if (stream_ok) {
     // one read of the image: cell sums + resampled planes; the lesion votes come from a mask-only pass
     if (int e = launch_scan_planes(p, G, stream)) return e;
