@@ -79,6 +79,44 @@ int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes,
                     void* d_workspace, size_t workspace_bytes,
                     int mode, void* stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Tissue segmentation (opt-in stage 1 background rejection; the reference has none, see SURVEY.md fact 1).  The CLAM-style
+ * recipe of CAMELYON16 pipelines on a low-resolution level, bit-exact against OpenCV 4.13's 8-bit code:
+ *   cv2.cvtColor(RGB2HSV) saturation -> cv2.medianBlur(S, ksize) (replicated borders) -> cv2.threshold(BINARY | OTSU),
+ * or a fixed threshold.  S = (d * sdiv[v] + 2048) >> 12 with v = max(R,G,B), d = v - min(R,G,B), sdiv[i] = round(255*4096/i);
+ * mask = blurred > t ? 255 : 0.
+ *   d_rgb        uint8 [H][pitch_bytes] RGB (channel order does not matter), pitch_bytes >= 3*W
+ *   ksize        1, 3, 5 or 7
+ *   threshold    -1 = Otsu's threshold of the blurred plane's histogram (OpenCV's fp64 loop), else t in [0, 255]
+ *   d_mask       uint8 [H][mask_pitch] output, 0 / 255
+ *   d_threshold  int32 [1] output: the t that was used (device memory; nothing waits on the host)
+ *   d_blur       uint8 [H][blur_pitch] output of the median blur, or NULL (kept in the workspace only)
+ *   d_workspace  >= hipac_tissue_workspace_bytes(H, W) bytes, 256-byte aligned
+ * Three kernels on `stream` (saturation + median + histogram, Otsu, binarize). */
+size_t hipac_tissue_workspace_bytes(int H, int W);
+int hipac_tissue_segment(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, int ksize, int threshold,
+                         uint8_t* d_mask, int64_t mask_pitch, int32_t* d_threshold,
+                         uint8_t* d_blur, int64_t blur_pitch,
+                         void* d_workspace, size_t workspace_bytes, void* stream);
+
+/* hipac_tile_scan with a tissue mask instead of the mean > 240 rule.  d_tissue: uint8 [tissue_h][tissue_pitch] (> 0 = tissue)
+ * at scale m = tissue_scale (1, 2, 4, 8, 16 or 32; S % m == 0 and P % m == 0): mask pixel (u, v) covers level pixels
+ * [v*m, v*m+m) x [u*m, u*m+m), row 0 = row 0 of d_rgb (a shard passes the mask rows of its own origin, a multiple of m).
+ * A candidate (x, y) survives iff at least min_tissue_pixels mask pixels > 0 lie inside [y/m, (y+P)/m) x [x/m, (x+P)/m);
+ * pixels outside the mask's extent count as background.  Everything else -- grid, emission order, labels, compaction,
+ * capacity, resample, HIPAC_SCAN_KEEP_ALL -- is as in hipac_tile_scan.
+ * d_workspace >= hipac_tile_scan_tissue_workspace_bytes(...) bytes, 256-byte aligned. */
+size_t hipac_tile_scan_tissue_workspace_bytes(int H, int W, int P, int S, int iy_begin, int iy_end, int mode, int tissue_scale);
+int hipac_tile_scan_tissue(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes,
+                           const uint8_t* d_mask, int64_t mask_pitch,
+                           int P, int S, int iy_begin, int iy_end,
+                           int32_t* d_coords, uint8_t* d_labels,
+                           uint8_t* d_batch_u8, void* d_batch, int layout,
+                           int32_t* d_count, int capacity,
+                           void* d_workspace, size_t workspace_bytes, int mode,
+                           const uint8_t* d_tissue, int tissue_h, int tissue_w, int64_t tissue_pitch,
+                           int tissue_scale, int min_tissue_pixels, void* stream);
+
 /* Early survivor count.  If a pinned host buffer int32[2] is registered (calling thread), every hipac_tile_scan copies
  * {survivors, candidates} into it right after the compaction kernel and records an event; hipac_tile_scan_wait_count
  * blocks only until that copy has landed -- the resample / gather kernels of the same call keep running, so the caller

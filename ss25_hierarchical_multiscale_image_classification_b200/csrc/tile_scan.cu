@@ -421,11 +421,32 @@ extern "C" size_t hipac_tile_scan_workspace_bytes(int H, int W, int P, int S, in
   return b + 1024;
 }
 
-extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask,
-                               int64_t mask_pitch, int P, int S, int iy_begin, int iy_end, int32_t* d_coords,
-                               uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch, int layout, int32_t* d_count,
-                               int capacity, void* d_workspace, size_t workspace_bytes, int mode, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+static int tissue_geometry(int P, int S, int m) {
+  HIPAC_REQUIRE(m == 1 || m == 2 || m == 4 || m == 8 || m == 16 || m == 32, "tissue_scale must be a power of two up to 32");
+  HIPAC_REQUIRE(S % m == 0 && P % m == 0, "stride and patch size must be multiples of tissue_scale");
+  return 0;
+}
+
+// bytes of the tissue cell grid, which precedes the hipac_tile_scan workspace layout (0 on error)
+static size_t tissue_cell_bytes(int H, int W, int P, int S, int iy_begin, int iy_end, int m) {
+  int nx, ny;
+  if (scan_geometry(H, W, P, S, iy_begin, iy_end, &nx, &ny) || tissue_geometry(P, S, m)) return 0;
+  if ((int64_t)nx * ny == 0) return 256;
+  int g, cy0, ncx, ncy;
+  tissue_cell_grid(S, P, iy_begin, nx, ny, &g, &cy0, &ncx, &ncy);
+  return align_up((size_t)ncx * ncy * 4, 256);
+}
+
+extern "C" size_t hipac_tile_scan_tissue_workspace_bytes(int H, int W, int P, int S, int iy_begin, int iy_end, int mode, int tissue_scale) {
+  const size_t cells = tissue_cell_bytes(H, W, P, S, iy_begin, iy_end, tissue_scale);
+  const size_t base = cells ? hipac_tile_scan_workspace_bytes(H, W, P, S, iy_begin, iy_end, mode) : 0;
+  return base ? cells + base : 0;
+}
+
+static int tile_scan_impl(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask, int64_t mask_pitch, int P,
+                          int S, int iy_begin, int iy_end, int32_t* d_coords, uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch,
+                          int layout, int32_t* d_count, int capacity, void* d_workspace, size_t workspace_bytes, int mode,
+                          TissueFilter* tissue, cudaStream_t stream) {
   const int keep_all = (mode & HIPAC_SCAN_KEEP_ALL) ? 1 : 0;
   const bool allow_stream = !(mode & HIPAC_SCAN_NO_STREAM);   // HIPAC_SCAN_NO_STREAM: force the cp.async kernels (cross-check)
   mode &= ~(HIPAC_SCAN_KEEP_ALL | HIPAC_SCAN_NO_STREAM);
@@ -462,18 +483,25 @@ extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch
     HIPAC_CHECK_CUDA(cudaMemsetAsync(d_count, 0, 8, stream));
     return publish_count(d_count, stream);
   }
+  if (tissue) {
+    tissue_cell_grid(S, P, iy_begin, nx, ny, &tissue->g, &tissue->cy0, &tissue->ncx, &tissue->ncy);
+    HIPAC_REQUIRE(tissue->ncy <= 65535, "too many tissue cell rows for one call; split the row range");
+  }
   FusedGeom geom;
   const bool fused_ok = n_cand > 0 && fused_geometry(p, &geom) && ((uintptr_t)d_rgb & 15) == 0;
   HIPAC_REQUIRE(mode != HIPAC_SCAN_FUSED || fused_ok,
                 "fused scan needs stride % (P/224) == 0, gcd(stride, P) % 32 == 0 and a 16-byte aligned image");
   if (mode != HIPAC_SCAN_DIRECT && fused_ok) {
-    return fused_scan_impl(p, o, flags, src_idx, block_tot, d_coords, d_labels, d_count, capacity, ws, stream, keep_all, allow_stream);
+    return fused_scan_impl(p, o, flags, src_idx, block_tot, d_coords, d_labels, d_count, capacity, ws, stream, keep_all, allow_stream,
+                           tissue);
   }
   {
     ProfileScope ps("stats_direct", stream, 0.0);
     k_stats_direct<<<n_cand, 256, 0, stream>>>(p, flags);
   }
   count_launch(1);
+  if (tissue)
+    if (int e = launch_tissue_filter(p, *tissue, flags, n_cand, stream)) return e;
   if (int e = launch_compact(p, flags, n_cand, d_coords, d_labels, src_idx, d_count, capacity, keep_all, block_tot, stream)) return e;
   if (int e = publish_count(d_count, stream)) return e;
   if ((d_batch_u8 || d_batch) && capacity > 0) {
@@ -484,6 +512,40 @@ extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch
   }
   HIPAC_CHECK_CUDA(cudaGetLastError());
   return 0;
+}
+
+extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask,
+                               int64_t mask_pitch, int P, int S, int iy_begin, int iy_end, int32_t* d_coords,
+                               uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch, int layout, int32_t* d_count,
+                               int capacity, void* d_workspace, size_t workspace_bytes, int mode, void* stream) {
+  return tile_scan_impl(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8, d_batch,
+                        layout, d_count, capacity, d_workspace, workspace_bytes, mode, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int hipac_tile_scan_tissue(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask,
+                                      int64_t mask_pitch, int P, int S, int iy_begin, int iy_end, int32_t* d_coords,
+                                      uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch, int layout, int32_t* d_count,
+                                      int capacity, void* d_workspace, size_t workspace_bytes, int mode, const uint8_t* d_tissue,
+                                      int tissue_h, int tissue_w, int64_t tissue_pitch, int tissue_scale, int min_tissue_pixels,
+                                      void* stream) {
+  if (int e = tissue_geometry(P, S, tissue_scale)) return e;
+  HIPAC_REQUIRE(tissue_h >= 0 && tissue_w >= 0, "negative tissue mask size");
+  HIPAC_REQUIRE(d_tissue || (int64_t)tissue_h * tissue_w == 0, "null tissue mask with a nonzero size");
+  HIPAC_REQUIRE(tissue_h == 0 || tissue_pitch >= tissue_w, "tissue mask pitch smaller than a row");
+  HIPAC_REQUIRE(min_tissue_pixels >= 0, "negative min_tissue_pixels");
+  const size_t cells = tissue_cell_bytes(H, W, P, S, iy_begin, iy_end, tissue_scale);
+  if (!cells) return -1;
+  HIPAC_REQUIRE(d_workspace, "null pointer");
+  HIPAC_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "workspace must be 256-byte aligned");
+  HIPAC_REQUIRE(workspace_bytes >= hipac_tile_scan_tissue_workspace_bytes(H, W, P, S, iy_begin, iy_end, mode, tissue_scale),
+                "workspace too small");
+  TissueFilter t{};
+  t.mask = d_tissue, t.h = d_tissue ? tissue_h : 0, t.w = d_tissue ? tissue_w : 0, t.pitch = tissue_pitch;
+  t.m = tissue_scale, t.min_pixels = min_tissue_pixels;
+  t.cells = reinterpret_cast<uint32_t*>(d_workspace);
+  return tile_scan_impl(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8, d_batch,
+                        layout, d_count, capacity, (uint8_t*)d_workspace + cells, workspace_bytes - cells, mode, &t,
+                        (cudaStream_t)stream);
 }
 
 extern "C" int hipac_upload_rows(void* d_dst, int64_t dst_pitch, const void* h_src, int64_t src_pitch, int64_t row_bytes,

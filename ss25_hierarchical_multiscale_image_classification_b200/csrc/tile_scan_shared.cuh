@@ -27,4 +27,19 @@ struct OutParams {
   int layout;
 };
 
+// Tissue-mask filter (tissue.cu): mask pixel (u, v) covers level pixels [u*m, u*m+m) x [v*m, v*m+m) of the call's image.
+struct TissueFilter {
+  const uint8_t* mask;  // [h][pitch], > 0 = tissue
+  int h, w;
+  int64_t pitch;
+  int m, min_pixels;
+  int g, cy0, ncx, ncy; // cells of g = gcd(S, P) level pixels: stored cell rows [cy0, cy0 + ncy), columns [0, ncx)
+  uint32_t* cells;      // [ncy][ncx] tissue pixel counts (workspace)
+};
+
+// The cell grid a candidate range [iy_begin, iy_begin + ny) x [0, nx) reads: every cell of every candidate footprint.
+void tissue_cell_grid(int S, int P, int iy_begin, int nx, int ny, int* g, int* cy0, int* ncx, int* ncy);
+// k_tissue_cells + k_tissue_flags: rewrites bit 0 of every flag with the tissue-mask rule (after the flag kernel).
+int launch_tissue_filter(const ScanParams& p, const TissueFilter& t, uint8_t* flags, int n_cand, cudaStream_t stream);
+
 }  // namespace hipac

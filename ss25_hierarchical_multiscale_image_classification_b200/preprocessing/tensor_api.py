@@ -8,8 +8,10 @@ buffers and moves pointers.  There is no CPU fallback.
 """
 from __future__ import annotations
 
+import math
 import threading
 from dataclasses import dataclass
+from fractions import Fraction
 
 import torch
 
@@ -151,24 +153,32 @@ def batch_shape(n: int, layout: str):
 def extract_patches_tensor(level_img: torch.Tensor, lesion_mask: torch.Tensor | None, level: int,
                            stride=None, row_range=None, patch_size: int = 224, layout: str | None = "s2d16",
                            want_u8: bool = False, mode: str = "auto", capacity: int | None = None,
-                           stream: torch.cuda.Stream | None = None, keep_all: bool = False) -> PatchBatch:
+                           stream: torch.cuda.Stream | None = None, keep_all: bool = False, tissue: torch.Tensor | None = None,
+                           tissue_scale: int = 1, min_tissue=0.5) -> PatchBatch:
     """``extract_patches_enqueue(...).resolve()``: see there."""
     return extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=row_range, patch_size=patch_size,
                                    layout=layout, want_u8=want_u8, mode=mode, capacity=capacity, stream=stream,
-                                   keep_all=keep_all).resolve()
+                                   keep_all=keep_all, tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue).resolve()
 
 
 def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor | None, level: int,
                             stride=None, row_range=None, patch_size: int = 224, layout: str | None = "s2d16",
                             want_u8: bool = False, mode: str = "auto", capacity: int | None = None,
-                            stream: torch.cuda.Stream | None = None, keep_all: bool = False) -> PendingPatchBatch:
+                            stream: torch.cuda.Stream | None = None, keep_all: bool = False, tissue: torch.Tensor | None = None,
+                            tissue_scale: int = 1, min_tissue=0.5) -> PendingPatchBatch:
     """Tile one level image (uint8 ``[H,W,3]`` on a CUDA device) exactly as the reference does.
 
     ``lesion_mask``: uint8 ``[H,W]`` (>0 = lesion, the rasterised ``parse_xml_mask`` output,
     reference ``src/main.py:372-410``) or ``None`` -> every patch "normal" (``src/main.py:714-716``).
     ``row_range=(i0,i1)`` restricts to candidate grid rows ``y//stride in [i0,i1)`` -- the
     multi-GPU shard unit.  ``keep_all`` disables the tissue rejection (used on stacks of already
-    extracted patches).  Nothing blocks: the call returns capacity-sized tensors and the device-side survivor
+    extracted patches).
+
+    ``tissue``: a tissue mask (uint8 ``[h, w]`` CUDA tensor, > 0 = tissue, e.g. ``tissue.segment_tissue`` of a coarser
+    level) at ``tissue_scale`` m in {1, 2, 4, 8, 16, 32}: mask pixel ``(u, v)`` covers level pixels ``[u*m, u*m+m) x
+    [v*m, v*m+m)`` of ``level_img``.  A candidate then survives iff at least ``ceil(min_tissue * (P/m)^2)`` mask pixels of
+    its footprint are tissue (mask pixels beyond the mask count as background), instead of the reference's ``mean > 240``
+    rule; ``keep_all`` still overrides.  Nothing blocks: the call returns capacity-sized tensors and the device-side survivor
     counter; ``resolve()`` waits only until the count is known (after the compaction kernel) and slices, and
     ``features.classify_tensor(..., count=pending.count)`` consumes the batch without any host round trip.
     """
@@ -185,6 +195,16 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
         if lesion_mask.stride(1) != 1:
             lesion_mask = lesion_mask.contiguous()
     P, S = patch_and_stride(level, stride, patch_size)
+    if tissue is not None:
+        if not (tissue.is_cuda and tissue.dtype == torch.uint8 and tissue.dim() == 2 and tissue.device == level_img.device):
+            raise ValueError("tissue must be a uint8 [h, w] tensor on the level image's device")
+        if tissue_scale not in (1, 2, 4, 8, 16, 32) or S % tissue_scale or P % tissue_scale:
+            raise ValueError(f"tissue_scale {tissue_scale} must be a power of two up to 32 dividing the stride {S} and patch {P}")
+        if not 0 <= min_tissue <= 1:
+            raise ValueError("min_tissue must be a fraction in [0, 1]")
+        if tissue.stride(1) != 1:
+            tissue = tissue.contiguous()
+        min_pixels = math.ceil(Fraction(min_tissue) * (P // tissue_scale) ** 2)
     if P > OUT and mode != "direct":
         # the read-once streaming pass wants 16-byte aligned rows; anything else would silently take the two-pass kernels
         with torch.cuda.device(level_img.device), torch.cuda.stream(stream or torch.cuda.current_stream(level_img.device)):
@@ -207,20 +227,25 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
         batch = torch.empty(batch_shape(max(cap, 1), layout), dtype=torch.bfloat16, device=dev) if layout else None
         u8 = torch.empty((max(cap, 1), OUT, OUT, 3), dtype=torch.uint8, device=dev) if want_u8 else None
         m = _MODES[mode] | (_lib.SCAN_KEEP_ALL if keep_all else 0)
-        ws_bytes = l.hipac_tile_scan_workspace_bytes(H, W, P, S, i0, i1, m)
+        ws_bytes = (l.hipac_tile_scan_workspace_bytes(H, W, P, S, i0, i1, m) if tissue is None else
+                    l.hipac_tile_scan_tissue_workspace_bytes(H, W, P, S, i0, i1, m, tissue_scale))
         if ws_bytes == 0:
             raise RuntimeError("hipac_tile_scan_workspace_bytes: " + l.hipac_last_error().decode())
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
         h_count = _pinned_count()
-        rc = l.hipac_tile_scan(
-            level_img.data_ptr(), H, W, pitch,
-            lesion_mask.data_ptr() if lesion_mask is not None else None,
-            int(lesion_mask.stride(0)) if lesion_mask is not None else 0,
-            P, S, i0, i1, coords.data_ptr(), labels.data_ptr(),
-            u8.data_ptr() if u8 is not None else None,
-            batch.data_ptr() if batch is not None else None, _LAYOUTS[layout] if layout else 0,
-            count.data_ptr(), cap, ws.data_ptr(), ws_bytes, m, st.cuda_stream)
-        _lib.check(rc, "hipac_tile_scan")
+        args = (level_img.data_ptr(), H, W, pitch,
+                lesion_mask.data_ptr() if lesion_mask is not None else None,
+                int(lesion_mask.stride(0)) if lesion_mask is not None else 0,
+                P, S, i0, i1, coords.data_ptr(), labels.data_ptr(),
+                u8.data_ptr() if u8 is not None else None,
+                batch.data_ptr() if batch is not None else None, _LAYOUTS[layout] if layout else 0,
+                count.data_ptr(), cap, ws.data_ptr(), ws_bytes, m)
+        if tissue is None:
+            _lib.check(l.hipac_tile_scan(*args, st.cuda_stream), "hipac_tile_scan")
+        else:
+            th, tw = int(tissue.shape[0]), int(tissue.shape[1])
+            _lib.check(l.hipac_tile_scan_tissue(*args, tissue.data_ptr() if th * tw else None, th, tw, int(tissue.stride(0)),
+                                                tissue_scale, min_pixels, st.cuda_stream), "hipac_tile_scan_tissue")
         ws.record_stream(st)
     del h_count   # registered with the library; read in resolve()
     _count_host.seq = getattr(_count_host, "seq", 0) + 1
