@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define HIPAC_ABI_VERSION 1
+#define HIPAC_ABI_VERSION 2
 
 /* batch layouts written by hipac_tile_scan / consumed by hipac_resnet18_forward */
 #define HIPAC_LAYOUT_NHWC3_BF16 1 /* bf16 [N,224,224,3], (u8/255-mean)/std, the reference's tensor (src/main.py:815-816) in NHWC */
@@ -197,21 +197,30 @@ int hipac_resnet18_forward_dcount(const void* d_packed, int num_classes,
                                   float* d_feats, float* d_logits,
                                   void* d_workspace, size_t workspace_bytes, int chunk, void* stream);
 
+/* The three test hooks below run one stage-2 kernel with the launch state the forward gives it:
+ *   reverse  nonzero: walk the tiles from the last to the first (the forward alternates the order from launch to launch);
+ *   d_count  NULL: work on all n_patches patches; else device-count mode as in hipac_resnet18_forward_dcount, the kernel
+ *            reads d_count[0] when it starts and works on clamp(d_count[0] - n_base, 0, n_patches) patches, leaving the
+ *            output rows of the others untouched;
+ *   n_base   >= 0: index of the first patch of d_in in the count (the forward's chunk offset).
+ * The output does not depend on `reverse`. */
+
 /* Test hook: one conv layer of the network on its own (layer index 1..19 in network order, except 7), bf16 NHWC in/out,
  * optional residual.  Used by the per-layer parity tests.  Layer 0 (conv1) exists only fused with the max pool and layer 7
  * (layer2.0's projection shortcut) only fused into layer2.0.conv2: both are refused with -1, see hipac_resnet18_stem and
  * hipac_resnet18_conv_ds_fused. */
 int hipac_resnet18_conv_layer(const void* d_packed, int num_classes, int layer,
                               const void* d_in, const void* d_residual, void* d_out,
-                              int n_patches, int relu, void* stream);
+                              int n_patches, int relu, void* stream, int reverse, const int32_t* d_count, int n_base);
 
 /* Test hook: conv2 of layer{2,3,4}.0 with its 1x1/stride-2 projection shortcut fused into the same accumulator:
  * out = relu(conv3x3(d_in) + bn + conv1x1_s2(d_block_in) + bn); stage 0/1/2 = layer2/3/4. */
 int hipac_resnet18_conv_ds_fused(const void* d_packed, int num_classes, int stage, const void* d_in, const void* d_block_in,
-                                 void* d_out, int n_patches, void* stream);
+                                 void* d_out, int n_patches, void* stream, int reverse, const int32_t* d_count, int n_base);
 
 /* Test hook: the fused stem (conv1 + folded BN + ReLU + 3x3/s2 max pool): S2D16 batch -> bf16 [n][56][56][64]. */
-int hipac_resnet18_stem(const void* d_packed, int num_classes, const void* d_in, void* d_out, int n_patches, void* stream);
+int hipac_resnet18_stem(const void* d_packed, int num_classes, const void* d_in, void* d_out, int n_patches, void* stream,
+                        int reverse, const int32_t* d_count, int n_base);
 
 /* ---------------------------------------------------------------------------------------
  * The exchange step (SURVEY.md section 8e): per-segment survivors -> ONE canonically ordered result.

@@ -149,9 +149,9 @@ def _declare(l):
     l.hipac_resnet18_forward_dcount.restype = i32
     l.hipac_resnet18_forward_dcount.argtypes = [vp, i32, vp, i32, i32, vp, vp, vp, vp, sz, i32, vp]
     l.hipac_resnet18_conv_ds_fused.restype = i32
-    l.hipac_resnet18_conv_ds_fused.argtypes = [vp, i32, i32, vp, vp, vp, i32, vp]
+    l.hipac_resnet18_conv_ds_fused.argtypes = [vp, i32, i32, vp, vp, vp, i32, vp, i32, vp, i32]
     l.hipac_resnet18_stem.restype = i32
-    l.hipac_resnet18_stem.argtypes = [vp, i32, vp, vp, i32, vp]
+    l.hipac_resnet18_stem.argtypes = [vp, i32, vp, vp, i32, vp, i32, vp, i32]
     l.hipac_exchange_row_bytes.restype = sz
     l.hipac_exchange_row_bytes.argtypes = [i32, i32]
     l.hipac_exchange_segment_bytes.restype = sz
@@ -183,7 +183,7 @@ def _declare(l):
     l.hipac_profile_report.restype = C.c_longlong
     l.hipac_profile_report.argtypes = [C.c_char_p, sz]
     l.hipac_resnet18_conv_layer.restype = i32
-    l.hipac_resnet18_conv_layer.argtypes = [vp, i32, i32, vp, vp, vp, i32, i32, vp]
+    l.hipac_resnet18_conv_layer.argtypes = [vp, i32, i32, vp, vp, vp, i32, i32, vp, i32, vp, i32]
 
 
 EXPORTS = [

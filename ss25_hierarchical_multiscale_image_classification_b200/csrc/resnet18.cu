@@ -212,7 +212,7 @@ static int init_driver_api() {
 }
 
 // What a stage-2 launch needs besides its operands.  Each C entry point builds one and passes it down; forward_impl
-// sets n_base per chunk and reverse per launch.
+// sets n_base per chunk and reverse per launch, the test hooks take all three from their caller.
 struct Launch {
   cudaStream_t stream;
   int sms;            // SM count of the current device
@@ -531,40 +531,45 @@ extern "C" size_t hipac_resnet18_workspace_bytes(int n_patches, int chunk) {
 }
 
 extern "C" int hipac_resnet18_conv_layer(const void* d_packed, int num_classes, int layer, const void* d_in,
-                                         const void* d_residual, void* d_out, int n_patches, int relu, void* stream_) {
+                                         const void* d_residual, void* d_out, int n_patches, int relu, void* stream_, int reverse,
+                                         const int32_t* d_count, int n_base) {
   HIPAC_REQUIRE(d_packed && d_in && d_out, "null pointer");
   HIPAC_REQUIRE(layer >= 0 && layer < HIPAC_RESNET18_NUM_CONVS, "layer index out of range");
   HIPAC_REQUIRE(layer != 0, "layer 0 (conv1) runs only fused with the max pool: use hipac_resnet18_stem");
   HIPAC_REQUIRE(layer != 7, "layer 7 (layer2.0.downsample) runs only fused into layer2.0.conv2: use hipac_resnet18_conv_ds_fused");
   HIPAC_REQUIRE(n_patches > 0, "n_patches must be positive");
+  HIPAC_REQUIRE(n_base >= 0, "n_base must be non-negative");
   int sms = 0;
   if (int e = init_driver_api()) return e;
   if (int e = device_sm_count(&sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
-  return run_conv({(cudaStream_t)stream_, sms, nullptr, 0, 0}, reinterpret_cast<const uint8_t*>(d_packed), L, layer, d_in, d_residual,
-                  d_out, n_patches, relu != 0);
+  return run_conv({(cudaStream_t)stream_, sms, d_count, n_base, reverse != 0}, reinterpret_cast<const uint8_t*>(d_packed), L, layer,
+                  d_in, d_residual, d_out, n_patches, relu != 0);
 }
 
 extern "C" int hipac_resnet18_conv_ds_fused(const void* d_packed, int num_classes, int stage, const void* d_in, const void* d_block_in,
-                                            void* d_out, int n_patches, void* stream_) {
+                                            void* d_out, int n_patches, void* stream_, int reverse, const int32_t* d_count, int n_base) {
   HIPAC_REQUIRE(d_packed && d_in && d_block_in && d_out && n_patches > 0, "bad arguments");
   HIPAC_REQUIRE(stage >= 0 && stage < 3, "stage must be 0 (layer2), 1 (layer3) or 2 (layer4)");
+  HIPAC_REQUIRE(n_base >= 0, "n_base must be non-negative");
   int sms = 0;
   if (int e = init_driver_api()) return e;
   if (int e = device_sm_count(&sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
-  return run_conv_ds_fused({(cudaStream_t)stream_, sms, nullptr, 0, 0}, reinterpret_cast<const uint8_t*>(d_packed), L, stage, d_in,
-                           d_block_in, d_out, n_patches);
+  return run_conv_ds_fused({(cudaStream_t)stream_, sms, d_count, n_base, reverse != 0}, reinterpret_cast<const uint8_t*>(d_packed), L,
+                           stage, d_in, d_block_in, d_out, n_patches);
 }
 
 extern "C" int hipac_resnet18_stem(const void* d_packed, int num_classes, const void* d_in, void* d_out, int n_patches,
-                                   void* stream_) {
+                                   void* stream_, int reverse, const int32_t* d_count, int n_base) {
   HIPAC_REQUIRE(d_packed && d_in && d_out && n_patches > 0, "bad arguments");
+  HIPAC_REQUIRE(n_base >= 0, "n_base must be non-negative");
   int sms = 0;
   if (int e = init_driver_api()) return e;
   if (int e = device_sm_count(&sms)) return e;
   const PackedLayout L = packed_layout(num_classes);
-  return run_stem({(cudaStream_t)stream_, sms, nullptr, 0, 0}, reinterpret_cast<const uint8_t*>(d_packed), L, d_in, d_out, n_patches);
+  return run_stem({(cudaStream_t)stream_, sms, d_count, n_base, reverse != 0}, reinterpret_cast<const uint8_t*>(d_packed), L, d_in,
+                  d_out, n_patches);
 }
 
 static int forward_impl(const void* d_packed, int num_classes, const void* d_batch, int layout, int n_patches,

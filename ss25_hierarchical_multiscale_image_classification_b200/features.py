@@ -119,41 +119,69 @@ def classify_tensor(batch: torch.Tensor, packed: PackedResNet18, chunk: int = 40
     return _forward(batch, packed, True, chunk, stream, count)
 
 
-def conv_layer(packed: PackedResNet18, layer: int, x: torch.Tensor, residual: torch.Tensor | None, relu: bool):
+def _launch_state(count: torch.Tensor | None, base: int):
+    """The trailing (d_count, n_base) arguments of the test hooks: host count when ``count`` is None."""
+    if count is None:
+        return None, int(base)
+    if not (count.is_cuda and count.dtype == torch.int32 and count.numel() >= 1):
+        raise ValueError("count must be a CUDA int32 tensor")
+    return count.data_ptr(), int(base)
+
+
+def _hook_out(out: torch.Tensor | None, shape, device) -> torch.Tensor:
+    if out is None:
+        return torch.empty(shape, dtype=torch.bfloat16, device=device)
+    if not (out.dtype == torch.bfloat16 and tuple(out.shape) == tuple(shape) and out.is_contiguous() and out.device == device):
+        raise ValueError(f"out must be a contiguous bf16 tensor of shape {tuple(shape)} on {device}")
+    return out
+
+
+def conv_layer(packed: PackedResNet18, layer: int, x: torch.Tensor, residual: torch.Tensor | None, relu: bool, *,
+               reverse: bool = False, count: torch.Tensor | None = None, base: int = 0, out: torch.Tensor | None = None):
     """Test hook: run one conv(+folded BN)(+residual)(+ReLU) layer on bf16 NHWC input.  Layers 0 and 7 exist only fused
-    (``stem``, ``conv_ds_fused``): the library refuses them, and out-of-range indices, with a RuntimeError."""
+    (``stem``, ``conv_ds_fused``): the library refuses them, and out-of-range indices, with a RuntimeError.
+
+    The keywords give the kernel the launch state the forward uses: ``reverse`` walks the tiles from the last to the
+    first; ``count`` (int32 device tensor) switches to device-count mode, where the kernel works on
+    ``clamp(count[0] - base, 0, n)`` patches and leaves the other rows of ``out`` untouched; ``out`` is written in
+    place instead of a fresh tensor."""
     l = _lib.lib()
     cout_hout = {**{i: (64, 56) for i in range(1, 5)}, **{i: (128, 28) for i in range(5, 10)},
                  **{i: (256, 14) for i in range(10, 15)}, **{i: (512, 7) for i in range(15, 20)}}
     cout, hout = cout_hout.get(layer, (1, 1))   # placeholder output for a layer the library refuses
     n = int(x.shape[0])
-    out = torch.empty((n, hout, hout, cout), dtype=torch.bfloat16, device=x.device)
+    out = _hook_out(out, (n, hout, hout, cout), x.device)
+    d_count, n_base = _launch_state(count, base)
     st = torch.cuda.current_stream(x.device)
     rc = l.hipac_resnet18_conv_layer(packed.blob.data_ptr(), packed.num_classes, layer, x.contiguous().data_ptr(),
                                      residual.contiguous().data_ptr() if residual is not None else None,
-                                     out.data_ptr(), n, int(relu), st.cuda_stream)
+                                     out.data_ptr(), n, int(relu), st.cuda_stream, int(reverse), d_count, n_base)
     _lib.check(rc, "hipac_resnet18_conv_layer")
     return out
 
 
-def stem(packed: PackedResNet18, x: torch.Tensor) -> torch.Tensor:
-    """Test hook: fused conv1 + BN + ReLU + max pool on an S2D16 batch -> bf16 ``[n,56,56,64]``."""
+def stem(packed: PackedResNet18, x: torch.Tensor, *, reverse: bool = False, count: torch.Tensor | None = None, base: int = 0,
+         out: torch.Tensor | None = None) -> torch.Tensor:
+    """Test hook: fused conv1 + BN + ReLU + max pool on an S2D16 batch -> bf16 ``[n,56,56,64]`` (keywords: ``conv_layer``)."""
     l = _lib.lib()
     n = int(x.shape[0])
-    out = torch.empty((n, 56, 56, 64), dtype=torch.bfloat16, device=x.device)
+    out = _hook_out(out, (n, 56, 56, 64), x.device)
+    d_count, n_base = _launch_state(count, base)
     rc = l.hipac_resnet18_stem(packed.blob.data_ptr(), packed.num_classes, x.contiguous().data_ptr(), out.data_ptr(), n,
-                               torch.cuda.current_stream(x.device).cuda_stream)
+                               torch.cuda.current_stream(x.device).cuda_stream, int(reverse), d_count, n_base)
     _lib.check(rc, "hipac_resnet18_stem")
     return out
 
 
-def conv_ds_fused(packed: PackedResNet18, stage: int, x: torch.Tensor, block_in: torch.Tensor) -> torch.Tensor:
-    """Test hook: conv2 of layer{2,3,4}.0 + fused 1x1/s2 projection shortcut + ReLU (stage 0/1/2)."""
+def conv_ds_fused(packed: PackedResNet18, stage: int, x: torch.Tensor, block_in: torch.Tensor, *, reverse: bool = False,
+                  count: torch.Tensor | None = None, base: int = 0, out: torch.Tensor | None = None) -> torch.Tensor:
+    """Test hook: conv2 of layer{2,3,4}.0 + fused 1x1/s2 projection shortcut + ReLU (stage 0/1/2; keywords: ``conv_layer``)."""
     l = _lib.lib()
     n, cout, hout = int(x.shape[0]), (128, 256, 512)[stage], (28, 14, 7)[stage]
-    out = torch.empty((n, hout, hout, cout), dtype=torch.bfloat16, device=x.device)
+    out = _hook_out(out, (n, hout, hout, cout), x.device)
+    d_count, n_base = _launch_state(count, base)
     rc = l.hipac_resnet18_conv_ds_fused(packed.blob.data_ptr(), packed.num_classes, stage, x.contiguous().data_ptr(),
                                         block_in.contiguous().data_ptr(), out.data_ptr(), n,
-                                        torch.cuda.current_stream(x.device).cuda_stream)
+                                        torch.cuda.current_stream(x.device).cuda_stream, int(reverse), d_count, n_base)
     _lib.check(rc, "hipac_resnet18_conv_ds_fused")
     return out

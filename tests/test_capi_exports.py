@@ -21,7 +21,7 @@ def test_library_exports_every_declared_symbol(built_lib):
     assert set(syms) == set(_lib.EXPORTS)
     for s in syms:
         assert hasattr(built_lib, s), s
-    assert built_lib.hipac_abi_version() == 1
+    assert built_lib.hipac_abi_version() == 2
 
 
 def test_pillow_coeff_tables_equal_oracle(built_lib):
