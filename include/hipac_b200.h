@@ -117,6 +117,42 @@ int hipac_tile_scan_tissue(const uint8_t* d_rgb, int H, int W, int64_t pitch_byt
                            const uint8_t* d_tissue, int tissue_h, int tissue_w, int64_t tissue_pitch,
                            int tissue_scale, int min_tissue_pixels, void* stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Coarse-to-fine cascade: tile a finer level only where a coarser level's classifier fires.
+ * Levels are exact powers of two; the coarse level Lc and the fine level Lf < Lc differ by shift = Lc - Lf >= 1.
+ *
+ * hipac_roi_grid  builds the ROI: uint8 d_grid [ny][nx] over the coarse CANDIDATE grid (nx, ny = the coarse level's grid
+ *                 shape at `stride`), cell (i, j) = 1 iff some survivor s < min(d_count[0], capacity) with
+ *                 d_scores[s] >= threshold has its cell (x / stride, y / stride) within Chebyshev distance `dilate`
+ *                 (cells) of (i, j); 0 otherwise.  d_coords int32 [capacity][2], d_scores float [capacity] (e.g.
+ *                 logits[:,1] - logits[:,0] with threshold = log(tau / (1 - tau))).  d_count is read on the device (the
+ *                 tile scan's survivor counter): nothing waits on the host.  Two kernels (clear, scatter) on `stream`.
+ *                 hipac_roi_grid_bytes(nx, ny) = nx * ny.
+ * hipac_tile_scan_roi  hipac_tile_scan_tissue (tissue_scale > 0) or hipac_tile_scan (tissue_scale = 0: no tissue mask, the
+ *                 mean > 240 rule; the tissue arguments are ignored), then the ROI test ANDed into the keep bit before the
+ *                 compaction.  A candidate at fine pixel (x, y_origin + y) -- y_origin = fine-level row of d_rgb's row 0 --
+ *                 is in the ROI iff its footprint [x, x+P) x [y, y+P) (white-padded border patches included) overlaps with
+ *                 positive area the footprint [i*roi_stride << shift, (i*roi_stride + roi_patch) << shift) (same on y) of
+ *                 at least one set cell of d_roi [roi_ny][roi_nx] (shift = roi_level_shift; cells outside the grid are
+ *                 not set).  Grid, emission order, labels, capacity, resample and d_count[1] (= candidates of the row
+ *                 range) are as in hipac_tile_scan.  HIPAC_SCAN_KEEP_ALL is refused.
+ *                 d_workspace >= hipac_tile_scan_roi_workspace_bytes(...) bytes, 256-byte aligned. */
+size_t hipac_roi_grid_bytes(int nx, int ny);
+int hipac_roi_grid(const int32_t* d_coords, const float* d_scores, const int32_t* d_count, int capacity, float threshold,
+                   int stride, int nx, int ny, int dilate, uint8_t* d_grid, void* stream);
+size_t hipac_tile_scan_roi_workspace_bytes(int H, int W, int P, int S, int iy_begin, int iy_end, int mode, int tissue_scale);
+int hipac_tile_scan_roi(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes,
+                        const uint8_t* d_mask, int64_t mask_pitch,
+                        int P, int S, int iy_begin, int iy_end,
+                        int32_t* d_coords, uint8_t* d_labels,
+                        uint8_t* d_batch_u8, void* d_batch, int layout,
+                        int32_t* d_count, int capacity,
+                        void* d_workspace, size_t workspace_bytes, int mode,
+                        const uint8_t* d_tissue, int tissue_h, int tissue_w, int64_t tissue_pitch,
+                        int tissue_scale, int min_tissue_pixels,
+                        const uint8_t* d_roi, int roi_nx, int roi_ny, int roi_level_shift, int roi_stride, int roi_patch,
+                        int64_t y_origin, void* stream);
+
 /* Early survivor count.  If a pinned host buffer int32[2] is registered (calling thread), every hipac_tile_scan copies
  * {survivors, candidates} into it right after the compaction kernel and records an event; hipac_tile_scan_wait_count
  * blocks only until that copy has landed -- the resample / gather kernels of the same call keep running, so the caller

@@ -5,5 +5,6 @@ Mirrors the reference's entry points (anacarsi/ss25_Hierarchical_Multiscale_Imag
 reached through the C ABI in ``include/hipac_b200.h``.
 """
 from . import _lib  # noqa: F401
+from .cascade import RoiGrid, process_cascade, roi_grid, threshold_of, tumor_margin  # noqa: F401
 
 __version__ = "0.1.0"

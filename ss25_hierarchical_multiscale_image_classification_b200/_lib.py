@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "libhipac_b200.so")
 # the same library with -DHIPAC_DEBUG_BOUNDS (device-side bounds assertions in the stage-1 kernels); loaded instead of
 # LIB_PATH when HIPAC_DEBUG_BOUNDS=1 is in the environment (tests/test_debug_bounds_gpu.py runs it in a subprocess)
 DBG_LIB_PATH = os.path.join(_HERE, "libhipac_b200_dbg.so")
-SOURCES = ["capi.cu", "tile_scan.cu", "resnet18.cu", "exchange.cu", "polygon.cu", "mil.cu", "debug_umma.cu", "tissue.cu"]
+SOURCES = ["capi.cu", "tile_scan.cu", "resnet18.cu", "exchange.cu", "polygon.cu", "mil.cu", "debug_umma.cu", "tissue.cu", "cascade.cu"]
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "hipac_b200.h")
 
 LAYOUT_NHWC3_BF16 = 1
@@ -124,6 +124,15 @@ def _declare(l):
     l.hipac_tile_scan_tissue.restype = i32
     l.hipac_tile_scan_tissue.argtypes = [vp, i32, i32, i64, vp, i64, i32, i32, i32, i32, vp, vp, vp, vp, i32, vp, i32,
                                          vp, sz, i32, vp, i32, i32, i64, i32, i32, vp]
+    l.hipac_tile_scan_roi_workspace_bytes.restype = sz
+    l.hipac_tile_scan_roi_workspace_bytes.argtypes = [i32] * 8
+    l.hipac_tile_scan_roi.restype = i32
+    l.hipac_tile_scan_roi.argtypes = [vp, i32, i32, i64, vp, i64, i32, i32, i32, i32, vp, vp, vp, vp, i32, vp, i32,
+                                      vp, sz, i32, vp, i32, i32, i64, i32, i32, vp, i32, i32, i32, i32, i32, i64, vp]
+    l.hipac_roi_grid_bytes.restype = sz
+    l.hipac_roi_grid_bytes.argtypes = [i32, i32]
+    l.hipac_roi_grid.restype = i32
+    l.hipac_roi_grid.argtypes = [vp, vp, vp, i32, C.c_float, i32, i32, i32, i32, vp, vp]
     l.hipac_tissue_workspace_bytes.restype = sz
     l.hipac_tissue_workspace_bytes.argtypes = [i32, i32]
     l.hipac_tissue_segment.restype = i32
@@ -194,6 +203,7 @@ EXPORTS = [
     "hipac_exchange_pack", "hipac_exchange_merge", "hipac_polygon_workspace_bytes", "hipac_polygon_fill", "hipac_polygon_overflowed", "hipac_mil_packed_floats", "hipac_mil_pack", "hipac_mil_workspace_bytes", "hipac_mil_forward",
     "hipac_profile_enable", "hipac_profile_report", "hipac_debug_umma_shift", "hipac_resnet18_stem", "hipac_resnet18_conv_ds_fused",
     "hipac_tile_scan_tissue_workspace_bytes", "hipac_tile_scan_tissue", "hipac_tissue_workspace_bytes", "hipac_tissue_segment",
+    "hipac_roi_grid_bytes", "hipac_roi_grid", "hipac_tile_scan_roi_workspace_bytes", "hipac_tile_scan_roi",
 ]
 
 

@@ -446,7 +446,7 @@ extern "C" size_t hipac_tile_scan_tissue_workspace_bytes(int H, int W, int P, in
 static int tile_scan_impl(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask, int64_t mask_pitch, int P,
                           int S, int iy_begin, int iy_end, int32_t* d_coords, uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch,
                           int layout, int32_t* d_count, int capacity, void* d_workspace, size_t workspace_bytes, int mode,
-                          TissueFilter* tissue, cudaStream_t stream) {
+                          TissueFilter* tissue, const RoiFilter* roi, cudaStream_t stream) {
   const int keep_all = (mode & HIPAC_SCAN_KEEP_ALL) ? 1 : 0;
   const bool allow_stream = !(mode & HIPAC_SCAN_NO_STREAM);   // HIPAC_SCAN_NO_STREAM: force the cp.async kernels (cross-check)
   mode &= ~(HIPAC_SCAN_KEEP_ALL | HIPAC_SCAN_NO_STREAM);
@@ -462,6 +462,7 @@ static int tile_scan_impl(const uint8_t* d_rgb, int H, int W, int64_t pitch_byte
   HIPAC_REQUIRE(workspace_bytes >= hipac_tile_scan_workspace_bytes(H, W, P, S, iy_begin, iy_end, mode), "workspace too small");
   HIPAC_REQUIRE((int64_t)nx * ny < (int64_t)1 << 30, "too many candidates for one call; split the row range");
   HIPAC_REQUIRE(mode == HIPAC_SCAN_AUTO || mode == HIPAC_SCAN_DIRECT || mode == HIPAC_SCAN_FUSED, "unknown scan mode");
+  HIPAC_REQUIRE(!(keep_all && roi), "HIPAC_SCAN_KEEP_ALL cannot be combined with an ROI");
   if (int e = upload_constants(stream)) return e;
 
   ScanParams p;
@@ -493,7 +494,7 @@ static int tile_scan_impl(const uint8_t* d_rgb, int H, int W, int64_t pitch_byte
                 "fused scan needs stride % (P/224) == 0, gcd(stride, P) % 32 == 0 and a 16-byte aligned image");
   if (mode != HIPAC_SCAN_DIRECT && fused_ok) {
     return fused_scan_impl(p, o, flags, src_idx, block_tot, d_coords, d_labels, d_count, capacity, ws, stream, keep_all, allow_stream,
-                           tissue);
+                           tissue, roi);
   }
   {
     ProfileScope ps("stats_direct", stream, 0.0);
@@ -502,6 +503,8 @@ static int tile_scan_impl(const uint8_t* d_rgb, int H, int W, int64_t pitch_byte
   count_launch(1);
   if (tissue)
     if (int e = launch_tissue_filter(p, *tissue, flags, n_cand, stream)) return e;
+  if (roi)
+    if (int e = launch_roi_filter(p, *roi, flags, n_cand, stream)) return e;
   if (int e = launch_compact(p, flags, n_cand, d_coords, d_labels, src_idx, d_count, capacity, keep_all, block_tot, stream)) return e;
   if (int e = publish_count(d_count, stream)) return e;
   if ((d_batch_u8 || d_batch) && capacity > 0) {
@@ -519,15 +522,19 @@ extern "C" int hipac_tile_scan(const uint8_t* d_rgb, int H, int W, int64_t pitch
                                uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch, int layout, int32_t* d_count,
                                int capacity, void* d_workspace, size_t workspace_bytes, int mode, void* stream) {
   return tile_scan_impl(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8, d_batch,
-                        layout, d_count, capacity, d_workspace, workspace_bytes, mode, nullptr, (cudaStream_t)stream);
+                        layout, d_count, capacity, d_workspace, workspace_bytes, mode, nullptr, nullptr, (cudaStream_t)stream);
 }
 
-extern "C" int hipac_tile_scan_tissue(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask,
-                                      int64_t mask_pitch, int P, int S, int iy_begin, int iy_end, int32_t* d_coords,
-                                      uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch, int layout, int32_t* d_count,
-                                      int capacity, void* d_workspace, size_t workspace_bytes, int mode, const uint8_t* d_tissue,
-                                      int tissue_h, int tissue_w, int64_t tissue_pitch, int tissue_scale, int min_tissue_pixels,
-                                      void* stream) {
+// hipac_tile_scan_tissue and hipac_tile_scan_roi: the tissue-mask filter (tissue_scale > 0) or the mean > 240 rule
+// (tissue_scale = 0, ROI only), then the optional ROI filter
+static int tile_scan_filtered(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask, int64_t mask_pitch,
+                              int P, int S, int iy_begin, int iy_end, int32_t* d_coords, uint8_t* d_labels, uint8_t* d_batch_u8,
+                              void* d_batch, int layout, int32_t* d_count, int capacity, void* d_workspace, size_t workspace_bytes,
+                              int mode, const uint8_t* d_tissue, int tissue_h, int tissue_w, int64_t tissue_pitch, int tissue_scale,
+                              int min_tissue_pixels, const RoiFilter* roi, cudaStream_t stream) {
+  if (roi && tissue_scale == 0)
+    return tile_scan_impl(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8, d_batch,
+                          layout, d_count, capacity, d_workspace, workspace_bytes, mode, nullptr, roi, stream);
   if (int e = tissue_geometry(P, S, tissue_scale)) return e;
   HIPAC_REQUIRE(tissue_h >= 0 && tissue_w >= 0, "negative tissue mask size");
   HIPAC_REQUIRE(d_tissue || (int64_t)tissue_h * tissue_w == 0, "null tissue mask with a nonzero size");
@@ -544,8 +551,45 @@ extern "C" int hipac_tile_scan_tissue(const uint8_t* d_rgb, int H, int W, int64_
   t.m = tissue_scale, t.min_pixels = min_tissue_pixels;
   t.cells = reinterpret_cast<uint32_t*>(d_workspace);
   return tile_scan_impl(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8, d_batch,
-                        layout, d_count, capacity, (uint8_t*)d_workspace + cells, workspace_bytes - cells, mode, &t,
-                        (cudaStream_t)stream);
+                        layout, d_count, capacity, (uint8_t*)d_workspace + cells, workspace_bytes - cells, mode, &t, roi, stream);
+}
+
+extern "C" int hipac_tile_scan_tissue(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask,
+                                      int64_t mask_pitch, int P, int S, int iy_begin, int iy_end, int32_t* d_coords,
+                                      uint8_t* d_labels, uint8_t* d_batch_u8, void* d_batch, int layout, int32_t* d_count,
+                                      int capacity, void* d_workspace, size_t workspace_bytes, int mode, const uint8_t* d_tissue,
+                                      int tissue_h, int tissue_w, int64_t tissue_pitch, int tissue_scale, int min_tissue_pixels,
+                                      void* stream) {
+  return tile_scan_filtered(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8,
+                            d_batch, layout, d_count, capacity, d_workspace, workspace_bytes, mode, d_tissue, tissue_h, tissue_w,
+                            tissue_pitch, tissue_scale, min_tissue_pixels, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" size_t hipac_tile_scan_roi_workspace_bytes(int H, int W, int P, int S, int iy_begin, int iy_end, int mode, int tissue_scale) {
+  return tissue_scale == 0 ? hipac_tile_scan_workspace_bytes(H, W, P, S, iy_begin, iy_end, mode)
+                           : hipac_tile_scan_tissue_workspace_bytes(H, W, P, S, iy_begin, iy_end, mode, tissue_scale);
+}
+
+extern "C" int hipac_tile_scan_roi(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes, const uint8_t* d_mask, int64_t mask_pitch,
+                                   int P, int S, int iy_begin, int iy_end, int32_t* d_coords, uint8_t* d_labels, uint8_t* d_batch_u8,
+                                   void* d_batch, int layout, int32_t* d_count, int capacity, void* d_workspace, size_t workspace_bytes,
+                                   int mode, const uint8_t* d_tissue, int tissue_h, int tissue_w, int64_t tissue_pitch, int tissue_scale,
+                                   int min_tissue_pixels, const uint8_t* d_roi, int roi_nx, int roi_ny, int roi_level_shift,
+                                   int roi_stride, int roi_patch, int64_t y_origin, void* stream) {
+  HIPAC_REQUIRE(!(mode & HIPAC_SCAN_KEEP_ALL), "HIPAC_SCAN_KEEP_ALL cannot be combined with an ROI");
+  HIPAC_REQUIRE(d_roi, "null ROI grid");
+  HIPAC_REQUIRE(roi_nx > 0 && roi_ny > 0 && (int64_t)roi_nx * roi_ny < ((int64_t)1 << 31), "ROI grid must have 1 to 2^31 - 1 cells");
+  HIPAC_REQUIRE(roi_level_shift >= 1 && roi_level_shift <= 16,
+                "roi_level_shift = coarse level - fine level must be in [1, 16]: the ROI must come from a coarser level");
+  HIPAC_REQUIRE(roi_stride > 0, "roi_stride must be positive");
+  HIPAC_REQUIRE(roi_patch > 0, "roi_patch must be positive");
+  HIPAC_REQUIRE(y_origin >= 0, "negative y_origin");
+  RoiFilter r{};
+  r.grid = d_roi, r.nx = roi_nx, r.ny = roi_ny, r.shift = roi_level_shift, r.stride = roi_stride, r.patch = roi_patch;
+  r.y_origin = y_origin;
+  return tile_scan_filtered(d_rgb, H, W, pitch_bytes, d_mask, mask_pitch, P, S, iy_begin, iy_end, d_coords, d_labels, d_batch_u8,
+                            d_batch, layout, d_count, capacity, d_workspace, workspace_bytes, mode, d_tissue, tissue_h, tissue_w,
+                            tissue_pitch, tissue_scale, min_tissue_pixels, &r, (cudaStream_t)stream);
 }
 
 extern "C" int hipac_upload_rows(void* d_dst, int64_t dst_pitch, const void* h_src, int64_t src_pitch, int64_t row_bytes,

@@ -697,7 +697,7 @@ static int launch_scan_planes(const ScanParams& p, const FusedGeom& G, cudaStrea
 
 static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* flags, int32_t* src_idx, int32_t* block_tot, int32_t* d_coords,
                            uint8_t* d_labels, int32_t* d_count, int capacity, uint8_t* ws, cudaStream_t stream, int keep_all,
-                           bool allow_stream, const TissueFilter* tissue) {
+                           bool allow_stream, const TissueFilter* tissue, const RoiFilter* roi) {
   FusedGeom G;
   if (!fused_geometry(p, &G)) {
     set_error("fused scan not applicable to this stride / patch size");
@@ -742,6 +742,8 @@ static int fused_scan_impl(const ScanParams& p, const OutParams& o, uint8_t* fla
   count_launch(1);
   if (tissue)
     if (int e = launch_tissue_filter(p, *tissue, flags, n_cand, stream)) return e;
+  if (roi)
+    if (int e = launch_roi_filter(p, *roi, flags, n_cand, stream)) return e;
   if (int e = launch_compact(p, flags, n_cand, d_coords, d_labels, src_idx, d_count, capacity, keep_all, block_tot, stream)) return e;
   if (int e = publish_count(d_count, stream)) return e;
   if ((o.batch_u8 || o.batch) && capacity > 0) {

@@ -42,4 +42,16 @@ void tissue_cell_grid(int S, int P, int iy_begin, int nx, int ny, int* g, int* c
 // k_tissue_cells + k_tissue_flags: rewrites bit 0 of every flag with the tissue-mask rule (after the flag kernel).
 int launch_tissue_filter(const ScanParams& p, const TissueFilter& t, uint8_t* flags, int n_cand, cudaStream_t stream);
 
+// Region of interest from a coarser level (cascade.cu): cell (i, j) of the coarse candidate grid covers the fine-level pixels
+// [i*stride << shift, (i*stride + patch) << shift) on each axis.
+struct RoiFilter {
+  const uint8_t* grid;  // [ny][nx], nonzero = set
+  int nx, ny;
+  int shift;            // coarse level - fine level, >= 1
+  int stride, patch;    // S_c, P_c of the coarse level
+  int64_t y_origin;     // fine-level row of the scanned image's row 0
+};
+// k_roi_flags: clears bit 0 of every candidate whose footprint meets no set cell (after the tissue filter, before compaction).
+int launch_roi_filter(const ScanParams& p, const RoiFilter& r, uint8_t* flags, int n_cand, cudaStream_t stream);
+
 }  // namespace hipac

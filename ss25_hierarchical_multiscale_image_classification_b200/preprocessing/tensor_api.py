@@ -154,18 +154,19 @@ def extract_patches_tensor(level_img: torch.Tensor, lesion_mask: torch.Tensor | 
                            stride=None, row_range=None, patch_size: int = 224, layout: str | None = "s2d16",
                            want_u8: bool = False, mode: str = "auto", capacity: int | None = None,
                            stream: torch.cuda.Stream | None = None, keep_all: bool = False, tissue: torch.Tensor | None = None,
-                           tissue_scale: int = 1, min_tissue=0.5) -> PatchBatch:
+                           tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0) -> PatchBatch:
     """``extract_patches_enqueue(...).resolve()``: see there."""
     return extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=row_range, patch_size=patch_size,
                                    layout=layout, want_u8=want_u8, mode=mode, capacity=capacity, stream=stream,
-                                   keep_all=keep_all, tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue).resolve()
+                                   keep_all=keep_all, tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue,
+                                   roi=roi, roi_y_origin=roi_y_origin).resolve()
 
 
 def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor | None, level: int,
                             stride=None, row_range=None, patch_size: int = 224, layout: str | None = "s2d16",
                             want_u8: bool = False, mode: str = "auto", capacity: int | None = None,
                             stream: torch.cuda.Stream | None = None, keep_all: bool = False, tissue: torch.Tensor | None = None,
-                            tissue_scale: int = 1, min_tissue=0.5) -> PendingPatchBatch:
+                            tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0) -> PendingPatchBatch:
     """Tile one level image (uint8 ``[H,W,3]`` on a CUDA device) exactly as the reference does.
 
     ``lesion_mask``: uint8 ``[H,W]`` (>0 = lesion, the rasterised ``parse_xml_mask`` output,
@@ -178,7 +179,12 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
     level) at ``tissue_scale`` m in {1, 2, 4, 8, 16, 32}: mask pixel ``(u, v)`` covers level pixels ``[u*m, u*m+m) x
     [v*m, v*m+m)`` of ``level_img``.  A candidate then survives iff at least ``ceil(min_tissue * (P/m)^2)`` mask pixels of
     its footprint are tissue (mask pixels beyond the mask count as background), instead of the reference's ``mean > 240``
-    rule; ``keep_all`` still overrides.  Nothing blocks: the call returns capacity-sized tensors and the device-side survivor
+    rule; ``keep_all`` still overrides.
+
+    ``roi``: a ``cascade.RoiGrid`` of a coarser level (the coarse-to-fine cascade).  After the ``mean > 240`` or tissue-mask
+    rule, a candidate survives only if its footprint overlaps with positive area the footprint of a set ROI cell, both taken
+    at this level's resolution.  ``roi_y_origin`` is the level row of ``level_img``'s row 0 (a shard's slab).  Cannot be
+    combined with ``keep_all``.  Nothing blocks: the call returns capacity-sized tensors and the device-side survivor
     counter; ``resolve()`` waits only until the count is known (after the compaction kernel) and slices, and
     ``features.classify_tensor(..., count=pending.count)`` consumes the batch without any host round trip.
     """
@@ -195,6 +201,16 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
         if lesion_mask.stride(1) != 1:
             lesion_mask = lesion_mask.contiguous()
     P, S = patch_and_stride(level, stride, patch_size)
+    if roi is not None:
+        if keep_all:
+            raise ValueError("keep_all cannot be combined with an ROI")
+        if roi.level <= level:
+            raise ValueError(f"the ROI of level {roi.level} must come from a level coarser than {level}")
+        if not (roi.grid.is_cuda and roi.grid.device == level_img.device and roi.grid.dtype == torch.uint8
+                and tuple(roi.grid.shape) == (roi.ny, roi.nx) and roi.grid.is_contiguous()):
+            raise ValueError("roi.grid must be a contiguous uint8 [ny, nx] tensor on the level image's device")
+        if int(roi_y_origin) < 0:
+            raise ValueError("roi_y_origin must be >= 0")
     if tissue is not None:
         if not (tissue.is_cuda and tissue.dtype == torch.uint8 and tissue.dim() == 2 and tissue.device == level_img.device):
             raise ValueError("tissue must be a uint8 [h, w] tensor on the level image's device")
@@ -227,8 +243,12 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
         batch = torch.empty(batch_shape(max(cap, 1), layout), dtype=torch.bfloat16, device=dev) if layout else None
         u8 = torch.empty((max(cap, 1), OUT, OUT, 3), dtype=torch.uint8, device=dev) if want_u8 else None
         m = _MODES[mode] | (_lib.SCAN_KEEP_ALL if keep_all else 0)
-        ws_bytes = (l.hipac_tile_scan_workspace_bytes(H, W, P, S, i0, i1, m) if tissue is None else
-                    l.hipac_tile_scan_tissue_workspace_bytes(H, W, P, S, i0, i1, m, tissue_scale))
+        if roi is not None:
+            ws_bytes = l.hipac_tile_scan_roi_workspace_bytes(H, W, P, S, i0, i1, m, tissue_scale if tissue is not None else 0)
+        elif tissue is None:
+            ws_bytes = l.hipac_tile_scan_workspace_bytes(H, W, P, S, i0, i1, m)
+        else:
+            ws_bytes = l.hipac_tile_scan_tissue_workspace_bytes(H, W, P, S, i0, i1, m, tissue_scale)
         if ws_bytes == 0:
             raise RuntimeError("hipac_tile_scan_workspace_bytes: " + l.hipac_last_error().decode())
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
@@ -240,12 +260,17 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
                 u8.data_ptr() if u8 is not None else None,
                 batch.data_ptr() if batch is not None else None, _LAYOUTS[layout] if layout else 0,
                 count.data_ptr(), cap, ws.data_ptr(), ws_bytes, m)
-        if tissue is None:
+        if tissue is not None:
+            th, tw = int(tissue.shape[0]), int(tissue.shape[1])
+            tis = (tissue.data_ptr() if th * tw else None, th, tw, int(tissue.stride(0)), tissue_scale, min_pixels)
+        if roi is not None:
+            _lib.check(l.hipac_tile_scan_roi(*args, *(tis if tissue is not None else (None, 0, 0, 0, 0, 0)), roi.grid.data_ptr(),
+                                             roi.nx, roi.ny, roi.level - level, roi.stride, roi.patch, int(roi_y_origin),
+                                             st.cuda_stream), "hipac_tile_scan_roi")
+        elif tissue is None:
             _lib.check(l.hipac_tile_scan(*args, st.cuda_stream), "hipac_tile_scan")
         else:
-            th, tw = int(tissue.shape[0]), int(tissue.shape[1])
-            _lib.check(l.hipac_tile_scan_tissue(*args, tissue.data_ptr() if th * tw else None, th, tw, int(tissue.stride(0)),
-                                                tissue_scale, min_pixels, st.cuda_stream), "hipac_tile_scan_tissue")
+            _lib.check(l.hipac_tile_scan_tissue(*args, *tis, st.cuda_stream), "hipac_tile_scan_tissue")
         ws.record_stream(st)
     del h_count   # registered with the library; read in resolve()
     _count_host.seq = getattr(_count_host, "seq", 0) + 1
