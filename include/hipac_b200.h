@@ -233,6 +233,26 @@ int hipac_resnet18_forward_dcount(const void* d_packed, int num_classes,
                                   float* d_feats, float* d_logits,
                                   void* d_workspace, size_t workspace_bytes, int chunk, void* stream);
 
+/* Rotation/flip test-time augmentation: the forward on the eight views of every patch under the dihedral group D4, with the
+ * features averaged.  View v = 4*f + k (f in {0,1}, k in {0,1,2,3}) of an NHWC image x is
+ * torch.rot90(torch.flip(x, dims=[W]) if f else x, k, dims=(H, W)).  d_feats = (((f_0 + f_1) + ...) + f_7) * 0.125 in fp32,
+ * f_v = the features hipac_resnet18_forward gives for view v; d_logits = the head applied to d_feats.  Each chunk runs the
+ * view kernel (skipped for view 0 of an S2D16 batch), the network and an accumulating pool eight times: 8x the launches of
+ * hipac_resnet18_forward (+7 for an S2D16 batch).  Validation and workspace as for hipac_resnet18_forward.  d_count: NULL =
+ * host count (n_patches patches), else device-count mode as in hipac_resnet18_forward_dcount (n_patches = capacity; rows
+ * >= d_count[0] of d_feats / d_logits are left untouched). */
+int hipac_resnet18_forward_d4(const void* d_packed, int num_classes,
+                              const void* d_batch, int layout, int n_patches, const int32_t* d_count,
+                              float* d_feats, float* d_logits,
+                              void* d_workspace, size_t workspace_bytes, int chunk, void* stream);
+
+/* Test hook: D4 view `view` (0..7, see hipac_resnet18_forward_d4) of a bf16 batch in `layout` -> S2D16 d_out
+ * [n_patches][112][115][16] (padding columns and channels 12..15 written as zero).  View 0 of an NHWC3 batch is the repack
+ * hipac_resnet18_forward runs.  d_count / n_base as for the hooks below: only patches < clamp(d_count[0] - n_base, 0,
+ * n_patches) are written.  d_out must not overlap d_in. */
+int hipac_batch_d4_view(const void* d_in, int layout, int n_patches, int view, void* d_out, const int32_t* d_count, int n_base,
+                        void* stream);
+
 /* The three test hooks below run one stage-2 kernel with the launch state the forward gives it:
  *   reverse  nonzero: walk the tiles from the last to the first (the forward alternates the order from launch to launch);
  *   d_count  NULL: work on all n_patches patches; else device-count mode as in hipac_resnet18_forward_dcount, the kernel

@@ -157,6 +157,10 @@ def _declare(l):
     l.hipac_resnet18_forward.argtypes = [vp, i32, vp, i32, i32, vp, vp, vp, sz, i32, vp]
     l.hipac_resnet18_forward_dcount.restype = i32
     l.hipac_resnet18_forward_dcount.argtypes = [vp, i32, vp, i32, i32, vp, vp, vp, vp, sz, i32, vp]
+    l.hipac_resnet18_forward_d4.restype = i32
+    l.hipac_resnet18_forward_d4.argtypes = [vp, i32, vp, i32, i32, vp, vp, vp, vp, sz, i32, vp]
+    l.hipac_batch_d4_view.restype = i32
+    l.hipac_batch_d4_view.argtypes = [vp, i32, i32, i32, vp, vp, i32, vp]
     l.hipac_resnet18_conv_ds_fused.restype = i32
     l.hipac_resnet18_conv_ds_fused.argtypes = [vp, i32, i32, vp, vp, vp, i32, vp, i32, vp, i32]
     l.hipac_resnet18_stem.restype = i32
@@ -204,6 +208,7 @@ EXPORTS = [
     "hipac_profile_enable", "hipac_profile_report", "hipac_debug_umma_shift", "hipac_resnet18_stem", "hipac_resnet18_conv_ds_fused",
     "hipac_tile_scan_tissue_workspace_bytes", "hipac_tile_scan_tissue", "hipac_tissue_workspace_bytes", "hipac_tissue_segment",
     "hipac_roi_grid_bytes", "hipac_roi_grid", "hipac_tile_scan_roi_workspace_bytes", "hipac_tile_scan_roi",
+    "hipac_resnet18_forward_d4", "hipac_batch_d4_view",
 ]
 
 

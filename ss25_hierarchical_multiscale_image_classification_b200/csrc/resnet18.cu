@@ -161,22 +161,105 @@ __global__ void __launch_bounds__(256) k_avgpool_fc(const __nv_bfloat16* __restr
   }
 }
 
-// bf16 NHWC3 [n,224,224,3] -> S2D16 [n,112,115,16] (used when the caller hands the plain layout).
-__global__ void __launch_bounds__(256) k_pack_s2d16(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, int n_img) {
-  const int64_t total = (int64_t)n_img * 112 * kS2dW;
+// k_avgpool_fc of one view of the D4 test-time augmentation (forward_impl with 8 views).  The pooled features of the view
+// are computed as in k_avgpool_fc; view 0 stores them into feats, views 1..7 add them to feats (an fp32 running sum in
+// view order), and after view 7 the sum is multiplied by 1/8 and k_avgpool_fc's head is applied to it.  The _rn
+// intrinsics keep s * (1/49) + acc from being contracted into one FMA, which would round once where the definition
+// rounds twice.
+__global__ void __launch_bounds__(256) k_avgpool_fc_d4(const __nv_bfloat16* __restrict__ in, float* __restrict__ feats,
+                                                       float* __restrict__ logits, const float* __restrict__ fc_w,
+                                                       const float* __restrict__ fc_b, int num_classes,
+                                                       const int* __restrict__ n_dev, int n_base, int view) {
+  const int img = blockIdx.x;
+  ptx::pdl_launch_dependents();
+  ptx::pdl_wait();   // also orders the read of feats after the previous view's pool
+  if (n_dev && img >= __ldg(n_dev) - n_base) return;
+  __shared__ float f[512];
+  const __nv_bfloat16* src = in + (int64_t)img * 49 * 512;
+  float* dst = feats + (int64_t)img * 512;
+  for (int c2 = threadIdx.x; c2 < 256; c2 += 256) {
+    float s0 = 0.f, s1 = 0.f;
+    for (int px = 0; px < 49; px++) {
+      const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(src + px * 512 + 2 * c2);
+      s0 += __bfloat162float(v.x), s1 += __bfloat162float(v.y);
+    }
+    s0 = __fmul_rn(s0, 1.0f / 49.0f), s1 = __fmul_rn(s1, 1.0f / 49.0f);
+    if (view > 0) s0 = __fadd_rn(dst[2 * c2], s0), s1 = __fadd_rn(dst[2 * c2 + 1], s1);
+    if (view == 7) s0 = __fmul_rn(s0, 0.125f), s1 = __fmul_rn(s1, 0.125f);
+    f[2 * c2] = s0, f[2 * c2 + 1] = s1;
+    dst[2 * c2] = s0;
+    dst[2 * c2 + 1] = s1;
+  }
+  if (view != 7 || !logits) return;
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int k = warp; k < num_classes; k += 8) {
+    float s = 0.f;
+    for (int c = lane; c < 512; c += 32) s += f[c] * __ldg(fc_w + k * 512 + c);
+    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) logits[(int64_t)img * num_classes + k] = s + __ldg(fc_b + k);
+  }
+}
+
+// Pixel (i, j) of D4 view v = 4 f + k of a 224 x 224 image x is pixel (a, b) of x, where the view is
+// torch.rot90(flip(x, W) if f else x, k, dims=(H, W)).
+__device__ __forceinline__ void d4_source(int view, int i, int j, int& a, int& b) {
+  const int k = view & 3;
+  a = k == 0 ? i : k == 1 ? j : k == 2 ? 223 - i : 223 - j;
+  b = k == 0 ? j : k == 1 ? 223 - i : k == 2 ? 223 - j : i;
+  if (view & 4) b = 223 - b;
+}
+
+// D4 view `view` of a bf16 batch in `layout` (NHWC3 [n,224,224,3] or S2D16 [n,112,115,16]) -> S2D16 [n,112,115,16], the
+// stem's operand.  224 is even, so every view maps 2x2 blocks onto 2x2 blocks: output pixel (Y, X) is one input block with
+// its four sub-pixels permuted, i.e. one 32-byte S2D16 load (or two 12-byte NHWC3 row runs) and one 32-byte store.  The
+// padding columns and channels 12..15 are written as zero whatever the input holds there.  View 0 of NHWC3 is the plain
+// repack of the forward.  Device-count mode: only patches < clamp(*n_dev - n_base, 0, n_img) are written.
+__global__ void __launch_bounds__(256) k_d4_view(const uint16_t* __restrict__ in, int layout, uint16_t* __restrict__ out, int n_img,
+                                                 int view, const int* __restrict__ n_dev, int n_base) {
+  const int64_t total = (int64_t)effective_patches(n_dev, n_base, n_img) * 112 * kS2dW;
+  // sub-pixel q = dy * 2 + dx of an output block comes from sub-pixel perm[q] of its input block (independent of the block)
+  int perm[4];
+#pragma unroll
+  for (int q = 0; q < 4; q++) {
+    int a, b;
+    d4_source(view, q >> 1, q & 1, a, b);
+    perm[q] = (a & 1) * 2 + (b & 1);
+  }
   for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
     const int X = (int)(t % kS2dW) - 2;
     const int Y = (int)((t / kS2dW) % 112);
     const int64_t img = t / (112 * kS2dW);
-    uint16_t v[16];
+    alignas(16) uint16_t v[16] = {};
+    if (X >= 0 && X < 112) {
+      int a, b;
+      d4_source(view, 2 * Y, 2 * X, a, b);
+      const int BY = a >> 1, BX = b >> 1;
+      alignas(16) uint16_t s[16];   // the input block, channel (sy * 2 + sx) * 3 + c
+      if (layout == HIPAC_LAYOUT_S2D16_BF16) {
+        const uint4* p = reinterpret_cast<const uint4*>(in + ((img * 112 + BY) * kS2dW + BX + 2) * 16);
+        *reinterpret_cast<uint4*>(&s[0]) = __ldg(p);
+        *reinterpret_cast<uint4*>(&s[8]) = __ldg(p + 1);
+      } else {
 #pragma unroll
-    for (int dy = 0; dy < 2; dy++)
+        for (int sy = 0; sy < 2; sy++) {
+          // pixels 2BX, 2BX + 1 of row 2BY + sy: 12 bytes at a multiple of 12 bytes (4-byte aligned)
+          const uint32_t* p = reinterpret_cast<const uint32_t*>(in + ((img * 224 + 2 * BY + sy) * 224 + 2 * BX) * 3);
 #pragma unroll
-      for (int dx = 0; dx < 2; dx++)
+          for (int w = 0; w < 3; w++) {
+            const uint32_t u = __ldg(p + w);
+            s[sy * 6 + 2 * w] = (uint16_t)(u & 0xFFFFu), s[sy * 6 + 2 * w + 1] = (uint16_t)(u >> 16);
+          }
+        }
+      }
 #pragma unroll
-        for (int c = 0; c < 3; c++)
-          v[(dy * 2 + dx) * 3 + c] = (X >= 0 && X < 112) ? in[((img * 224 + 2 * Y + dy) * 224 + 2 * X + dx) * 3 + c] : (uint16_t)0;
-    v[12] = v[13] = v[14] = v[15] = 0;
+      for (int q = 0; q < 4; q++)
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+          const int pq = perm[q];   // selects, not a dynamically indexed (local-memory) array
+          v[q * 3 + c] = pq == 0 ? s[c] : pq == 1 ? s[3 + c] : pq == 2 ? s[6 + c] : s[9 + c];
+        }
+    }
     uint4* dst = reinterpret_cast<uint4*>(out + t * 16);
     dst[0] = *reinterpret_cast<uint4*>(&v[0]);
     dst[1] = *reinterpret_cast<uint4*>(&v[8]);
@@ -525,8 +608,8 @@ extern "C" int hipac_resnet18_pack(const float* const* t, int num_tensors, int n
 extern "C" size_t hipac_resnet18_workspace_bytes(int n_patches, int chunk) {
   if (n_patches <= 0) return 256;
   const size_t c = (size_t)clamp_chunk(chunk, n_patches);
-  // three activation buffers; the S2D16 repack buffer is needed only when the caller hands the plain NHWC3 layout (sized
-  // for it unconditionally: 0.4 MB / patch)
+  // three activation buffers; the S2D16 scratch buffer is needed only when the caller hands the plain NHWC3 layout or asks
+  // for the D4 views (sized for it unconditionally: 0.4 MB / patch)
   return c * (3 * kActBytes + kS2dBytes) + 6 * 1024;
 }
 
@@ -572,9 +655,11 @@ extern "C" int hipac_resnet18_stem(const void* d_packed, int num_classes, const 
                   d_out, n_patches);
 }
 
+// views = 1: the plain forward.  views = 8: the D4 test-time augmentation, every chunk runs the network on each of its
+// eight views in turn (view kernel into the S2D16 scratch buffer, stem, convs, accumulating pool).
 static int forward_impl(const void* d_packed, int num_classes, const void* d_batch, int layout, int n_patches,
                         float* d_feats, float* d_logits, void* d_workspace, size_t workspace_bytes, int chunk,
-                        void* stream_, const int* d_count) {
+                        void* stream_, const int* d_count, int views) {
   HIPAC_REQUIRE(n_patches >= 0, "negative n_patches");
   if (n_patches == 0) return 0;
   HIPAC_REQUIRE(d_packed && d_batch && d_feats && d_workspace, "null pointer");
@@ -599,50 +684,63 @@ static int forward_impl(const void* d_packed, int num_classes, const void* d_bat
   uint8_t* C = carve(cmax * kActBytes);
   uint8_t* s2d = carve(cmax * kS2dBytes);
 
+  const bool s2d_in = layout == HIPAC_LAYOUT_S2D16_BF16;
+  const size_t in_bytes = s2d_in ? kS2dBytes : (size_t)224 * 224 * 3 * 2;   // per patch
   for (int i0 = 0; i0 < n_patches; i0 += cmax) {
     const int n = n_patches - i0 < cmax ? n_patches - i0 : cmax;
     ctx.n_base = i0;
-    const void* x0;
-    if (layout == HIPAC_LAYOUT_S2D16_BF16) {
-      x0 = reinterpret_cast<const uint8_t*>(d_batch) + (size_t)i0 * kS2dBytes;
-    } else {
-      const uint16_t* src = reinterpret_cast<const uint16_t*>(d_batch) + (size_t)i0 * 224 * 224 * 3;
-      {
-        ProfileScope ps("pack_s2d16", ctx.stream, (double)n * (224 * 224 * 3 * 2 + kS2dBytes));
-        k_pack_s2d16<<<ctx.sms * 8, 256, 0, ctx.stream>>>(src, reinterpret_cast<uint16_t*>(s2d), n);
+    const uint8_t* chunk_in = reinterpret_cast<const uint8_t*>(d_batch) + (size_t)i0 * in_bytes;
+    for (int view = 0; view < views; view++) {
+      const void* x0 = chunk_in;   // view 0 of an S2D16 batch is the batch itself
+      if (!s2d_in || view > 0) {
+        // a plain launch: it starts after the previous view's kernels, whose stem may have read the scratch buffer
+        {
+          ProfileScope ps("d4_view", ctx.stream, (double)n * (in_bytes + kS2dBytes));
+          k_d4_view<<<ctx.sms * 8, 256, 0, ctx.stream>>>(reinterpret_cast<const uint16_t*>(chunk_in), layout,
+                                                         reinterpret_cast<uint16_t*>(s2d), n, view, ctx.n_dev, ctx.n_base);
+        }
+        count_launch(1);
+        x0 = s2d;
+      }
+      // the batch was written in ascending patch order, so the first launch of the chain walks it descending, the next
+      // ascending, ...
+      int pos = 0;   // position of the next launch in the chain
+      auto next = [&] {
+        Launch c = ctx;
+        c.reverse = pos++ % 2 == 0;
+        return c;
+      };
+      auto conv = [&](int layer, const void* in, const void* res, void* out, bool relu) {
+        return run_conv(next(), pk, L, layer, in, res, out, n, relu);
+      };
+      int e = 0;
+      if ((e = run_stem(next(), pk, L, x0, A, n))) return e;
+      // layer1 (two basic blocks, identity shortcuts)
+      if ((e = conv(1, A, nullptr, B, true)) || (e = conv(2, B, A, C, true))) return e;
+      if ((e = conv(3, C, nullptr, B, true)) || (e = conv(4, B, C, A, true))) return e;
+      // layer2..4: first block has a strided 1x1 projection shortcut
+      for (int s = 0; s < 3; s++) {
+        const int l0 = 5 + 5 * s;
+        if ((e = conv(l0, A, nullptr, B, true))) return e;           // 3x3 / stride 2
+        if ((e = run_conv_ds_fused(next(), pk, L, s, B, A, C, n))) return e;   // 3x3 + 1x1/s2 projection + ReLU, one accumulator
+        if ((e = conv(l0 + 3, C, nullptr, B, true)) || (e = conv(l0 + 4, B, C, A, true))) return e;
+      }
+      const auto* pool_in = reinterpret_cast<const __nv_bfloat16*>(A);
+      float* feats = d_feats + (size_t)i0 * 512;
+      float* logits = d_logits ? d_logits + (size_t)i0 * num_classes : nullptr;
+      const float* fc_w = reinterpret_cast<const float*>(pk + L.fc_w_off);
+      const float* fc_b = reinterpret_cast<const float*>(pk + L.fc_b_off);
+      if (views == 1) {
+        ProfileScope ps_pool("avgpool_fc", ctx.stream, (double)n * (49 * 512 * 2 + 512 * 4));
+        HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc, dim3(n), dim3(256), 0, ctx.stream, 1, pool_in, feats, logits, fc_w, fc_b,
+                                   num_classes, ctx.n_dev, ctx.n_base));
+      } else {
+        ProfileScope ps_pool("avgpool_fc_d4", ctx.stream, (double)n * (49 * 512 * 2 + 2 * 512 * 4));
+        HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc_d4, dim3(n), dim3(256), 0, ctx.stream, 1, pool_in, feats, logits, fc_w, fc_b,
+                                   num_classes, ctx.n_dev, ctx.n_base, view));
       }
       count_launch(1);
-      x0 = s2d;
     }
-    // the batch was written in ascending patch order, so the first launch of the chunk walks it descending, the next
-    // ascending, ...
-    int pos = 0;   // position of the next launch in the chunk
-    auto next = [&] {
-      Launch c = ctx;
-      c.reverse = pos++ % 2 == 0;
-      return c;
-    };
-    auto conv = [&](int layer, const void* in, const void* res, void* out, bool relu) {
-      return run_conv(next(), pk, L, layer, in, res, out, n, relu);
-    };
-    int e = 0;
-    if ((e = run_stem(next(), pk, L, x0, A, n))) return e;
-    // layer1 (two basic blocks, identity shortcuts)
-    if ((e = conv(1, A, nullptr, B, true)) || (e = conv(2, B, A, C, true))) return e;
-    if ((e = conv(3, C, nullptr, B, true)) || (e = conv(4, B, C, A, true))) return e;
-    // layer2..4: first block has a strided 1x1 projection shortcut
-    for (int s = 0; s < 3; s++) {
-      const int l0 = 5 + 5 * s;
-      if ((e = conv(l0, A, nullptr, B, true))) return e;           // 3x3 / stride 2
-      if ((e = run_conv_ds_fused(next(), pk, L, s, B, A, C, n))) return e;   // 3x3 + 1x1/s2 projection + ReLU, one accumulator
-      if ((e = conv(l0 + 3, C, nullptr, B, true)) || (e = conv(l0 + 4, B, C, A, true))) return e;
-    }
-    ProfileScope ps_pool("avgpool_fc", ctx.stream, (double)n * (49 * 512 * 2 + 512 * 4));
-    HIPAC_CHECK_CUDA(launch_ex(k_avgpool_fc, dim3(n), dim3(256), 0, ctx.stream, 1, reinterpret_cast<const __nv_bfloat16*>(A),
-                               d_feats + (size_t)i0 * 512, d_logits ? d_logits + (size_t)i0 * num_classes : nullptr,
-                               reinterpret_cast<const float*>(pk + L.fc_w_off), reinterpret_cast<const float*>(pk + L.fc_b_off),
-                               num_classes, ctx.n_dev, ctx.n_base));
-    count_launch(1);
   }
   HIPAC_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -652,7 +750,7 @@ extern "C" int hipac_resnet18_forward(const void* d_packed, int num_classes, con
                                       float* d_feats, float* d_logits, void* d_workspace, size_t workspace_bytes, int chunk,
                                       void* stream) {
   return forward_impl(d_packed, num_classes, d_batch, layout, n_patches, d_feats, d_logits, d_workspace, workspace_bytes, chunk,
-                      stream, nullptr);
+                      stream, nullptr, 1);
 }
 
 extern "C" int hipac_resnet18_forward_dcount(const void* d_packed, int num_classes, const void* d_batch, int layout, int capacity,
@@ -660,5 +758,36 @@ extern "C" int hipac_resnet18_forward_dcount(const void* d_packed, int num_class
                                              size_t workspace_bytes, int chunk, void* stream) {
   HIPAC_REQUIRE(d_count != nullptr, "null device count");
   return forward_impl(d_packed, num_classes, d_batch, layout, capacity, d_feats, d_logits, d_workspace, workspace_bytes, chunk,
-                      stream, d_count);
+                      stream, d_count, 1);
+}
+
+extern "C" int hipac_resnet18_forward_d4(const void* d_packed, int num_classes, const void* d_batch, int layout, int n_patches,
+                                         const int32_t* d_count, float* d_feats, float* d_logits, void* d_workspace,
+                                         size_t workspace_bytes, int chunk, void* stream) {
+  return forward_impl(d_packed, num_classes, d_batch, layout, n_patches, d_feats, d_logits, d_workspace, workspace_bytes, chunk,
+                      stream, d_count, 8);
+}
+
+extern "C" int hipac_batch_d4_view(const void* d_in, int layout, int n_patches, int view, void* d_out, const int32_t* d_count,
+                                   int n_base, void* stream) {
+  HIPAC_REQUIRE(d_in && d_out, "null pointer");
+  HIPAC_REQUIRE(layout == HIPAC_LAYOUT_S2D16_BF16 || layout == HIPAC_LAYOUT_NHWC3_BF16, "unknown batch layout");
+  HIPAC_REQUIRE(view >= 0 && view < 8, "view must be in 0..7");
+  HIPAC_REQUIRE(n_patches >= 0, "negative n_patches");
+  HIPAC_REQUIRE(n_base >= 0, "n_base must be non-negative");
+  const uintptr_t in = (uintptr_t)d_in, out = (uintptr_t)d_out;
+  const size_t in_bytes = (size_t)n_patches * (layout == HIPAC_LAYOUT_S2D16_BF16 ? kS2dBytes : (size_t)224 * 224 * 3 * 2);
+  const size_t out_bytes = (size_t)n_patches * kS2dBytes;
+  HIPAC_REQUIRE(n_patches == 0 || in + in_bytes <= out || out + out_bytes <= in, "d_out overlaps d_in");
+  if (n_patches == 0) return 0;
+  int sms = 0;
+  if (int e = device_sm_count(&sms)) return e;
+  {
+    ProfileScope ps("d4_view", (cudaStream_t)stream, (double)(in_bytes + out_bytes));
+    k_d4_view<<<sms * 8, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const uint16_t*>(d_in), layout,
+                                                          reinterpret_cast<uint16_t*>(d_out), n_patches, view, d_count, n_base);
+  }
+  count_launch(1);
+  HIPAC_CHECK_CUDA(cudaGetLastError());
+  return 0;
 }

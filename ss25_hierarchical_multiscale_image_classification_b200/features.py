@@ -69,9 +69,10 @@ _LAYOUT_BY_SHAPE = {(224, 224, 3): _lib.LAYOUT_NHWC3_BF16, (112, 115, 16): _lib.
 
 
 def _forward(batch: torch.Tensor, packed: PackedResNet18, want_logits: bool, chunk: int, stream=None,
-             count: torch.Tensor | None = None):
+             count: torch.Tensor | None = None, tta: bool = False):
     """``count``: int32 device tensor whose element 0 is the number of valid patches in ``batch`` (device-count mode:
-    ``batch.shape[0]`` is only the capacity; nothing here waits for the value)."""
+    ``batch.shape[0]`` is only the capacity; nothing here waits for the value).  ``tta``: the D4 test-time augmentation
+    (``hipac_resnet18_forward_d4``)."""
     l = _lib.lib()
     if not (batch.is_cuda and batch.dtype == torch.bfloat16 and batch.dim() == 4 and tuple(batch.shape[1:]) in _LAYOUT_BY_SHAPE):
         raise ValueError("batch must be a CUDA bf16 tensor [N,224,224,3] or [N,112,115,16]")
@@ -90,14 +91,20 @@ def _forward(batch: torch.Tensor, packed: PackedResNet18, want_logits: bool, chu
             return feats, logits
         ws_bytes = l.hipac_resnet18_workspace_bytes(n, chunk)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-        if count is None:
+        if count is not None and not (count.is_cuda and count.dtype == torch.int32 and count.numel() >= 1):
+            raise ValueError("count must be a CUDA int32 tensor")
+        if tta:
+            rc = l.hipac_resnet18_forward_d4(packed.blob.data_ptr(), packed.num_classes, batch.data_ptr(),
+                                             _LAYOUT_BY_SHAPE[tuple(batch.shape[1:])], n,
+                                             count.data_ptr() if count is not None else None, feats.data_ptr(),
+                                             logits.data_ptr() if logits is not None else None, ws.data_ptr(), ws_bytes,
+                                             chunk, st.cuda_stream)
+        elif count is None:
             rc = l.hipac_resnet18_forward(packed.blob.data_ptr(), packed.num_classes, batch.data_ptr(),
                                           _LAYOUT_BY_SHAPE[tuple(batch.shape[1:])], n, feats.data_ptr(),
                                           logits.data_ptr() if logits is not None else None, ws.data_ptr(), ws_bytes,
                                           chunk, st.cuda_stream)
         else:
-            if not (count.is_cuda and count.dtype == torch.int32 and count.numel() >= 1):
-                raise ValueError("count must be a CUDA int32 tensor")
             rc = l.hipac_resnet18_forward_dcount(packed.blob.data_ptr(), packed.num_classes, batch.data_ptr(),
                                                  _LAYOUT_BY_SHAPE[tuple(batch.shape[1:])], n, count.data_ptr(),
                                                  feats.data_ptr(), logits.data_ptr() if logits is not None else None,
@@ -108,15 +115,41 @@ def _forward(batch: torch.Tensor, packed: PackedResNet18, want_logits: bool, chu
 
 
 def extract_features_tensor(batch: torch.Tensor, packed: PackedResNet18, chunk: int = 4096, stream=None,
-                            count: torch.Tensor | None = None) -> torch.Tensor:
-    """float32 ``[N,512]`` pooled trunk features of a bf16 patch batch (asynchronous)."""
-    return _forward(batch, packed, False, chunk, stream, count)[0]
+                            count: torch.Tensor | None = None, *, tta: bool = False) -> torch.Tensor:
+    """float32 ``[N,512]`` pooled trunk features of a bf16 patch batch (asynchronous).
+
+    ``tta=True``: rotation/flip test-time augmentation.  Each patch's features are the mean of the features of its eight
+    views under the dihedral group D4 (``d4_view``), summed in fp32 in view order 0..7 and multiplied by 0.125, so they do
+    not depend on the patch's orientation.  Costs eight forwards."""
+    return _forward(batch, packed, False, chunk, stream, count, tta)[0]
 
 
 def classify_tensor(batch: torch.Tensor, packed: PackedResNet18, chunk: int = 4096, stream=None,
-                    count: torch.Tensor | None = None):
-    """(features float32 ``[N,512]``, logits float32 ``[N,k]``) of a bf16 patch batch (asynchronous)."""
-    return _forward(batch, packed, True, chunk, stream, count)
+                    count: torch.Tensor | None = None, *, tta: bool = False):
+    """(features float32 ``[N,512]``, logits float32 ``[N,k]``) of a bf16 patch batch (asynchronous).  ``tta=True``: the
+    features of ``extract_features_tensor(..., tta=True)`` and the head applied to them (which, the head being affine,
+    is the mean of the eight views' logits up to rounding)."""
+    return _forward(batch, packed, True, chunk, stream, count, tta)
+
+
+def d4_view(batch: torch.Tensor, view: int, *, count: torch.Tensor | None = None, base: int = 0,
+            out: torch.Tensor | None = None) -> torch.Tensor:
+    """View ``view`` = 4 f + k (0..7) of a bf16 patch batch (``[N,224,224,3]`` or ``[N,112,115,16]``) under the dihedral
+    group D4, as the S2D16 batch ``[N,112,115,16]`` the network reads: the S2D16 form of
+    ``torch.rot90(torch.flip(x, dims=[2]) if f else x, k, dims=(1, 2))`` for the NHWC image ``x``.  The padding columns and
+    channels 12..15 of the output are zero.  ``count`` / ``base`` / ``out``: device-count mode and in-place output as for
+    ``conv_layer``."""
+    if not (batch.is_cuda and batch.dtype == torch.bfloat16 and batch.dim() == 4 and tuple(batch.shape[1:]) in _LAYOUT_BY_SHAPE):
+        raise ValueError("batch must be a CUDA bf16 tensor [N,224,224,3] or [N,112,115,16]")
+    l = _lib.lib()
+    batch = batch.contiguous()
+    n = int(batch.shape[0])
+    out = _hook_out(out, (n, 112, 115, 16), batch.device)
+    d_count, n_base = _launch_state(count, base)
+    rc = l.hipac_batch_d4_view(batch.data_ptr(), _LAYOUT_BY_SHAPE[tuple(batch.shape[1:])], n, int(view), out.data_ptr(),
+                               d_count, n_base, torch.cuda.current_stream(batch.device).cuda_stream)
+    _lib.check(rc, "hipac_batch_d4_view")
+    return out
 
 
 def _launch_state(count: torch.Tensor | None, base: int):

@@ -41,7 +41,7 @@ class _HipacForwardMixin:
             self._pack_key = key
         return self._pack
 
-    def _run(self, x: torch.Tensor, chunk: int = 4096):
+    def _run(self, x: torch.Tensor, chunk: int = 4096, tta: bool = False):
         if self.training:
             raise RuntimeError("the B200 path is inference-only: call .eval() first (training is out of scope)")
         if not x.is_cuda:
@@ -51,12 +51,13 @@ class _HipacForwardMixin:
             x = x.permute(0, 2, 3, 1).contiguous().to(torch.bfloat16)
         packed = self._packed(x.device)
         if packed.num_classes > 0 and self._wants_logits:
-            return _features.classify_tensor(x, packed, chunk)[1]
-        return _features.extract_features_tensor(x, packed, chunk)
+            return _features.classify_tensor(x, packed, chunk, tta=tta)[1]
+        return _features.extract_features_tensor(x, packed, chunk, tta=tta)
 
-    def forward_batch(self, batch: torch.Tensor, chunk: int = 4096):
-        """Native entry: bf16 ``[N,224,224,3]`` or ``[N,112,115,16]`` batch from ``extract_patches_tensor``."""
-        return self._run(batch, chunk)
+    def forward_batch(self, batch: torch.Tensor, chunk: int = 4096, tta: bool = False):
+        """Native entry: bf16 ``[N,224,224,3]`` or ``[N,112,115,16]`` batch from ``extract_patches_tensor``.  ``tta=True``:
+        the mean over the eight D4 rotations / flips of each patch (``features.extract_features_tensor(..., tta=True)``)."""
+        return self._run(batch, chunk, tta)
 
 
 def _sequential_to_tv(sd: dict, prefix: str = "features.") -> dict:

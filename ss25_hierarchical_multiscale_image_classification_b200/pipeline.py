@@ -54,22 +54,22 @@ class PendingLevel:
 
 def process_level_enqueue(level_img, lesion_mask, level, packed, stride=None, row_range=None, chunk: int = 8192,
                           mode: str = "auto", tissue=None, tissue_scale: int = 1, min_tissue=0.5, roi=None,
-                          roi_y_origin: int = 0) -> PendingLevel:
+                          roi_y_origin: int = 0, tta: bool = False) -> PendingLevel:
     """Enqueue tile scan + ResNet18 of candidate grid rows ``row_range`` without any host wait (the network kernels read
     the survivor count from device memory).  Feed the result to ``sharding.SurvivorExchange.pack``.  ``tissue`` /
     ``tissue_scale`` / ``min_tissue``: the tissue-mask filter, ``roi`` / ``roi_y_origin``: the coarse-level ROI of
-    ``extract_patches_enqueue``."""
+    ``extract_patches_enqueue``.  ``tta``: the D4 test-time augmentation of ``features.classify_tensor``."""
     pend = extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=row_range, layout="s2d16", mode=mode,
                                    tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin)
     if packed.num_classes > 0:
-        feats, logits = _features.classify_tensor(pend.batch, packed, chunk, count=pend.count)
+        feats, logits = _features.classify_tensor(pend.batch, packed, chunk, count=pend.count, tta=tta)
     else:
-        feats, logits = _features.extract_features_tensor(pend.batch, packed, chunk, count=pend.count), None
+        feats, logits = _features.extract_features_tensor(pend.batch, packed, chunk, count=pend.count, tta=tta), None
     return PendingLevel(pend, feats, logits)
 
 
 def _process_rows(level_img, lesion_mask, level, packed, stride, rows, chunk, mode, tissue=None, tissue_scale=1, min_tissue=0.5,
-                  roi=None, roi_y_origin=0):
+                  roi=None, roi_y_origin=0, tta=False):
     """Tile scan + ResNet18 of one candidate-row group, enqueued back to back: the network kernels take the survivor
     count from device memory (``hipac_resnet18_forward_dcount``), so the host only learns it afterwards, to slice the
     capacity-sized outputs -- while the GPU is already running the network."""
@@ -78,16 +78,16 @@ def _process_rows(level_img, lesion_mask, level, packed, stride, rows, chunk, mo
         pb = extract_patches_tensor(level_img, lesion_mask, level, stride=stride, row_range=rows, layout="s2d16", mode=mode,
                                     tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin)
         if packed.num_classes > 0:
-            feats, logits = _features.classify_tensor(pb.batch, packed, chunk)
+            feats, logits = _features.classify_tensor(pb.batch, packed, chunk, tta=tta)
         else:
-            feats, logits = _features.extract_features_tensor(pb.batch, packed, chunk), None
+            feats, logits = _features.extract_features_tensor(pb.batch, packed, chunk, tta=tta), None
         return LevelResult(pb.coords, pb.labels, feats, logits, pb.candidates)
     pend = extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=rows, layout="s2d16", mode=mode,
                                    tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin)
     if packed.num_classes > 0:
-        feats, logits = _features.classify_tensor(pend.batch, packed, chunk, count=pend.count)
+        feats, logits = _features.classify_tensor(pend.batch, packed, chunk, count=pend.count, tta=tta)
     else:
-        feats, logits = _features.extract_features_tensor(pend.batch, packed, chunk, count=pend.count), None
+        feats, logits = _features.extract_features_tensor(pend.batch, packed, chunk, count=pend.count, tta=tta), None
     pb = pend.resolve()
     n = len(pb)
     return LevelResult(pb.coords, pb.labels, feats[:n], logits[:n] if logits is not None else None, pb.candidates)
@@ -95,7 +95,7 @@ def _process_rows(level_img, lesion_mask, level, packed, stride, rows, chunk, mo
 
 def process_level(level_img: torch.Tensor, lesion_mask, level: int, packed: _features.PackedResNet18, stride=None,
                   row_range=None, chunk: int = 8192, mode: str = "auto", max_candidates: int = 16384, tissue=None,
-                  tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0) -> LevelResult:
+                  tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0, tta: bool = False) -> LevelResult:
     """Tile + tissue/lesion mask + ResNet18 features of a level image resident on the GPU.
 
     ``tissue`` / ``tissue_scale`` / ``min_tissue``: keep the candidates a tissue mask covers (e.g. ``segment_tissue`` of a
@@ -103,6 +103,9 @@ def process_level(level_img: torch.Tensor, lesion_mask, level: int, packed: _fea
 
     ``roi`` / ``roi_y_origin``: keep only the candidates inside a coarser level's ``cascade.RoiGrid`` (see
     ``extract_patches_enqueue`` and ``cascade.process_cascade``).
+
+    ``tta``: rotation/flip test-time augmentation in stage 2 (``features.classify_tensor(..., tta=True)``): features and
+    logits of every survivor are those of its eight D4 views averaged; coordinates, labels and candidates do not change.
 
     The batch buffer is sized for the worst case (every candidate survives), so levels with more than
     ``max_candidates`` candidates are processed in groups of whole candidate-grid rows (a 100k x 100k level at
@@ -113,7 +116,7 @@ def process_level(level_img: torch.Tensor, lesion_mask, level: int, packed: _fea
     nx, ny_all = grid_shape(W, H, S)
     i0, i1 = (0, ny_all) if row_range is None else (int(row_range[0]), int(row_range[1]))
     rows_per_group = max(1, max_candidates // max(nx, 1))
-    tis = dict(tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue)
+    tis = dict(tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, tta=tta)
     if roi is not None:
         tis.update(roi=roi, roi_y_origin=roi_y_origin)
     if i1 - i0 <= rows_per_group:
@@ -143,7 +146,7 @@ def exchange_for_level(device, width: int, rows_per_rank: int, stride: int, num_
 
 def process_level_exchanged(level_img, lesion_mask, level: int, packed: _features.PackedResNet18, exchange, stride=None,
                             row_range=None, y_offset: int = 0, chunk: int = 8192, mode: str = "auto", tissue=None,
-                            tissue_scale: int = 1, min_tissue=0.5, roi=None) -> int:
+                            tissue_scale: int = 1, min_tissue=0.5, roi=None, tta: bool = False) -> int:
     """``process_level`` whose result goes straight into the exchange step: the rank's grid rows are cut into the exchange's
     row groups, each group is enqueued (tile scan + ResNet18, survivor count on the device) and packed as one segment, then
     ``exchange.merge()`` is enqueued.  No host wait anywhere; call ``exchange.result()`` for the merged, canonically
@@ -155,7 +158,7 @@ def process_level_exchanged(level_img, lesion_mask, level: int, packed: _feature
     same mask and an N-rank result equals a single-rank one.
 
     ``roi``: a ``cascade.RoiGrid`` of a coarser level over the WHOLE slide (every rank builds the same one from the
-    exchanged coarse result); the rank's slab is placed in it by ``y_offset``."""
+    exchanged coarse result); the rank's slab is placed in it by ``y_offset``.  ``tta``: as in ``process_level``."""
     H, W = int(level_img.shape[0]), int(level_img.shape[1])
     P, S = patch_and_stride(level, stride)
     nx, ny_all = grid_shape(W, H, S)
@@ -167,7 +170,7 @@ def process_level_exchanged(level_img, lesion_mask, level: int, packed: _feature
     for a in range(i0, i1, rows_per_group):
         seg = process_level_enqueue(level_img, lesion_mask, level, packed, stride=stride, row_range=(a, min(a + rows_per_group, i1)),
                                     chunk=chunk, mode=mode, tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue,
-                                    roi=roi, roi_y_origin=y_offset)
+                                    roi=roi, roi_y_origin=y_offset, tta=tta)
         exchange.pack(g, seg.pend.coords, seg.pend.labels, seg.features, seg.logits, seg.count, y_offset=y_offset)
         g += 1
     for e in range(g, exchange.spr):
