@@ -153,6 +153,47 @@ int hipac_tile_scan_roi(const uint8_t* d_rgb, int H, int W, int64_t pitch_bytes,
                         const uint8_t* d_roi, int roi_nx, int roi_ny, int roi_level_shift, int roi_stride, int roi_patch,
                         int64_t y_origin, void* stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Macenko stain normalisation (torchstain's NumpyMacenkoNormalizer, the stain matrix estimated once per slide).
+ * OD(v) = -log((v + 1) / Io) per channel, fp64.
+ *
+ * Stain block, fp64 [HIPAC_STAIN_BLOCK_DOUBLES]: [0..5] HE row-major [3][2] (column 0 haematoxylin, column 1 eosin),
+ * [6..7] maxC, [8] valid (1 or 0), [9] n_hat (pixels whose three ODs are all >= beta), [10..15] zero.
+ * Parameter block, fp64 [HIPAC_STAIN_PARAMS_DOUBLES]: [0] valid, [1] Io, [2..10] M row-major [3][3], [11..266] od[256].
+ *
+ * hipac_stain_estimate  (HE, maxC) of the uint8 RGB image d_rgb [H][pitch] (e.g. a slide thumbnail): ODhat = the pixels with
+ *                       all three ODs >= beta; E = the eigenvectors of np.cov(ODhat) with the two largest eigenvalues;
+ *                       phi = atan2 of ODhat . E; vMin / vMax = E (cos, sin) of numpy's linear percentiles alpha and
+ *                       100 - alpha of phi; HE = [vMin, vMax] if vMin[0] > vMax[0] else [vMax, vMin]; C = P . OD over all
+ *                       pixels with P below; maxC = the 99th percentiles of C's rows.  valid = 0 when n_hat < 2,
+ *                       det(HE^T HE) <= 0, a value is not finite or maxC <= 0.  A fixed sequence of kernels on `stream`
+ *                       with no host wait and no floating-point atomics: the block is the same bits on every run.
+ *                       Io in 1..255, alpha in (0, 50), beta finite and >= 0; H * W < 2^31.
+ *                       d_ws >= hipac_stain_workspace_bytes(H, W) bytes (16 per pixel + 48 KB), 256-byte aligned.
+ * hipac_stain_normalizer  the parameter block that maps d_src's stain to d_target's (NULL: torchstain's reference,
+ *                       HERef = [[0.5626, 0.2159], [0.7201, 0.8012], [0.4062, 0.5581]], maxCRef = [1.9705, 1.0308]).
+ *                       In fp64, every operation rounded on its own:  g_ij = (HE[0][i] HE[0][j] + HE[1][i] HE[1][j])
+ *                       + HE[2][i] HE[2][j];  det = g00 g11 - g01 g01;  P = [[g11, -g01], [-g01, g00]] / det . HE^T;
+ *                       s_i = maxCRef_i / maxC_i;  M[c][j] = (HERef[c][0] s_0) P[0][j] + (HERef[c][1] s_1) P[1][j];
+ *                       od[v] = -log((v + 1) / Io).  valid = both blocks valid, det > 0 and M finite.  One kernel.
+ * hipac_stain_apply     d_in uint8 [n_patches][224][224][3]; per pixel and channel c
+ *                       y = (M[c][0] od[r] + M[c][1] od[g]) + M[c][2] od[b] (products rounded, no FMA) and
+ *                       out_c = #{v in 0..254 : y <= od[v]}, which is uint8(min(255, Io exp(-y))) = torchstain's
+ *                       normalize with the source's (HE, maxC).  valid = 0: out = in.  Outputs: d_out_u8 (uint8, may be
+ *                       d_in itself, otherwise disjoint) and / or d_batch in `layout` (the stage-1 ToTensor/Normalize
+ *                       of out; S2D16 padding columns and channels 12..15 written as zero; layout 0 = no d_batch).
+ *                       d_count: NULL = all n_patches, else only patches < clamp(d_count[0] - n_base, 0, n_patches)
+ *                       are read and written.  Buffers 16-byte aligned.  One kernel.
+ * ------------------------------------------------------------------------------------- */
+#define HIPAC_STAIN_BLOCK_DOUBLES 16
+#define HIPAC_STAIN_PARAMS_DOUBLES 267
+size_t hipac_stain_workspace_bytes(int H, int W);
+int hipac_stain_estimate(const uint8_t* d_rgb, int H, int W, int64_t pitch, int Io, double alpha, double beta, double* d_stain,
+                         void* d_ws, size_t ws_bytes, void* stream);
+int hipac_stain_normalizer(const double* d_src, const double* d_target, int Io, double* d_params, void* stream);
+int hipac_stain_apply(const uint8_t* d_in, int n_patches, const int32_t* d_count, int n_base, const double* d_params,
+                      uint8_t* d_out_u8, void* d_batch, int layout, void* stream);
+
 /* Early survivor count.  If a pinned host buffer int32[2] is registered (calling thread), every hipac_tile_scan copies
  * {survivors, candidates} into it right after the compaction kernel and records an event; hipac_tile_scan_wait_count
  * blocks only until that copy has landed -- the resample / gather kernels of the same call keep running, so the caller

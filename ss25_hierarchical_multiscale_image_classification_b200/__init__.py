@@ -6,5 +6,6 @@ reached through the C ABI in ``include/hipac_b200.h``.
 """
 from . import _lib  # noqa: F401
 from .cascade import RoiGrid, process_cascade, roi_grid, threshold_of, tumor_margin  # noqa: F401
+from .preprocessing.stain import Stain, StainNormalizer, estimate_stain  # noqa: F401
 
 __version__ = "0.1.0"

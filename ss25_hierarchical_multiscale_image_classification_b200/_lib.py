@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "libhipac_b200.so")
 # the same library with -DHIPAC_DEBUG_BOUNDS (device-side bounds assertions in the stage-1 kernels); loaded instead of
 # LIB_PATH when HIPAC_DEBUG_BOUNDS=1 is in the environment (tests/test_debug_bounds_gpu.py runs it in a subprocess)
 DBG_LIB_PATH = os.path.join(_HERE, "libhipac_b200_dbg.so")
-SOURCES = ["capi.cu", "tile_scan.cu", "resnet18.cu", "exchange.cu", "polygon.cu", "mil.cu", "debug_umma.cu", "tissue.cu", "cascade.cu"]
+SOURCES = ["capi.cu", "tile_scan.cu", "resnet18.cu", "exchange.cu", "polygon.cu", "mil.cu", "debug_umma.cu", "tissue.cu", "cascade.cu", "stain.cu"]
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "hipac_b200.h")
 
 LAYOUT_NHWC3_BF16 = 1
@@ -25,6 +25,8 @@ SCAN_AUTO, SCAN_DIRECT, SCAN_FUSED = 0, 1, 2
 SCAN_KEEP_ALL = 0x100
 SCAN_NO_STREAM = 0x200
 RESNET18_NUM_CONVS = 20
+STAIN_BLOCK_DOUBLES = 16
+STAIN_PARAMS_DOUBLES = 267
 
 _lock = threading.Lock()
 _lib = None
@@ -137,6 +139,14 @@ def _declare(l):
     l.hipac_tissue_workspace_bytes.argtypes = [i32, i32]
     l.hipac_tissue_segment.restype = i32
     l.hipac_tissue_segment.argtypes = [vp, i32, i32, i64, i32, i32, vp, i64, vp, vp, i64, vp, sz, vp]
+    l.hipac_stain_workspace_bytes.restype = sz
+    l.hipac_stain_workspace_bytes.argtypes = [i32, i32]
+    l.hipac_stain_estimate.restype = i32
+    l.hipac_stain_estimate.argtypes = [vp, i32, i32, i64, i32, C.c_double, C.c_double, vp, vp, sz, vp]
+    l.hipac_stain_normalizer.restype = i32
+    l.hipac_stain_normalizer.argtypes = [vp, vp, i32, vp, vp]
+    l.hipac_stain_apply.restype = i32
+    l.hipac_stain_apply.argtypes = [vp, i32, vp, i32, vp, vp, vp, i32, vp]
     l.hipac_tile_scan_set_count_buffer.restype = i32
     l.hipac_tile_scan_set_count_buffer.argtypes = [vp]
     l.hipac_tile_scan_wait_count.restype = i32
@@ -209,6 +219,7 @@ EXPORTS = [
     "hipac_tile_scan_tissue_workspace_bytes", "hipac_tile_scan_tissue", "hipac_tissue_workspace_bytes", "hipac_tissue_segment",
     "hipac_roi_grid_bytes", "hipac_roi_grid", "hipac_tile_scan_roi_workspace_bytes", "hipac_tile_scan_roi",
     "hipac_resnet18_forward_d4", "hipac_batch_d4_view",
+    "hipac_stain_workspace_bytes", "hipac_stain_estimate", "hipac_stain_normalizer", "hipac_stain_apply",
 ]
 
 

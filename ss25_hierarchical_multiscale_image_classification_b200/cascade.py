@@ -85,7 +85,8 @@ def roi_grid(coords: torch.Tensor, scores: torch.Tensor, level: int, width: int,
 
 
 def process_cascade(levels: dict, packed, order=(3, 0), tau: float = 0.5, dilate: int = 0, stride=None, tissue=None,
-                    tissue_level: int | None = None, min_tissue=0.5, chunk: int = 8192, tta: bool = False) -> dict:
+                    tissue_level: int | None = None, min_tissue=0.5, chunk: int = 8192, tta: bool = False,
+                    stain=None) -> dict:
     """Coarse-to-fine cascade over the levels in ``order`` (strictly decreasing, e.g. ``(3, 0)`` or the chain ``(3, 1, 0)``).
 
     ``levels`` maps a level number to ``(img, lesion_mask)`` on the device (``lesion_mask`` may be None); ``packed`` is one
@@ -94,7 +95,8 @@ def process_cascade(levels: dict, packed, order=(3, 0), tau: float = 0.5, dilate
     ``tumor_margin(logits) >= threshold_of(tau)`` (dilated by ``dilate`` cells).  ``tissue``: optional tissue mask of level
     ``tissue_level`` (e.g. ``segment_tissue`` of the thumbnail), used at scale ``2 ** (tissue_level - L)`` for every level
     ``L`` in place of the ``mean > 240`` rule.  ``tta``: every level is classified with the D4 test-time augmentation
-    (``process_level(tta=True)``), so each ROI is scored on the averaged logits.  Returns ``{level: LevelResult}``; each fine result equals the full
+    (``process_level(tta=True)``), so each ROI is scored on the averaged logits.  ``stain``: one ``StainNormalizer`` for
+    every level (one slide, one stain), applied to every survivor before the network.  Returns ``{level: LevelResult}``; each fine result equals the full
     ``process_level`` of that level restricted to the ROI."""
     order = tuple(int(L) for L in order)
     if not order or any(a <= b for a, b in zip(order, order[1:])):
@@ -107,7 +109,7 @@ def process_cascade(levels: dict, packed, order=(3, 0), tau: float = 0.5, dilate
         img, mask = levels[L]
         net = packed[L] if isinstance(packed, dict) else packed
         tis = {} if tissue is None else dict(tissue=tissue, tissue_scale=1 << (tissue_level - L), min_tissue=min_tissue)
-        r = _pipeline.process_level(img, mask, L, net, stride=stride, chunk=chunk, roi=roi, tta=tta, **tis)
+        r = _pipeline.process_level(img, mask, L, net, stride=stride, chunk=chunk, roi=roi, tta=tta, stain=stain, **tis)
         results[L] = r
         if k + 1 < len(order):
             if r.logits is None or r.logits.shape[1] < 2:

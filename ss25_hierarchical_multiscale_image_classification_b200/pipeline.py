@@ -54,13 +54,15 @@ class PendingLevel:
 
 def process_level_enqueue(level_img, lesion_mask, level, packed, stride=None, row_range=None, chunk: int = 8192,
                           mode: str = "auto", tissue=None, tissue_scale: int = 1, min_tissue=0.5, roi=None,
-                          roi_y_origin: int = 0, tta: bool = False) -> PendingLevel:
+                          roi_y_origin: int = 0, tta: bool = False, stain=None) -> PendingLevel:
     """Enqueue tile scan + ResNet18 of candidate grid rows ``row_range`` without any host wait (the network kernels read
     the survivor count from device memory).  Feed the result to ``sharding.SurvivorExchange.pack``.  ``tissue`` /
     ``tissue_scale`` / ``min_tissue``: the tissue-mask filter, ``roi`` / ``roi_y_origin``: the coarse-level ROI of
-    ``extract_patches_enqueue``.  ``tta``: the D4 test-time augmentation of ``features.classify_tensor``."""
+    ``extract_patches_enqueue``.  ``tta``: the D4 test-time augmentation of ``features.classify_tensor``.  ``stain``: the
+    ``StainNormalizer`` applied to every survivor before the network (see ``extract_patches_enqueue``)."""
     pend = extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=row_range, layout="s2d16", mode=mode,
-                                   tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin)
+                                   tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin,
+                                   stain=stain)
     if packed.num_classes > 0:
         feats, logits = _features.classify_tensor(pend.batch, packed, chunk, count=pend.count, tta=tta)
     else:
@@ -69,21 +71,23 @@ def process_level_enqueue(level_img, lesion_mask, level, packed, stride=None, ro
 
 
 def _process_rows(level_img, lesion_mask, level, packed, stride, rows, chunk, mode, tissue=None, tissue_scale=1, min_tissue=0.5,
-                  roi=None, roi_y_origin=0, tta=False):
+                  roi=None, roi_y_origin=0, tta=False, stain=None):
     """Tile scan + ResNet18 of one candidate-row group, enqueued back to back: the network kernels take the survivor
     count from device memory (``hipac_resnet18_forward_dcount``), so the host only learns it afterwards, to slice the
     capacity-sized outputs -- while the GPU is already running the network."""
     if _lib.profiling():
         # the per-kernel profiler attributes flops by the host-side patch count: use the host-count path
         pb = extract_patches_tensor(level_img, lesion_mask, level, stride=stride, row_range=rows, layout="s2d16", mode=mode,
-                                    tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin)
+                                    tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin,
+                                    stain=stain)
         if packed.num_classes > 0:
             feats, logits = _features.classify_tensor(pb.batch, packed, chunk, tta=tta)
         else:
             feats, logits = _features.extract_features_tensor(pb.batch, packed, chunk, tta=tta), None
         return LevelResult(pb.coords, pb.labels, feats, logits, pb.candidates)
     pend = extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=rows, layout="s2d16", mode=mode,
-                                   tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin)
+                                   tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, roi=roi, roi_y_origin=roi_y_origin,
+                                   stain=stain)
     if packed.num_classes > 0:
         feats, logits = _features.classify_tensor(pend.batch, packed, chunk, count=pend.count, tta=tta)
     else:
@@ -95,7 +99,8 @@ def _process_rows(level_img, lesion_mask, level, packed, stride, rows, chunk, mo
 
 def process_level(level_img: torch.Tensor, lesion_mask, level: int, packed: _features.PackedResNet18, stride=None,
                   row_range=None, chunk: int = 8192, mode: str = "auto", max_candidates: int = 16384, tissue=None,
-                  tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0, tta: bool = False) -> LevelResult:
+                  tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0, tta: bool = False,
+                  stain=None) -> LevelResult:
     """Tile + tissue/lesion mask + ResNet18 features of a level image resident on the GPU.
 
     ``tissue`` / ``tissue_scale`` / ``min_tissue``: keep the candidates a tissue mask covers (e.g. ``segment_tissue`` of a
@@ -107,6 +112,9 @@ def process_level(level_img: torch.Tensor, lesion_mask, level: int, packed: _fea
     ``tta``: rotation/flip test-time augmentation in stage 2 (``features.classify_tensor(..., tta=True)``): features and
     logits of every survivor are those of its eight D4 views averaged; coordinates, labels and candidates do not change.
 
+    ``stain``: a ``preprocessing.StainNormalizer`` (Macenko, e.g. from ``estimate_stain`` of the slide's thumbnail): every
+    survivor is normalised before ToTensor/Normalize; coordinates, labels and candidates do not change.
+
     The batch buffer is sized for the worst case (every candidate survives), so levels with more than
     ``max_candidates`` candidates are processed in groups of whole candidate-grid rows (a 100k x 100k level at
     224-px tiles has 200k candidates = 82 GB of batch at once); the result is returned in canonical ``(x, y)``
@@ -116,7 +124,7 @@ def process_level(level_img: torch.Tensor, lesion_mask, level: int, packed: _fea
     nx, ny_all = grid_shape(W, H, S)
     i0, i1 = (0, ny_all) if row_range is None else (int(row_range[0]), int(row_range[1]))
     rows_per_group = max(1, max_candidates // max(nx, 1))
-    tis = dict(tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, tta=tta)
+    tis = dict(tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue, tta=tta, stain=stain)
     if roi is not None:
         tis.update(roi=roi, roi_y_origin=roi_y_origin)
     if i1 - i0 <= rows_per_group:
@@ -146,7 +154,7 @@ def exchange_for_level(device, width: int, rows_per_rank: int, stride: int, num_
 
 def process_level_exchanged(level_img, lesion_mask, level: int, packed: _features.PackedResNet18, exchange, stride=None,
                             row_range=None, y_offset: int = 0, chunk: int = 8192, mode: str = "auto", tissue=None,
-                            tissue_scale: int = 1, min_tissue=0.5, roi=None, tta: bool = False) -> int:
+                            tissue_scale: int = 1, min_tissue=0.5, roi=None, tta: bool = False, stain=None) -> int:
     """``process_level`` whose result goes straight into the exchange step: the rank's grid rows are cut into the exchange's
     row groups, each group is enqueued (tile scan + ResNet18, survivor count on the device) and packed as one segment, then
     ``exchange.merge()`` is enqueued.  No host wait anywhere; call ``exchange.result()`` for the merged, canonically
@@ -158,7 +166,8 @@ def process_level_exchanged(level_img, lesion_mask, level: int, packed: _feature
     same mask and an N-rank result equals a single-rank one.
 
     ``roi``: a ``cascade.RoiGrid`` of a coarser level over the WHOLE slide (every rank builds the same one from the
-    exchanged coarse result); the rank's slab is placed in it by ``y_offset``.  ``tta``: as in ``process_level``."""
+    exchanged coarse result); the rank's slab is placed in it by ``y_offset``.  ``tta``, ``stain``: as in ``process_level``
+    (every rank estimates the same stain from the same thumbnail, bit for bit)."""
     H, W = int(level_img.shape[0]), int(level_img.shape[1])
     P, S = patch_and_stride(level, stride)
     nx, ny_all = grid_shape(W, H, S)
@@ -170,7 +179,7 @@ def process_level_exchanged(level_img, lesion_mask, level: int, packed: _feature
     for a in range(i0, i1, rows_per_group):
         seg = process_level_enqueue(level_img, lesion_mask, level, packed, stride=stride, row_range=(a, min(a + rows_per_group, i1)),
                                     chunk=chunk, mode=mode, tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue,
-                                    roi=roi, roi_y_origin=y_offset, tta=tta)
+                                    roi=roi, roi_y_origin=y_offset, tta=tta, stain=stain)
         exchange.pack(g, seg.pend.coords, seg.pend.labels, seg.features, seg.logits, seg.count, y_offset=y_offset)
         g += 1
     for e in range(g, exchange.spr):

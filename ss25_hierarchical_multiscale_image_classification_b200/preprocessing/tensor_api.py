@@ -154,19 +154,20 @@ def extract_patches_tensor(level_img: torch.Tensor, lesion_mask: torch.Tensor | 
                            stride=None, row_range=None, patch_size: int = 224, layout: str | None = "s2d16",
                            want_u8: bool = False, mode: str = "auto", capacity: int | None = None,
                            stream: torch.cuda.Stream | None = None, keep_all: bool = False, tissue: torch.Tensor | None = None,
-                           tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0) -> PatchBatch:
+                           tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0, stain=None) -> PatchBatch:
     """``extract_patches_enqueue(...).resolve()``: see there."""
     return extract_patches_enqueue(level_img, lesion_mask, level, stride=stride, row_range=row_range, patch_size=patch_size,
                                    layout=layout, want_u8=want_u8, mode=mode, capacity=capacity, stream=stream,
                                    keep_all=keep_all, tissue=tissue, tissue_scale=tissue_scale, min_tissue=min_tissue,
-                                   roi=roi, roi_y_origin=roi_y_origin).resolve()
+                                   roi=roi, roi_y_origin=roi_y_origin, stain=stain).resolve()
 
 
 def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor | None, level: int,
                             stride=None, row_range=None, patch_size: int = 224, layout: str | None = "s2d16",
                             want_u8: bool = False, mode: str = "auto", capacity: int | None = None,
                             stream: torch.cuda.Stream | None = None, keep_all: bool = False, tissue: torch.Tensor | None = None,
-                            tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0) -> PendingPatchBatch:
+                            tissue_scale: int = 1, min_tissue=0.5, roi=None, roi_y_origin: int = 0,
+                            stain=None) -> PendingPatchBatch:
     """Tile one level image (uint8 ``[H,W,3]`` on a CUDA device) exactly as the reference does.
 
     ``lesion_mask``: uint8 ``[H,W]`` (>0 = lesion, the rasterised ``parse_xml_mask`` output,
@@ -184,9 +185,15 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
     ``roi``: a ``cascade.RoiGrid`` of a coarser level (the coarse-to-fine cascade).  After the ``mean > 240`` or tissue-mask
     rule, a candidate survives only if its footprint overlaps with positive area the footprint of a set ROI cell, both taken
     at this level's resolution.  ``roi_y_origin`` is the level row of ``level_img``'s row 0 (a shard's slab).  Cannot be
-    combined with ``keep_all``.  Nothing blocks: the call returns capacity-sized tensors and the device-side survivor
-    counter; ``resolve()`` waits only until the count is known (after the compaction kernel) and slices, and
-    ``features.classify_tensor(..., count=pending.count)`` consumes the batch without any host round trip.
+    combined with ``keep_all``.
+
+    ``stain``: a ``preprocessing.StainNormalizer`` (Macenko).  The survivors' resized uint8 patches are normalised
+    (``hipac_stain_apply``) before ToTensor/Normalize: ``batch`` and ``images_u8`` hold the normalised patches.  Grid,
+    tissue test, ROI, labels and survivor order are decided on the raw pixels and do not change.
+
+    Nothing blocks: the call returns capacity-sized tensors and the device-side survivor counter; ``resolve()`` waits only
+    until the count is known (after the compaction kernel) and slices, and ``features.classify_tensor(...,
+    count=pending.count)`` consumes the batch without any host round trip.
     """
     l = _lib.lib()
     if not (level_img.is_cuda and level_img.dtype == torch.uint8 and level_img.dim() == 3 and level_img.shape[2] == 3):
@@ -211,6 +218,8 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
             raise ValueError("roi.grid must be a contiguous uint8 [ny, nx] tensor on the level image's device")
         if int(roi_y_origin) < 0:
             raise ValueError("roi_y_origin must be >= 0")
+    if stain is not None and stain.device != level_img.device:
+        raise ValueError("the stain normaliser lives on another device than the level image")
     if tissue is not None:
         if not (tissue.is_cuda and tissue.dtype == torch.uint8 and tissue.dim() == 2 and tissue.device == level_img.device):
             raise ValueError("tissue must be a uint8 [h, w] tensor on the level image's device")
@@ -242,6 +251,10 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
         count = torch.zeros((2,), dtype=torch.int32, device=dev)
         batch = torch.empty(batch_shape(max(cap, 1), layout), dtype=torch.bfloat16, device=dev) if layout else None
         u8 = torch.empty((max(cap, 1), OUT, OUT, 3), dtype=torch.uint8, device=dev) if want_u8 else None
+        # with a normaliser stage 1 writes only the uint8 patches (into a scratch buffer unless they are wanted) and the
+        # apply kernel writes the batch from them
+        scan_u8 = u8 if stain is None or want_u8 else torch.empty((max(cap, 1), OUT, OUT, 3), dtype=torch.uint8, device=dev)
+        scan_batch = batch if stain is None else None
         m = _MODES[mode] | (_lib.SCAN_KEEP_ALL if keep_all else 0)
         if roi is not None:
             ws_bytes = l.hipac_tile_scan_roi_workspace_bytes(H, W, P, S, i0, i1, m, tissue_scale if tissue is not None else 0)
@@ -257,8 +270,8 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
                 lesion_mask.data_ptr() if lesion_mask is not None else None,
                 int(lesion_mask.stride(0)) if lesion_mask is not None else 0,
                 P, S, i0, i1, coords.data_ptr(), labels.data_ptr(),
-                u8.data_ptr() if u8 is not None else None,
-                batch.data_ptr() if batch is not None else None, _LAYOUTS[layout] if layout else 0,
+                scan_u8.data_ptr() if scan_u8 is not None else None,
+                scan_batch.data_ptr() if scan_batch is not None else None, _LAYOUTS[layout] if scan_batch is not None else 0,
                 count.data_ptr(), cap, ws.data_ptr(), ws_bytes, m)
         if tissue is not None:
             th, tw = int(tissue.shape[0]), int(tissue.shape[1])
@@ -272,6 +285,9 @@ def extract_patches_enqueue(level_img: torch.Tensor, lesion_mask: torch.Tensor |
         else:
             _lib.check(l.hipac_tile_scan_tissue(*args, *tis, st.cuda_stream), "hipac_tile_scan_tissue")
         ws.record_stream(st)
+        if stain is not None and (batch is not None or want_u8):
+            stain.apply(scan_u8, layout, count=count, out_u8=u8, out=batch, stream=st)
+            scan_u8.record_stream(st)
     del h_count   # registered with the library; read in resolve()
     _count_host.seq = getattr(_count_host, "seq", 0) + 1
     return PendingPatchBatch(coords=coords, labels=labels, batch=batch, images_u8=u8, count=count, capacity=cap,
